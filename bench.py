@@ -2,6 +2,7 @@
 """bench.py -- the headline benchmark of upretinex-b200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4|c5] [--no-named]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -134,6 +135,47 @@ def make_frames(torch, n, h, w, seed, device):
                 ys = torch.linspace(0, 1, h, device=device)[:, None].expand(h, w)
                 x[i, 0], x[i, 1], x[i, 2] = xs, ys, (xs + ys) / 2
     return x
+
+
+DUMP_BYTES = 48 << 20   # --dump-outputs: the files of one run stay well under 64 MB in all
+
+
+def dump_outputs(dirname, arrays):
+    """Write the arrays the timed path returned in its last step as DIR/<name>.npy (float32).  Arrays up to 1 MB are written
+    whole; a larger [N,C,H,W] output is reduced to a fixed, seeded sample (the same image rows of the same frames on every
+    run), so that two builds of the project can be compared output for output.  Everything written fits in DUMP_BYTES."""
+    import numpy as np
+    import torch
+    big = [k for k, t in arrays.items() if t.numel() * 4 > (1 << 20)]
+    small = sum(t.numel() * 4 for k, t in arrays.items() if k not in big)
+    if small > DUMP_BYTES or any(arrays[k].dim() != 4 for k in big):
+        raise ValueError("--dump-outputs samples one [N,C,H,W] output per name; these arrays do not fit its budget")
+    share = (DUMP_BYTES - small) // max(1, len(big))
+    os.makedirs(dirname, exist_ok=True)
+    written = 0
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if name in big:
+            n, c, h, w = t.shape
+            rng = np.random.default_rng(0)
+            row_bytes = c * w * 4
+            frames = min(n, max(1, share // row_bytes))
+            rows = min(h, max(1, share // (frames * row_bytes)))
+            ri = torch.from_numpy(np.sort(rng.choice(h, rows, replace=False))).to(t.device)
+            fi = torch.from_numpy(np.sort(rng.choice(n, frames, replace=False))).to(t.device)
+            t = t.index_select(2, ri).index_select(0, fi)
+        a = t.cpu().numpy()
+        written += a.nbytes
+        if written > DUMP_BYTES:
+            raise ValueError(f"--dump-outputs: {name} does not fit the {DUMP_BYTES} byte budget even as one row per frame")
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
+
+
+def output_dumper(args, rank):
+    """The --dump-outputs hook handed to a workload: rank 0 writes its own outputs; None without the flag and on other ranks."""
+    if not args.dump_outputs or rank != 0:
+        return None
+    return lambda arrays: dump_outputs(args.dump_outputs, arrays)
 
 
 def event_time_ms(torch, fn, iters):
@@ -338,16 +380,8 @@ def run_reference_arm(args):
                       f"the reference's own serial per-frame loop, cv2 {cv2.__version__} default threading on {cores} cores")
         except Exception as e:  # pragma: no cover
             sample += f" (reference import failed: {e!r})"
-    # bound the run: at most ~4 minutes for warmup + steps (the step itself stays 64 frames unless that is impossible)
-    t0 = time.perf_counter()
-    step()
-    first = time.perf_counter() - t0
-    warmup, steps, note = args.warmup, args.steps, None
-    if first * (warmup + steps) > 240.0:
-        steps = max(1, int(240.0 / first) - 1)
-        warmup = min(warmup, 1)
-        note = f"steps reduced from {args.steps} to {steps} (one step takes {first:.1f} s on this host)"
-    for _ in range(max(0, warmup - 1)):
+    warmup, steps = args.warmup, args.steps
+    for _ in range(max(1, warmup)):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
@@ -360,8 +394,6 @@ def run_reference_arm(args):
             "cpu_baseline": {"value": mpix, "unit": UNIT, "cores": cores, "kind": kind, "sample": sample, "port_threaded": port},
             "e2e": {"value": mpix, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
-    if note:
-        line["note"] = note
     emit(line)
     return 0
 
@@ -381,7 +413,7 @@ class StubMaps:
         return x.mean(dim=1, keepdim=True) * 0.5 + 0.25, self.torch.sqrt(x)
 
 
-def record_c3(torch, dist, rank, world, local, steps, warmup, total_frames=256):
+def record_c3(torch, dist, rank, world, local, steps, warmup, total_frames=256, dump=None):
     """BASELINE config 3: multi-scale statistics (a4) + gain/clamp (a5) on 256 4K frames sharded over the GPUs of the run
     (strong scaling: 256 / N frames per GPU; x read once, enhanced read, out written = 36 B/px)."""
     from retinex_image_enhancement_b200 import native
@@ -392,12 +424,15 @@ def record_c3(torch, dist, rank, world, local, steps, warmup, total_frames=256):
     enh = torch.rand((n, 3, h, w), device=dev, generator=torch.Generator(device=dev).manual_seed(3000 + rank))
     out = torch.empty_like(enh)
     px = n * h * w
+    last = []
 
     def step():
-        native.multiscale_enhance(x, enh, out=out)
+        last[:] = native.multiscale_enhance(x, enh, out=out)
 
     with ClockSampler(local) as clk:
         ms_step = timed_steps(torch, dist, step, steps, warmup) / steps
+    if dump is not None:
+        dump(dict(zip(("out", "means", "gain"), last)))
     k_stats = statistics.mean(event_time_ms(torch, lambda: native.multiscale_stats(x), 3))
     gain = native.multiscale_stats(x)[1]
     k_clamp = statistics.mean(event_time_ms(torch, lambda: native.scale_clamp(enh, gain, out=out), 3))
@@ -421,7 +456,7 @@ def record_c3(torch, dist, rank, world, local, steps, warmup, total_frames=256):
     return rec
 
 
-def record_c4(torch, dist, rank, world, local, steps, warmup, frames=8, size=256, extras=True):
+def record_c4(torch, dist, rank, world, local, steps, warmup, frames=8, size=256, extras=True, dump=None):
     """BASELINE config 4: texture statistics (a9/a10), per rank 8x3x256x256; the batch mean is one all-reduce of 2 floats.
     Latency bound: us/step for (kernel + NCCL all-reduce + weight kernel), the same as one CUDA graph, and for the ONE fused
     kernel that exchanges the pair over NVLink peer memory; and whether the three agree bit for bit."""
@@ -434,9 +469,11 @@ def record_c4(torch, dist, rank, world, local, steps, warmup, frames=8, size=256
     # the product's default path (losses/loss.py DynamicSmoothWeight): one process = ONE kernel (statistics + batch mean + weight);
     # data-parallel = statistics kernel + NCCL all-reduce of [sum, count] + weight kernel
     default_dsw = L.DynamicSmoothWeight(1.0, True, "tv")
+    last = []
 
     def step():
-        return default_dsw(x)
+        last[:] = [default_dsw(x)]
+        return last[0]
 
     def three_ops():
         _per, stats = L.batch_texture_stats(x, "tv")
@@ -445,6 +482,8 @@ def record_c4(torch, dist, rank, world, local, steps, warmup, frames=8, size=256
 
     with ClockSampler(local) as clk:
         ms_step = timed_steps(torch, dist, step, steps, warmup) / steps
+    if dump is not None:
+        dump({"weight": last[0]})
     w_nccl = three_ops().clone()
     assert torch.equal(step(), w_nccl), "the one-kernel path and the three-operation path disagree"
     three_us = statistics.median(event_time_ms(torch, three_ops, 20)) * 1e3 if world == 1 else None
@@ -540,7 +579,7 @@ def c4_loss_extras(torch, native, L, x, rank, dev):
         return {"error": repr(e)}
 
 
-def record_c5(torch, dist, rank, world, local, steps, warmup, frames=128, chunk=16):
+def record_c5(torch, dist, rank, world, local, steps, warmup, frames=128, chunk=16, dump=None):
     """BASELINE config 5: a stream of 4K frames, 128 per GPU (1024 over 8 GPUs), processed in chunks of 16 through the
     content-aware AND multi-scale enhancers chained in ONE call with ONE shared epilogue (upr_content_multiscale_f32: the
     multi-scale statistics run inside the chunk schedule of the content-aware passes):
@@ -554,13 +593,16 @@ def record_c5(torch, dist, rank, world, local, steps, warmup, frames=128, chunk=
     out = torch.empty_like(enh)
     px = n * h * w
     chunks = [(a, min(a + chunk, n)) for a in range(0, n, chunk)]
+    gains = [None] * len(chunks)
 
     def step():
-        for a, b in chunks:
-            native.content_multiscale_apply(x[a:b], enh[a:b], out=out[a:b])
+        for i, (a, b) in enumerate(chunks):
+            gains[i] = native.content_multiscale_apply(x[a:b], enh[a:b], out=out[a:b])[1]
 
     with ClockSampler(local) as clk:
         ms_step = timed_steps(torch, dist, step, steps, warmup) / steps
+    if dump is not None:
+        dump({"out": out, "gain": torch.cat(gains)})
     a, b = chunks[0]
     cpx = (b - a) * h * w
     k_ca = statistics.mean(event_time_ms(torch, lambda: native.content_aware_apply(x[a:b], enh[a:b], out=out[a:b]), 3))
@@ -608,6 +650,9 @@ def bench_c2(torch, dist, rank, world, local, args):
 
     with ClockSampler(local) as clk:
         ms_total = timed_steps(torch, dist, step, args.steps, args.warmup)
+    dump = output_dumper(args, rank)
+    if dump is not None:
+        dump({"out": out})      # before the kernel legs below overwrite `out`
     ms_step = ms_total / args.steps
     value = world * px / 1e6 / (ms_step / 1e3)
 
@@ -743,19 +788,21 @@ def bench_c2(torch, dist, rank, world, local, args):
 
 
 def bench_c3(torch, dist, rank, world, local, args):
-    rec = record_c3(torch, dist, rank, world, local, args.steps, args.warmup, total_frames=(args.frames * world) if args.frames else 256)
+    rec = record_c3(torch, dist, rank, world, local, args.steps, args.warmup, total_frames=(args.frames * world) if args.frames else 256,
+                    dump=output_dumper(args, rank))
     rec["vs_baseline"] = None
     return rec
 
 
 def bench_c4(torch, dist, rank, world, local, args):
-    rec = record_c4(torch, dist, rank, world, local, args.steps, args.warmup, frames=args.frames or 8, size=args.size or 256)
+    rec = record_c4(torch, dist, rank, world, local, args.steps, args.warmup, frames=args.frames or 8, size=args.size or 256,
+                    dump=output_dumper(args, rank))
     rec["vs_baseline"] = None
     return rec
 
 
 def bench_c5(torch, dist, rank, world, local, args):
-    rec = record_c5(torch, dist, rank, world, local, args.steps, args.warmup, frames=args.frames or 128)
+    rec = record_c5(torch, dist, rank, world, local, args.steps, args.warmup, frames=args.frames or 128, dump=output_dumper(args, rank))
     rec["vs_baseline"] = None
     return rec
 
@@ -799,7 +846,14 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=15.0)
     ap.add_argument("--traffic", type=float, default=None,
                     help="dram bytes per launch of the dominant kernel from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (rank 0; a fixed sample of "
+                         "outputs over 1 MB, at most 48 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":

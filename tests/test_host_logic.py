@@ -191,11 +191,11 @@ def test_dp_batch_stats_world2_gloo(tmp_path):
 
 
 def test_accelerate_reference_total_loss_patches_the_real_class(monkeypatch):
-    """With the reference tree at hand (build container only): the names accelerate_reference_total_loss relies on exist in
+    """With the unmodified reference at hand (UPR_REFERENCE): the names accelerate_reference_total_loss relies on exist in
     the unmodified losses/loss.py -- TotalLoss().smoothness_loss and the module-level calculate_texture_complexity."""
-    ref = os.environ.get("UPR_REFERENCE", "/root/reference")
+    ref = os.environ.get("UPR_REFERENCE", "")
     if not os.path.isdir(os.path.join(ref, "losses")):
-        pytest.skip("reference tree not present")
+        pytest.skip("set UPR_REFERENCE to an unmodified checkout of xh92117/Retinex-image-Enhancement to run this comparison")
     import importlib.util
     import sys
     import types
@@ -219,9 +219,9 @@ def test_accelerate_reference_total_loss_patches_the_real_class(monkeypatch):
 
 
 def _reference_model_module(monkeypatch):
-    ref = os.environ.get("UPR_REFERENCE", "/root/reference")
+    ref = os.environ.get("UPR_REFERENCE", "")
     if not os.path.isfile(os.path.join(ref, "models", "model.py")):
-        pytest.skip("reference tree not present")
+        pytest.skip("set UPR_REFERENCE to an unmodified checkout of xh92117/Retinex-image-Enhancement to run this comparison")
     import importlib.util
     import sys
     spec = importlib.util.spec_from_file_location("upr_ref_model", os.path.join(ref, "models", "model.py"))
@@ -233,7 +233,7 @@ def _reference_model_module(monkeypatch):
 
 @pytest.mark.parametrize("use_preact,use_aspp", [(False, False), (True, True)])
 def test_model_matches_reference_class(monkeypatch, use_preact, use_aspp):
-    """Build container only: this package's UP_Retinex has the reference's module tree -- a state_dict of the unmodified class
+    """With the unmodified reference at hand (UPR_REFERENCE): this package's UP_Retinex has the reference's module tree -- a state_dict of the unmodified class
     loads with strict=True (the trainer's checkpoint format, trainers/train.py:134-162) and the forward pass reproduces the
     reference's three outputs bit for bit (stock torch ops on both sides: CPU, autograd enabled)."""
     mod = _reference_model_module(monkeypatch)
@@ -278,3 +278,24 @@ def test_accelerate_reference_model_on_the_real_class(monkeypatch):
         acc(x.detach())
     with pytest.raises(TypeError):
         accelerate_reference_model(torch.nn.Linear(2, 2))
+
+
+def test_bench_dump_outputs_writes_a_fixed_bounded_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: small arrays are written whole; a large [N,C,H,W] output becomes the same image rows of every
+    frame on every run, float32, within the byte budget."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 << 20)
+    big = torch.rand((8, 3, 256, 320), generator=torch.Generator().manual_seed(1))
+    gain = torch.rand(8, dtype=torch.float64)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"out": big, "gain": gain})
+    a, b = np.load(tmp_path / "a" / "out.npy"), np.load(tmp_path / "b" / "out.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert a.nbytes <= 2 << 20 and a.shape[:2] == (8, 3) and a.shape[3] == 320 and 1 < a.shape[2] < 256
+    src = big.numpy()
+    rows = [next(r for r in range(256) if np.array_equal(src[:, :, r], a[:, :, k])) for k in range(a.shape[2])]
+    assert rows == sorted(set(rows))
+    g = np.load(tmp_path / "a" / "gain.npy")
+    assert g.dtype == np.float32 and np.array_equal(g, gain.float().numpy())
+    with pytest.raises(ValueError):                     # only [N,C,H,W] outputs can be sampled into the budget
+        bench.dump_outputs(str(tmp_path / "c"), {"flat": big.reshape(-1)})

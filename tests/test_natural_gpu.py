@@ -1,5 +1,5 @@
 """GPU parity on NATURAL image content: crops of the reference's own sample photographs (tests/golden/natural.npz, made by
-tests/golden/make_golden_natural.py from /root/reference/data/input/*.jpg), checked against (i) what the unmodified reference
+tests/golden/make_golden_natural.py from the reference's data/input/*.jpg), checked against (i) what the unmodified reference
 computed on them (hashes, scalars, sub-sampled maps) and (ii) the oracle's full maps; and the same content mirrored / tiled up to
 the BASELINE shapes (1080p, 4K) against the oracle.  Everything goes through the C ABI.
 

@@ -1,7 +1,7 @@
-"""The oracle against the UNMODIFIED reference, live, on random shapes (CPU; runs in the build container where /root/reference
-exists and is skipped elsewhere -- the GPU box only sees the committed golden vectors).  The golden files pin a handful of fixed
-inputs; this sweeps shapes, content kinds and batch rows nobody picked by hand, so that `oracle/` keeps meaning "what the
-reference computes" wherever the GPU parity tests use it.
+"""The oracle against the UNMODIFIED upstream reference, live, on random shapes (CPU; runs where UPR_REFERENCE names a checkout
+of xh92117/Retinex-image-Enhancement and is skipped elsewhere).  The golden files pin a handful of fixed inputs; this sweeps
+shapes, content kinds and batch rows nobody picked by hand, so that `oracle/` keeps meaning "what the reference computes"
+wherever the GPU parity tests use it.
 
 Reference functions executed (paths relative to the reference root): enhancers/adaptive_params.py
 AdaptiveParameterAdjuster.{apply_clahe_enhancement, calculate_brightness_features, adjust_parameters}; enhancers/multi_scale.py
@@ -14,8 +14,8 @@ import sys
 import numpy as np
 import pytest
 
-REF = os.environ.get("UPR_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "enhancers")), reason="the reference tree is not present")
+REF = os.environ.get("UPR_REFERENCE", "")
+pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "enhancers")), reason="set UPR_REFERENCE to an unmodified checkout of xh92117/Retinex-image-Enhancement to run this comparison")
 
 torch = pytest.importorskip("torch")
 pytest.importorskip("cv2")

@@ -241,14 +241,14 @@ def test_resize_linear_u8_recipe_matches_cv2_downscale(sh, sw, dh, dw):
 
 
 def test_letterbox_ref_is_the_reference_function():
-    """oracle/cv2_chain.letterbox_ref against the unmodified reference (when its tree is mounted)."""
-    import os, sys
-    if not os.path.isdir("/root/reference/utils"):
-        pytest.skip("reference tree not mounted")
+    """oracle/cv2_chain.letterbox_ref against the unmodified reference's utils/letterbox.py (UPR_REFERENCE)."""
+    ref_root = os.environ.get("UPR_REFERENCE", "")
+    if not os.path.isdir(os.path.join(ref_root, "utils")):
+        pytest.skip("set UPR_REFERENCE to an unmodified checkout of xh92117/Retinex-image-Enhancement to run this comparison")
     pytest.importorskip("cv2")
     import importlib.util
     import torch
-    spec = importlib.util.spec_from_file_location("ref_letterbox", "/root/reference/utils/letterbox.py")
+    spec = importlib.util.spec_from_file_location("ref_letterbox", os.path.join(ref_root, "utils", "letterbox.py"))
     ref = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref)
     from oracle import cv2_chain
