@@ -15,29 +15,8 @@ import torch
 from . import native
 
 
-def _declare():
-    L = native.lib()
-    if getattr(L, "_upr_ext_declared", False):
-        return L
-    vp, i32 = C.c_void_p, C.c_int
-    L.upr_ext_gaussian_blur_f32.restype = i32
-    L.upr_ext_gaussian_blur_f32.argtypes = [vp, vp, i32, i32, i32, i32, C.c_double, vp]
-    L.upr_ext_msr_f32.restype = i32
-    L.upr_ext_msr_f32.argtypes = [vp, vp, i32, i32, i32, i32, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_float),
-                                  C.c_float, vp]
-    L.upr_ext_pyr_down_f32.restype = i32
-    L.upr_ext_pyr_down_f32.argtypes = [vp, vp, i32, i32, i32, vp]
-    L.upr_ext_gamma_f32.restype = i32
-    L.upr_ext_gamma_f32.argtypes = [vp, vp, C.c_longlong, C.c_float, vp]
-    L._upr_ext_declared = True
-    return L
-
-
 def _prep(x: torch.Tensor) -> torch.Tensor:
-    x = native._require_cuda_f32(x, "x")
-    if x.dim() != 4:
-        raise ValueError(f"expected [N,C,H,W], got {tuple(x.shape)}")
-    return x
+    return native._cuda(x, "x", shape=(None, None, None, None))
 
 
 def gaussian_blur(x: torch.Tensor, ksize: int, sigma: float = 0.0) -> torch.Tensor:
@@ -45,9 +24,8 @@ def gaussian_blur(x: torch.Tensor, ksize: int, sigma: float = 0.0) -> torch.Tens
     x = _prep(x)
     n, c, h, w = x.shape
     out = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        native.check(_declare().upr_ext_gaussian_blur_f32(x.data_ptr(), out.data_ptr(), n * c, h, w, int(ksize), float(sigma),
-                                                          native._stream()), "upr_ext_gaussian_blur_f32")
+    with native._dev(x.device):
+        native._run("upr_ext_gaussian_blur_f32", x.data_ptr(), out.data_ptr(), n * c, h, w, int(ksize), float(sigma))
     return out
 
 
@@ -66,9 +44,8 @@ def multi_scale_retinex(x: torch.Tensor, ksizes: Sequence[int] = (7, 15, 31), si
     ks = (C.c_int * k)(*[int(v) for v in ksizes])
     sg = (C.c_double * k)(*[float(v) for v in sigmas])
     wt = (C.c_float * k)(*[float(v) for v in weights])
-    with torch.cuda.device(x.device):
-        native.check(_declare().upr_ext_msr_f32(x.data_ptr(), out.data_ptr(), n * c, h, w, k, ks, sg, wt, float(eps), native._stream()),
-                     "upr_ext_msr_f32")
+    with native._dev(x.device):
+        native._run("upr_ext_msr_f32", x.data_ptr(), out.data_ptr(), n * c, h, w, k, ks, sg, wt, float(eps))
     return out
 
 
@@ -81,8 +58,8 @@ def pyr_down(x: torch.Tensor) -> torch.Tensor:
     x = _prep(x)
     n, c, h, w = x.shape
     out = torch.empty((n, c, (h + 1) // 2, (w + 1) // 2), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        native.check(_declare().upr_ext_pyr_down_f32(x.data_ptr(), out.data_ptr(), n * c, h, w, native._stream()), "upr_ext_pyr_down_f32")
+    with native._dev(x.device):
+        native._run("upr_ext_pyr_down_f32", x.data_ptr(), out.data_ptr(), n * c, h, w)
     return out
 
 
@@ -96,9 +73,8 @@ def gaussian_pyramid(x: torch.Tensor, levels: int = 3) -> List[torch.Tensor]:
 
 def gamma_correct(x: torch.Tensor, gamma: float) -> torch.Tensor:
     """clamp(x, 0, 1) ** gamma."""
-    x = native._require_cuda_f32(x, "x")
+    x = native._cuda(x, "x")
     out = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        native.check(_declare().upr_ext_gamma_f32(x.data_ptr(), out.data_ptr(), x.numel(), float(gamma), native._stream()),
-                     "upr_ext_gamma_f32")
+    with native._dev(x.device):
+        native._run("upr_ext_gamma_f32", x.data_ptr(), out.data_ptr(), x.numel(), float(gamma))
     return out

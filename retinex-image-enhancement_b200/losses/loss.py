@@ -60,7 +60,7 @@ class PeerBatchStats:
             raise RuntimeError("PeerBatchStats needs an initialised process group")
         group = dist.group.WORLD if group is None else group
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
-        nfloats = (native.lib().upr_peer_stats_buffer_bytes() + 3) // 4
+        nfloats = (native.peer_stats_buffer_bytes() + 3) // 4
         self.buf = symm.empty(nfloats, dtype=torch.float32, device=device)
         self.buf.zero_()
         self.handle = symm.rendezvous(self.buf, group=group.group_name)
@@ -76,12 +76,10 @@ class PeerBatchStats:
     def check(self) -> None:
         """Raise if an exchange on this rank timed out waiting for a peer (the kernel then returned NaN statistics instead of
         hanging or trapping).  Synchronises the current stream: call it once per epoch / when a NaN weight shows up."""
-        import ctypes
-        st = (ctypes.c_uint * 2)()
-        native.check(native.lib().upr_peer_status(self.buf.data_ptr(), st, torch.cuda.current_stream().cuda_stream), "upr_peer_status")
-        if st[0] != 0:
-            raise native.UprError(-4, f"upr_texture_weight_peer_f32: call #{st[0]} on rank {self.rank} timed out waiting for rank "
-                                      f"{st[1]} (every rank must call once per step, in lockstep)")
+        call, peer = native.peer_status(self.buf)
+        if call != 0:
+            raise native.UprError(-4, f"upr_texture_weight_peer_f32: call #{call} on rank {self.rank} timed out waiting for rank "
+                                      f"{peer} (every rank must call once per step, in lockstep)")
 
 
 class DynamicSmoothWeight:

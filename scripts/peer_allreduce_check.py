@@ -63,7 +63,7 @@ def main():
     # a peer that skips a step: the waiting rank gets NaN after the time-out and an exception from check_peers() -- no hang, no trap
     from retinex_image_enhancement_b200 import native
     fused.check_peers()                                   # nothing failed so far
-    native.check(native.lib().upr_peer_set_timeout_ms(150.0), "upr_peer_set_timeout_ms")
+    native.peer_set_timeout_ms(150.0)
     torch.cuda.synchronize()
     dist.barrier()
     timeout_ok = True

@@ -9,9 +9,17 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "upretinex_b200.h")
 
 
+def declared_prototypes():
+    """{entry point: (return type, parameter count)} as include/upretinex_b200.h declares them."""
+    src = re.sub(r"/\*.*?\*/", "", open(HEADER).read(), flags=re.S)
+    protos = {}
+    for ret, name, params in re.findall(r"UPR_API\s+([\w\s\*]+?)\b(upr_\w+)\s*\(([^)]*)\)", src):
+        protos[name] = (" ".join(ret.split()), 0 if params.strip() == "void" else params.count(",") + 1)
+    return protos
+
+
 def declared_symbols():
-    src = open(HEADER).read()
-    return sorted(set(re.findall(r"UPR_API\s+[\w\s\*]+?\b(upr_\w+)\s*\(", src)))
+    return sorted(declared_prototypes())
 
 
 @pytest.fixture(scope="module")
@@ -30,6 +38,15 @@ def test_header_declares_symbols():
 def test_library_exports_every_declared_symbol(lib):
     missing = [s for s in declared_symbols() if not hasattr(lib, s)]
     assert not missing, f"declared in include/upretinex_b200.h but not exported: {missing}"
+
+
+def test_every_entry_point_has_a_prototype(lib):
+    """Loading the library declares every entry point: the header's return type, and one argtype per parameter.  An entry
+    point called without argtypes would get its 64-bit pointers truncated to a C int."""
+    restypes = {"int": ctypes.c_int, "size_t": ctypes.c_size_t, "const char*": ctypes.c_char_p}
+    wrong = {name: (ret, nparams) for name, (ret, nparams) in declared_prototypes().items()
+             if getattr(lib, name).restype is not restypes[ret] or len(getattr(lib, name).argtypes or ()) != nparams}
+    assert not wrong, f"declared differently by native._declare than in include/upretinex_b200.h (return type, parameters): {wrong}"
 
 
 def test_no_torch_types_in_abi():
