@@ -104,6 +104,11 @@ UPR_API int upr_clahe_lab_stages_f32(const float* in_nchw, float* out_nchw, int 
 UPR_API int upr_clahe_debug_dump(const void* workspace, int n, int h, int w, int tiles_x, int tiles_y,
                                  int32_t* hist_out, uint8_t* lut_out, uint8_t* lab_out,
                                  upr_stream_t stream);
+/* The mirror of upr_clahe_debug_dump: copies caller device LUTs ([n][tiles_y*tiles_x][256] u8) and/or Lab planes
+ * ([n][3][h][w] u8) into `workspace` (either may be NULL).  With upr_clahe_lab_stages_f32(stage_mask = 2) this runs the
+ * map kernel alone on chosen inputs. */
+UPR_API int upr_clahe_debug_load(void* workspace, int n, int h, int w, int tiles_x, int tiles_y, const uint8_t* lut_in,
+                                 const uint8_t* lab_in, upr_stream_t stream);
 /* Host copies of the constant tables the kernels use (for tests/audits). Any may be NULL.
  * gamma[256] u16, cbrt[2048] u16, labyf[256] u32 (ify | y<<16), invgamma[4096] u8. */
 UPR_API int upr_get_tables(uint16_t* gamma, uint16_t* cbrt, uint32_t* labyf, uint8_t* invgamma);

@@ -125,6 +125,20 @@ def clahe_u8(src, clip_limit=2.0, tiles=(8, 8), taps=False):
     return (dst, hist, lut) if taps else dst
 
 
+def clahe_map_u8(src, lut, tiles=(8, 8)) -> np.ndarray:
+    """The interpolation step of clahe_u8 alone: src [H,W] u8 through the tile LUTs lut [ty*tx,256] u8 -> [H,W] u8."""
+    a = np.ascontiguousarray(src, dtype=np.uint8)
+    h, w = a.shape
+    tx, ty = tiles
+    t = np.ascontiguousarray(lut, dtype=np.uint8)
+    assert t.shape == (ty * tx, 256), t.shape
+    dst = np.empty_like(a)
+    rc = lib().orc_clahe_map_u8(_p(a), _p(dst), h, w, tx, ty, _p(t))
+    if rc:
+        raise ValueError(f"orc_clahe_map_u8 rc={rc}")
+    return dst
+
+
 def clahe_lab(img, clip_limit=2.0, tiles=(8, 8), taps=False):
     """a1.  img: [1,3,H,W] or [3,H,W] f32 -> [1,3,H,W] f32 (C-contiguous)."""
     a = _chw(img)

@@ -1330,6 +1330,21 @@ int upr_clahe_debug_dump(const void* workspace, int n, int h, int w, int tiles_x
     return UPR_OK;
 }
 
+int upr_clahe_debug_load(void* workspace, int n, int h, int w, int tiles_x, int tiles_y, const uint8_t* lut_in,
+                         const uint8_t* lab_in, upr_stream_t stream)
+{
+    if (!upr::valid_shape(n, h, w, tiles_x, tiles_y)) return UPR_E_SHAPE;
+    if (!workspace) return UPR_E_NULL;
+    if (n == 0) return UPR_OK;
+    const upr::ClaheLayout lay = upr::clahe_layout(n, h, w, tiles_x, tiles_y);
+    auto* base = static_cast<unsigned char*>(workspace);
+    auto s = static_cast<cudaStream_t>(stream);
+    const size_t nt = size_t(n) * tiles_x * tiles_y;
+    if (lut_in) UPR_CUDA_TRY(cudaMemcpyAsync(base + lay.off_lut, lut_in, nt * 256, cudaMemcpyDeviceToDevice, s));
+    if (lab_in) UPR_CUDA_TRY(cudaMemcpyAsync(base + lay.off_lab, lab_in, size_t(n) * 3 * h * w, cudaMemcpyDeviceToDevice, s));
+    return UPR_OK;
+}
+
 int upr_get_tables(uint16_t* gamma, uint16_t* cbrt, uint32_t* labyf, uint8_t* invgamma)
 {
     if (gamma) std::memcpy(gamma, upr::h_gamma, sizeof upr::h_gamma);

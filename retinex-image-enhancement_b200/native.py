@@ -51,6 +51,8 @@ def _declare(lib):
     lib.upr_clahe_lab_stages_f32.argtypes = [vp, vp, i32, i32, i32, f64, i32, i32, vp, sz, i32, vp]
     lib.upr_clahe_debug_dump.restype = i32
     lib.upr_clahe_debug_dump.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.upr_clahe_debug_load.restype = i32
+    lib.upr_clahe_debug_load.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp]
     lib.upr_get_tables.restype = i32
     lib.upr_get_tables.argtypes = [vp] * 4
     f32 = C.c_float
@@ -354,6 +356,24 @@ def clahe_debug(x_shape, tiles: Tuple[int, int] = (8, 8), device=None, want_lab:
         check(L.upr_clahe_debug_dump(ws.data_ptr(), n, h, w, tx, ty, hist.data_ptr(), lut.data_ptr(),
                                      lab.data_ptr() if lab is not None else None, _stream()), "upr_clahe_debug_dump")
     return hist, lut, lab
+
+
+def clahe_map_only(lab_u8: torch.Tensor, lut_u8: torch.Tensor, tiles: Tuple[int, int] = (8, 8)) -> torch.Tensor:
+    """The map stage of clahe_lab() alone on chosen inputs: lab_u8 [N,3,H,W] uint8 (L, a, b planes) and lut_u8
+    [N,ty*tx,256] uint8 (one LUT per tile) -> [N,3,H,W] f32, the de-quantised sRGB of (bilinear LUT interpolation of L, a, b).
+    Loads both into the workspace (upr_clahe_debug_load) and runs upr_clahe_lab_stages_f32 with stage_mask = 2."""
+    lab_u8 = _cuda(lab_u8, "lab_u8", torch.uint8, shape=(None, 3, None, None))
+    n, _, h, w = lab_u8.shape
+    tx, ty = int(tiles[0]), int(tiles[1])
+    dev = lab_u8.device
+    lut_u8 = _cuda(lut_u8, "lut_u8", torch.uint8, shape=(n, ty * tx, 256), device=dev)
+    out = _out(None, lab_u8.shape, torch.float32, dev)
+    with _dev(dev):
+        ws = _ws("upr_clahe_workspace_bytes", (n, h, w, tx, ty), dev)
+        _run("upr_clahe_debug_load", ws.data_ptr(), n, h, w, tx, ty, lut_u8.data_ptr(), lab_u8.data_ptr())
+        # the stages entry checks its input pointer although the map stage does not read it: pass the output
+        _run("upr_clahe_lab_stages_f32", out.data_ptr(), out.data_ptr(), n, h, w, 2.0, tx, ty, ws.data_ptr(), ws.numel(), 2)
+    return out
 
 
 def tables():

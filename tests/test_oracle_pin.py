@@ -111,6 +111,7 @@ def test_clahe_vs_cv2(shape, kind):
     ref = cv2.createCLAHE(clipLimit=2.0, tileGridSize=(8, 8)).apply(src)
     got, hist, lut = O.clahe_u8(src, taps=True)
     assert np.array_equal(got, ref)
+    assert np.array_equal(O.clahe_map_u8(src, lut), got)     # the map step alone, fed the LUTs of the same call
     hp, wp = (h, w) if (h % 8 == 0 and w % 8 == 0) else (h + 8 - h % 8, w + 8 - w % 8)
     assert hist.sum() == hp * wp and (hist.sum(1) == hp * wp // 64).all()
 
@@ -120,7 +121,9 @@ def test_clahe_other_params_vs_cv2(clip, tiles):
     rng = np.random.default_rng(77)
     src = rng.integers(0, 256, (200, 320), dtype=np.uint8)
     ref = cv2.createCLAHE(clipLimit=clip, tileGridSize=tiles).apply(src)
-    assert np.array_equal(O.clahe_u8(src, clip_limit=clip, tiles=tiles), ref)
+    got, _, lut = O.clahe_u8(src, clip_limit=clip, tiles=tiles, taps=True)
+    assert np.array_equal(got, ref)
+    assert np.array_equal(O.clahe_map_u8(src, lut, tiles), got)
 
 
 def test_golden_clahe(golden, small_cases):
