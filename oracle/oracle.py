@@ -11,6 +11,7 @@ clahe_lab              enhancers/adaptive_params.py:121-169
 brightness_features    enhancers/adaptive_params.py:24-68
 adjust_parameters      enhancers/adaptive_params.py:70-119
 multiscale_means       enhancers/multi_scale.py:17-60, :87-94
+multiscale_features    enhancers/multi_scale.py:17-60
 scale_clamp            enhancers/multi_scale.py:97-98
 saliency               enhancers/content_aware.py:19-59
 attention              enhancers/content_aware.py:61-91
@@ -205,6 +206,20 @@ def multiscale_means(img):
     m = np.zeros(3, np.float64)
     f = lib().orc_multiscale_means_f32(_p(a), a.shape[1], a.shape[2], _p(m))
     return m, float(f)
+
+
+def multiscale_features(img):
+    """a4 feature maps of one image: ([7,H,W], [7,int(H/2),int(W/2)], [7,int(H/4),int(W/4)]) f32, channels
+    {R, G, B, luma, |grad R|, |grad G|, |grad B|} -- the values whose means multiscale_means returns."""
+    a = _chw(img)
+    _, h, w = a.shape
+    f = [np.empty((7, int(h * s), int(w * s)), np.float32) for s in (1.0, 0.5, 0.25)]
+    if min(f[2].shape[1:]) < 1:
+        raise ValueError("image too small for the 1/4 scale")
+    rc = lib().orc_multiscale_features_f32(_p(a), h, w, _p(f[0]), _p(f[1]), _p(f[2]))
+    if rc:
+        raise ValueError(f"orc_multiscale_features_f32 rc={rc}")
+    return tuple(f)
 
 
 def scale_clamp(enh, gain: float) -> np.ndarray:

@@ -3,7 +3,8 @@ and the golden vectors produced by the unmodified reference (tests/golden/make_g
 
 Tolerances (SURVEY.md section 8c): a3 exact histogram; a4/a5 means <= 1e-4 relative (stated: 2e-6 achieved);
 a6/a7 <= 1e-4 relative to the map's range (maps are normalised to [0,1]: atol 2e-6); a8 bit-exact vs the oracle
-(<= 1 ulp vs torch); a9 tv <= 1e-4 relative (2e-6 achieved), edge density <= 4/N absolute; a10 <= 1e-6.
+(<= 1 ulp vs torch); a9 tv <= 1e-4 relative (2e-6 achieved), edge density <= 4/N absolute against the reference's golden vectors (its torch
+Sobel sums in another order) and exact against the oracle (same per-pixel fp32 operations, same threshold); a10 <= 1e-6.
 """
 import numpy as np
 import pytest
@@ -228,7 +229,7 @@ def test_texture_vs_oracle(native, shape):
     tv = native.texture_complexity(dev(a), "tv").cpu().numpy()
     np.testing.assert_allclose(tv, O.texture_tv(a), rtol=2e-6)
     ed = native.texture_complexity(dev(a), "edge_density").cpu().numpy()
-    assert np.abs(ed - O.texture_edge_density(a)).max() <= 4.0 / (shape[2] * shape[3])
+    assert np.array_equal(ed, O.texture_edge_density(a))
     # repeated calls reuse the (self-cleaning) workspace
     assert np.array_equal(native.texture_complexity(dev(a), "tv").cpu().numpy(), tv)
 
@@ -319,7 +320,7 @@ def test_zeroed_once_workspaces_survive_shape_and_batch_changes(native):
             if method == "tv":
                 np.testing.assert_allclose(got.cpu().numpy(), ref, rtol=2e-6)
             else:
-                assert np.abs(got.cpu().numpy() - ref).max() <= 4.0 / (96 * 128)
+                assert np.array_equal(got.cpu().numpy(), ref)
             assert float(stats[1]) == b and abs(float(stats[0]) - float(got.double().sum())) <= 1e-5 * b
 
 

@@ -155,6 +155,36 @@ def test_golden_multiscale(golden):
         assert abs(factor - rec["factor"]) <= 1e-7
 
 
+@pytest.mark.parametrize("h,w", [(72, 104), (100, 260), (64, 8), (101, 67), (9, 13), (1081, 1919)])
+def test_multiscale_feature_maps(h, w):
+    """O.multiscale_features against the reference's own torch formulation on the CPU (multi_scale.py:17-60): bilinear
+    F.interpolate to (int(h*s), int(w*s)), luma .299/.587/.114, sqrt(gx^2 + gy^2) of torch.gradient -- at exact scales (h, w
+    multiples of 4) and inexact ones.  The maps' fp64 means are multiscale_means (both come from one per-pixel function, so the
+    golden pins of the means vouch for the maps too).  Largest difference seen: 1.8e-7 absolute on values in [0, 1], i.e. one
+    or two fp32 ulps, from the interpolation and the luma evaluated in another fp32 order (the full-scale image and gradients
+    are equal); the magnitude is taken in fp64 from torch's gradients."""
+    import torch
+    import torch.nn.functional as F
+    x = O.kat_input(h * 7 + w, h, w, "uniform")
+    maps = O.multiscale_features(x)
+    means, _ = O.multiscale_means(x)
+    xt = torch.from_numpy(x)
+    for k, (s, f) in enumerate(zip((1.0, 0.5, 0.25), maps)):
+        size = (int(h * s), int(w * s))
+        assert f.shape == (7,) + size
+        np.testing.assert_allclose(f.astype(np.float64).mean(), means[k], rtol=1e-12, atol=0)
+        img = xt if s == 1.0 else F.interpolate(xt, size=size, mode="bilinear", align_corners=False)
+        img = img[0]
+        luma = 0.299 * img[0] + 0.587 * img[1] + 0.114 * img[2]
+        gx, gy = torch.gradient(img, dim=2)[0].double(), torch.gradient(img, dim=1)[0].double()
+        mag = torch.sqrt(gx * gx + gy * gy)
+        want = torch.cat([img, luma[None]]).numpy()
+        np.testing.assert_allclose(f[:4], want, rtol=0, atol=3e-7, err_msg=f"scale {s}: image / luma")
+        np.testing.assert_allclose(f[4:], mag.numpy(), rtol=0, atol=3e-7, err_msg=f"scale {s}: |grad|")
+        if s == 1.0:
+            assert np.array_equal(f[:3], x[0])
+
+
 def test_golden_content(golden, small_cases):
     for rec in golden["content"]:
         x = O.kat_input(rec["seed"], rec["h"], rec["w"], rec["kind"])
