@@ -206,6 +206,28 @@ UPR_API int upr_retinex_recombine_f32(const float* x, const float* illu, const f
                                       int n, int h, int w, float eps, upr_stream_t stream);
 UPR_API int upr_retinex_decompose_f32(const float* x, const float* illu, float* refl, int n, int h, int w, float eps,
                                       upr_stream_t stream);
+/* The same two lines for training, forward and gradient, with the illumination / enhancement maps in the dtype the CNN
+ * produced them: f32, or fp16 / bf16 under autocast (map_dtype, both maps the same).  x, refl, enh and their gradients are
+ * f32.  Results equal torch eager + autograd bit for bit.  With T the map dtype, f(.) widening to f32, T(.) rounding to T
+ * and every step one IEEE f32 operation (no FMA):
+ *   forward   d = T(f(illu) + eps);  R = x / f(d);  c = e*e, rounded to T unless flags has UPR_RETINEX_AUTOCAST (CUDA
+ *             autocast runs pow in f32);  enh = R*f(e) + (1-R)*f(c)
+ *   gradient  gRt = (-(gE*f(c)) + gR) + gE*f(e)           (autograd's accumulation order; no gR: -(gE*f(c)) + gE*f(e))
+ *             g_x = gRt / f(d)
+ *             g_illu = T(((0 + gd0) + gd1) + gd2),  gd_k = -gRt * ((x/f(d)) / f(d)) of channel k
+ *             g_e = T(f(T(gE*R)) + f(T(f(gc) * f(T(2*f(e))))))   with gc = T(gE*(1-R));
+ *                   under UPR_RETINEX_AUTOCAST gc = gE*(1-R) and 2*f(e) stay f32
+ * x, e, refl, enh: [n][3][h][w]; illu: [n][1][h][w].  e == NULL: decompose only (R).  refl / enh may be NULL when that
+ * output is not wanted (enh needs e).  The gradient entry reads only the forward's inputs (d, R and c are recomputed).
+ * g_enh (gE) and g_refl (gR) are the upstream gradients; either may be NULL (that output received none; not both, and
+ * g_enh needs e); without g_enh a requested g_e is 0.  g_x, g_illu (T, [n][1][h][w]) and g_e (T) are written when non-NULL. */
+enum { UPR_DT_F32 = 0, UPR_DT_F16 = 1, UPR_DT_BF16 = 2 };
+enum { UPR_RETINEX_AUTOCAST = 1 };
+UPR_API int upr_retinex_recombine_maps(const float* x, const void* illu, const void* e, int map_dtype, int flags,
+                                       float* refl, float* enh, int n, int h, int w, float eps, upr_stream_t stream);
+UPR_API int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
+                                       const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e,
+                                       int n, int h, int w, float eps, upr_stream_t stream);
 
 /* ---- a9/a10: texture complexity and the dynamic smoothness weight ------------------------
  * losses/loss.py:523-583: per_image[i] = mean|dx| + mean|dy| ('tv') or the fraction of pixels whose Sobel

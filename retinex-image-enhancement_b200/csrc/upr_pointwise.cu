@@ -1,7 +1,7 @@
 // upr_pointwise.cu -- the three pointwise epilogues of the classical path (sm_100a).
 //
 //   a8  Retinex decomposition + recombination   /root/reference/models/model.py:405-413, :442
-//         R = x / (illu + eps);  enhanced = R*e + (1 - R)*e^2
+//         R = x / (illu + eps);  enhanced = R*e + (1 - R)*e^2   (+ its gradient, for training)
 //   a5  multi-scale gain + clamp                /root/reference/enhancers/multi_scale.py:97-98
 //         out = clamp(enhanced * gain[image], 0, 1)
 //   a7  attention gain + clamp                  /root/reference/enhancers/content_aware.py:119-120
@@ -12,6 +12,9 @@
 // frame-major index space.  Every product/sum is an explicitly rounded fp32 operation
 // (__fmul_rn/__fadd_rn/__fdiv_rn): torch eager evaluates each Python operator as its own
 // kernel, so there is no FMA contraction in the reference and none here -> bit-exact.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "upr_common.cuh"
 
 namespace upr {
@@ -25,17 +28,77 @@ __device__ __forceinline__ float clamp01_keep_nan(float v)
     return v < 0.0f ? 0.0f : (v > 1.0f ? 1.0f : v);
 }
 
+// ---- map storage -------------------------------------------------------------------------
+// The CNN's illumination and enhancement maps are f32, or fp16 / bf16 when the model runs under autocast.  Every map value
+// is widened to f32 on load; rnd<T>(v) = f(T(v)) is the rounding torch applies when an op's result has the map's dtype.
+template <typename T> struct MapIO;
+
+template <> struct MapIO<float> {
+    using Raw4 = float4;   // 4 pixels as loaded
+    static __device__ __forceinline__ float wide(float v) { return v; }
+    static __device__ __forceinline__ float narrow(float v) { return v; }
+    static __device__ __forceinline__ float4 ld4raw(const float* p, uint64_t pol) { return ld_stream_f4(p, pol); }
+    static __device__ __forceinline__ float4 wide4(float4 v) { return v; }
+    static __device__ __forceinline__ float4 ld4(const float* p, uint64_t pol) { return ld_stream_f4(p, pol); }
+    static __device__ __forceinline__ void st4(float* p, float4 v, uint64_t pol) { st_stream_f4(p, v, pol); }
+};
+
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ __half from_f32(float v, const __half*) { return __float2half_rn(v); }
+__device__ __forceinline__ __nv_bfloat16 from_f32(float v, const __nv_bfloat16*) { return __float2bfloat16_rn(v); }
+__device__ __forceinline__ __half from_bits(uint32_t b, const __half*) { return __ushort_as_half((unsigned short)b); }
+__device__ __forceinline__ __nv_bfloat16 from_bits(uint32_t b, const __nv_bfloat16*) { return __ushort_as_bfloat16((unsigned short)b); }
+__device__ __forceinline__ uint32_t to_bits(__half v) { return __half_as_ushort(v); }
+__device__ __forceinline__ uint32_t to_bits(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
+
+template <typename H> struct MapIO16 {   // H = __half or __nv_bfloat16
+    using Raw4 = uint2;    // kept packed until use: fewer registers live across the division slow path
+    static __device__ __forceinline__ float wide(H v) { return to_f32(v); }
+    static __device__ __forceinline__ H narrow(float v) { return from_f32(v, (const H*)nullptr); }
+    static __device__ __forceinline__ float lo(uint32_t u) { return to_f32(from_bits(u & 0xffffu, (const H*)nullptr)); }
+    static __device__ __forceinline__ float hi(uint32_t u) { return to_f32(from_bits(u >> 16, (const H*)nullptr)); }
+    static __device__ __forceinline__ uint32_t pack(float a, float b) { return to_bits(narrow(a)) | (to_bits(narrow(b)) << 16); }
+    // 4 pixels = 8 bytes: one 64-bit streaming access
+    static __device__ __forceinline__ uint2 ld4raw(const H* p, uint64_t pol)
+    {
+        uint2 v;
+        asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.u32 {%0,%1}, [%2], %3;" : "=r"(v.x), "=r"(v.y) : "l"(p), "l"(pol));
+        return v;
+    }
+    static __device__ __forceinline__ float4 wide4(uint2 v) { return make_float4(lo(v.x), hi(v.x), lo(v.y), hi(v.y)); }
+    static __device__ __forceinline__ float4 ld4(const H* p, uint64_t pol) { return wide4(ld4raw(p, pol)); }
+    static __device__ __forceinline__ void st4(H* p, float4 v, uint64_t pol)
+    {
+        asm volatile("st.global.L1::no_allocate.L2::cache_hint.v2.u32 [%0], {%1,%2}, %3;" ::"l"(p), "r"(pack(v.x, v.y)),
+                     "r"(pack(v.z, v.w)), "l"(pol)
+                     : "memory");
+    }
+};
+template <> struct MapIO<__half> : MapIO16<__half> {};
+template <> struct MapIO<__nv_bfloat16> : MapIO16<__nv_bfloat16> {};
+
+template <typename T> __device__ __forceinline__ float rnd(float v) { return MapIO<T>::wide(MapIO<T>::narrow(v)); }
+
+// e^2 with the map dtype T: torch rounds pow's result to T, except under CUDA autocast, where pow runs in fp32
+template <typename T, bool kAutocast> __device__ __forceinline__ float square(float e)
+{
+    return kAutocast ? __fmul_rn(e, e) : rnd<T>(__fmul_rn(e, e));
+}
+
+template <typename T, bool kAutocast>
 __device__ __forceinline__ void recombine1(float x, float d, float e, float& r, float& o)
 {
     r = __fdiv_rn(x, d);
-    o = __fadd_rn(__fmul_rn(r, e), __fmul_rn(__fsub_rn(1.0f, r), __fmul_rn(e, e)));
+    o = __fadd_rn(__fmul_rn(r, e), __fmul_rn(__fsub_rn(1.0f, r), square<T, kAutocast>(e)));
 }
 
 // ---- a8 ---------------------------------------------------------------------------------
-// plane4 = H*W/4 ; one work item = 4 consecutive pixels of one frame (all three channels)
-template <bool kWriteRefl, bool kWriteEnh>
+// plane4 = H*W/4 ; one work item = 4 consecutive pixels of one frame (all three channels).  T = map storage type; d = illu + eps
+// is rounded to T (torch adds the scalar in fp32 and stores a T tensor), R and enhanced are f32 (type promotion).
+template <typename T, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
 __global__ void __launch_bounds__(kPwThreads)
-k_recombine_vec(const float* __restrict__ x, const float* __restrict__ illu, const float* __restrict__ e,
+k_recombine_vec(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
                 float* __restrict__ refl, float* __restrict__ enh, long long plane4, long long items, float eps)
 {
     const uint64_t pol = policy_evict_first();
@@ -43,22 +106,25 @@ k_recombine_vec(const float* __restrict__ x, const float* __restrict__ illu, con
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane4, p = it - f * plane4;
         const long long o3 = (f * 3 * plane4 + p) * 4, o1 = (f * plane4 + p) * 4;
-        const float4 il = ld_stream_f4(illu + o1, pol);
-        const float d[4] = {__fadd_rn(il.x, eps), __fadd_rn(il.y, eps), __fadd_rn(il.z, eps), __fadd_rn(il.w, eps)};
-        float4 xv[3], ev[3];
+        const float4 il = MapIO<T>::ld4(illu + o1, pol);
+        const float d[4] = {rnd<T>(__fadd_rn(il.x, eps)), rnd<T>(__fadd_rn(il.y, eps)), rnd<T>(__fadd_rn(il.z, eps)),
+                            rnd<T>(__fadd_rn(il.w, eps))};
+        float4 xv[3];
+        typename MapIO<T>::Raw4 ev[3];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             xv[c] = ld_stream_f4(x + o3 + c * plane4 * 4, pol);
-            if (kWriteEnh) ev[c] = ld_stream_f4(e + o3 + c * plane4 * 4, pol);
+            if (kWriteEnh) ev[c] = MapIO<T>::ld4raw(e + o3 + c * plane4 * 4, pol);
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             float4 r, o;
             if (kWriteEnh) {
-                recombine1(xv[c].x, d[0], ev[c].x, r.x, o.x);
-                recombine1(xv[c].y, d[1], ev[c].y, r.y, o.y);
-                recombine1(xv[c].z, d[2], ev[c].z, r.z, o.z);
-                recombine1(xv[c].w, d[3], ev[c].w, r.w, o.w);
+                const float4 ef = MapIO<T>::wide4(ev[c]);
+                recombine1<T, kAutocast>(xv[c].x, d[0], ef.x, r.x, o.x);
+                recombine1<T, kAutocast>(xv[c].y, d[1], ef.y, r.y, o.y);
+                recombine1<T, kAutocast>(xv[c].z, d[2], ef.z, r.z, o.z);
+                recombine1<T, kAutocast>(xv[c].w, d[3], ef.w, r.w, o.w);
                 st_stream_f4(enh + o3 + c * plane4 * 4, o, pol);
             } else {
                 r.x = __fdiv_rn(xv[c].x, d[0]);
@@ -71,27 +137,133 @@ k_recombine_vec(const float* __restrict__ x, const float* __restrict__ illu, con
     }
 }
 
-template <bool kWriteRefl, bool kWriteEnh>
+template <typename T, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
 __global__ void __launch_bounds__(kPwThreads)
-k_recombine_scalar(const float* __restrict__ x, const float* __restrict__ illu, const float* __restrict__ e,
+k_recombine_scalar(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
                    float* __restrict__ refl, float* __restrict__ enh, long long plane, long long items, float eps)
 {
     const long long stride = (long long)gridDim.x * kPwThreads;
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane, p = it - f * plane;
-        const float d = __fadd_rn(illu[it], eps);
+        const float d = rnd<T>(__fadd_rn(MapIO<T>::wide(illu[it]), eps));
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const long long o = (f * 3 + c) * plane + p;
             float r, v;
             if (kWriteEnh) {
-                recombine1(x[o], d, e[o], r, v);
+                recombine1<T, kAutocast>(x[o], d, MapIO<T>::wide(e[o]), r, v);
                 enh[o] = v;
             } else {
                 r = __fdiv_rn(x[o], d);
             }
             if (kWriteRefl) refl[o] = r;
         }
+    }
+}
+
+// ---- a8 gradient --------------------------------------------------------------------------
+// What torch autograd computes for the two lines, recomputing d, R and e^2 from the inputs (nothing is saved by the forward).
+// gRt, the gradient reaching R, accumulates in the order the autograd engine adds its parts: g_refl (from R's consumers, which
+// run first) onto -(gE*c) (rsub), then gE*e (the R*e product, created first, runs last).  The e gradient sums the R*e
+// branch, rounded to T, and the e^2 branch, rounded to T once (in T arithmetic without autocast; by the fp32 cast's backward
+// under autocast).  The illu gradient is the channel sum of div's "other" gradient in f32 (torch's sum starts from 0),
+// then rounded to T.
+struct GradPx {
+    float gx, ge, gd;
+};
+
+template <typename T, bool kAutocast>
+__device__ __forceinline__ GradPx grad1(float x, float d, float e, float gE, float gR, bool has_gE, bool has_gR)
+{
+    const float r = __fdiv_rn(x, d);
+    const float q = __fdiv_rn(r, d);
+    float g = gR;
+    GradPx o;
+    o.ge = 0.0f;
+    if (has_gE) {
+        const float c = square<T, kAutocast>(e);
+        const float t = -__fmul_rn(gE, c);
+        g = __fadd_rn(has_gR ? __fadd_rn(t, gR) : t, __fmul_rn(gE, e));
+        float gc = __fmul_rn(gE, __fsub_rn(1.0f, r));
+        if (!kAutocast) gc = rnd<T>(gc);
+        const float two_e = kAutocast ? __fmul_rn(2.0f, e) : rnd<T>(__fmul_rn(2.0f, e));
+        o.ge = __fadd_rn(rnd<T>(__fmul_rn(gE, r)), rnd<T>(__fmul_rn(gc, two_e)));
+    }
+    o.gx = __fdiv_rn(g, d);
+    o.gd = __fmul_rn(-g, q);
+    return o;
+}
+
+// Nullable operands: g_enh / g_refl absent = that output got no gradient (g_enh == NULL also when e == NULL, decompose only);
+// g_x / g_illu / g_e NULL = that gradient is not wanted.
+// (kPwThreads, 1): without a minimum-blocks bound ptxas aims at 64 registers and the f32 instantiation spills 12 bytes around
+// the division slow path; it needs 72 (3 CTAs per SM).  The grid stays pw_grid's 148 x 8 CTAs: the later ones start as earlier
+// ones finish and keep more loads in flight; a one-wave grid of 148 x 3 measured slower (32x3x640^2: 0.32 -> 0.35 ms f32,
+// 0.32 -> 0.37 ms fp16; the same at 16x1080p)
+template <typename T, bool kAutocast>
+__global__ void __launch_bounds__(kPwThreads, 1)
+k_recombine_grad_vec(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+                     const float* __restrict__ g_enh, const float* __restrict__ g_refl, float* __restrict__ g_x,
+                     T* __restrict__ g_illu, T* __restrict__ g_e, long long plane4, long long items, float eps)
+{
+    const uint64_t pol = policy_evict_first();
+    const long long stride = (long long)gridDim.x * kPwThreads;
+    const bool has_gE = g_enh != nullptr, has_gR = g_refl != nullptr;
+    const float4 zero = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
+        const long long f = it / plane4, p = it - f * plane4;
+        const long long o3 = (f * 3 * plane4 + p) * 4, o1 = (f * plane4 + p) * 4;
+        const float4 il = MapIO<T>::ld4(illu + o1, pol);
+        const float d[4] = {rnd<T>(__fadd_rn(il.x, eps)), rnd<T>(__fadd_rn(il.y, eps)), rnd<T>(__fadd_rn(il.z, eps)),
+                            rnd<T>(__fadd_rn(il.w, eps))};
+        // one channel at a time: what stays live across the division slow path fits the callee-saved registers (no spills)
+        float gd[4];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const long long o = o3 + c * plane4 * 4;
+            const float4 xv = ld_stream_f4(x + o, pol);
+            const float4 ev = has_gE ? MapIO<T>::ld4(e + o, pol) : zero;
+            const float4 gev = has_gE ? ld_stream_f4(g_enh + o, pol) : zero;
+            const float4 grv = has_gR ? ld_stream_f4(g_refl + o, pol) : zero;
+            const float xs[4] = {xv.x, xv.y, xv.z, xv.w}, es[4] = {ev.x, ev.y, ev.z, ev.w};
+            const float gEs[4] = {gev.x, gev.y, gev.z, gev.w}, gRs[4] = {grv.x, grv.y, grv.z, grv.w};
+            float gx[4], ge[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const GradPx g = grad1<T, kAutocast>(xs[k], d[k], es[k], gEs[k], gRs[k], has_gE, has_gR);
+                gx[k] = g.gx;
+                ge[k] = g.ge;
+                gd[k] = c == 0 ? __fadd_rn(0.0f, g.gd) : __fadd_rn(gd[k], g.gd);
+            }
+            if (g_x) st_stream_f4(g_x + o, make_float4(gx[0], gx[1], gx[2], gx[3]), pol);
+            if (g_e) MapIO<T>::st4(g_e + o, make_float4(ge[0], ge[1], ge[2], ge[3]), pol);
+        }
+        if (g_illu) MapIO<T>::st4(g_illu + o1, make_float4(gd[0], gd[1], gd[2], gd[3]), pol);
+    }
+}
+
+template <typename T, bool kAutocast>
+__global__ void __launch_bounds__(kPwThreads)
+k_recombine_grad_scalar(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+                        const float* __restrict__ g_enh, const float* __restrict__ g_refl, float* __restrict__ g_x,
+                        T* __restrict__ g_illu, T* __restrict__ g_e, long long plane, long long items, float eps)
+{
+    const long long stride = (long long)gridDim.x * kPwThreads;
+    const bool has_gE = g_enh != nullptr, has_gR = g_refl != nullptr;
+    for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
+        const long long f = it / plane, p = it - f * plane;
+        const float d = rnd<T>(__fadd_rn(MapIO<T>::wide(illu[it]), eps));
+        float gd = 0.0f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const long long o = (f * 3 + c) * plane + p;
+            const GradPx g = grad1<T, kAutocast>(x[o], d, has_gE ? MapIO<T>::wide(e[o]) : 0.0f, has_gE ? g_enh[o] : 0.0f,
+                                                 has_gR ? g_refl[o] : 0.0f, has_gE, has_gR);
+            gd = __fadd_rn(gd, g.gd);
+            if (g_x) g_x[o] = g.gx;
+            if (g_e) g_e[o] = MapIO<T>::narrow(g.ge);
+        }
+        if (g_illu) g_illu[it] = MapIO<T>::narrow(gd);
     }
 }
 
@@ -152,19 +324,62 @@ static inline int pw_grid(long long items)
     return int(std::max<long long>(1, std::min<long long>(want, (long long)kNumSMsB200 * kPwCtasPerSm)));
 }
 
-template <bool R, bool E>
-static int recombine_launch(const float* x, const float* illu, const float* e, float* refl, float* enh, int n, int h,
-                            int w, float eps, cudaStream_t s)
+template <typename T> static inline bool aligned4px(const T* p)
+{
+    return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0;
+}
+
+template <typename T, bool AC, bool R, bool E>
+static int recombine_launch(const float* x, const T* illu, const T* e, float* refl, float* enh, int n, int h, int w,
+                            float eps, cudaStream_t s)
 {
     const long long plane = (long long)h * w;
-    const bool vec = plane % 4 == 0 && aligned16(x) && aligned16(illu) && (!E || (aligned16(e) && aligned16(enh))) &&
+    const bool vec = plane % 4 == 0 && aligned16(x) && aligned4px(illu) && (!E || (aligned4px(e) && aligned16(enh))) &&
                      (!R || aligned16(refl));
     if (vec) {
         const long long items = (long long)n * (plane / 4);
-        k_recombine_vec<R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane / 4, items, eps);
+        k_recombine_vec<T, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane / 4, items, eps);
     } else {
         const long long items = (long long)n * plane;
-        k_recombine_scalar<R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane, items, eps);
+        k_recombine_scalar<T, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane, items, eps);
+    }
+    UPR_LAUNCH_CHECK();
+    return UPR_OK;
+}
+
+// upr_retinex_recombine_maps on map type T; the arguments are checked (refl or enh is given; enh only with e).  Without e,
+// or without enh, only R is formed, and the flag is moot.
+template <typename T, bool AC>
+static int recombine_maps(const float* x, const void* illu_v, const void* e_v, float* refl, float* enh, int n, int h,
+                          int w, float eps, cudaStream_t s)
+{
+    const T* illu = static_cast<const T*>(illu_v);
+    const T* e = static_cast<const T*>(e_v);
+    if (!e || !enh) return recombine_launch<T, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps, s);
+    return refl ? recombine_launch<T, AC, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                : recombine_launch<T, AC, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
+}
+
+template <typename T, bool AC>
+static int recombine_grad(const float* x, const void* illu_v, const void* e_v, const float* g_enh, const float* g_refl,
+                          float* g_x, void* g_illu_v, void* g_e_v, int n, int h, int w, float eps, cudaStream_t s)
+{
+    const T* illu = static_cast<const T*>(illu_v);
+    const T* e = static_cast<const T*>(e_v);
+    T* g_illu = static_cast<T*>(g_illu_v);
+    T* g_e = static_cast<T*>(g_e_v);
+    const long long plane = (long long)h * w;
+    const bool vec = plane % 4 == 0 && aligned16(x) && aligned4px(illu) && (!e || aligned4px(e)) &&
+                     (!g_enh || aligned16(g_enh)) && (!g_refl || aligned16(g_refl)) && (!g_x || aligned16(g_x)) &&
+                     (!g_illu || aligned4px(g_illu)) && (!g_e || aligned4px(g_e));
+    if (vec) {
+        const long long items = (long long)n * (plane / 4);
+        k_recombine_grad_vec<T, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e,
+                                                                         plane / 4, items, eps);
+    } else {
+        const long long items = (long long)n * plane;
+        k_recombine_grad_scalar<T, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e,
+                                                                            plane, items, eps);
     }
     UPR_LAUNCH_CHECK();
     return UPR_OK;
@@ -267,8 +482,8 @@ int upr_retinex_recombine_f32(const float* x, const float* illu, const float* e,
     if (n == 0) return UPR_OK;
     if (!x || !illu || !e || !enh) return UPR_E_NULL;
     auto s = static_cast<cudaStream_t>(stream);
-    return refl ? upr::recombine_launch<true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
-                : upr::recombine_launch<false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
+    return refl ? upr::recombine_launch<float, false, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                : upr::recombine_launch<float, false, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
 }
 
 int upr_retinex_decompose_f32(const float* x, const float* illu, float* refl, int n, int h, int w, float eps,
@@ -277,8 +492,50 @@ int upr_retinex_decompose_f32(const float* x, const float* illu, float* refl, in
     if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
     if (n == 0) return UPR_OK;
     if (!x || !illu || !refl) return UPR_E_NULL;
-    return upr::recombine_launch<true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps,
-                                              static_cast<cudaStream_t>(stream));
+    return upr::recombine_launch<float, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps,
+                                                            static_cast<cudaStream_t>(stream));
+}
+
+int upr_retinex_recombine_maps(const float* x, const void* illu, const void* e, int map_dtype, int flags, float* refl,
+                               float* enh, int n, int h, int w, float eps, upr_stream_t stream)
+{
+    if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    if (map_dtype < UPR_DT_F32 || map_dtype > UPR_DT_BF16 || (flags & ~UPR_RETINEX_AUTOCAST)) return UPR_E_PARAM;
+    if (n == 0) return UPR_OK;
+    if (!x || !illu || (!refl && !enh) || (!e && enh)) return UPR_E_NULL;
+    auto s = static_cast<cudaStream_t>(stream);
+    const bool ac = flags & UPR_RETINEX_AUTOCAST;
+    switch (map_dtype) {
+    case UPR_DT_F32: return upr::recombine_maps<float, false>(x, illu, e, refl, enh, n, h, w, eps, s);
+    case UPR_DT_F16:
+        return ac ? upr::recombine_maps<__half, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                  : upr::recombine_maps<__half, false>(x, illu, e, refl, enh, n, h, w, eps, s);
+    default:
+        return ac ? upr::recombine_maps<__nv_bfloat16, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                  : upr::recombine_maps<__nv_bfloat16, false>(x, illu, e, refl, enh, n, h, w, eps, s);
+    }
+}
+
+int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
+                               const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e, int n, int h,
+                               int w, float eps, upr_stream_t stream)
+{
+    if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    if (map_dtype < UPR_DT_F32 || map_dtype > UPR_DT_BF16 || (flags & ~UPR_RETINEX_AUTOCAST)) return UPR_E_PARAM;
+    if (n == 0) return UPR_OK;
+    if (!x || !illu || (!g_enh && !g_refl) || (!e && (g_enh || g_e))) return UPR_E_NULL;
+    if (!g_x && !g_illu && !g_e) return UPR_OK;
+    auto s = static_cast<cudaStream_t>(stream);
+    const bool ac = flags & UPR_RETINEX_AUTOCAST;
+    switch (map_dtype) {
+    case UPR_DT_F32: return upr::recombine_grad<float, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
+    case UPR_DT_F16:
+        return ac ? upr::recombine_grad<__half, true>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s)
+                  : upr::recombine_grad<__half, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
+    default:
+        return ac ? upr::recombine_grad<__nv_bfloat16, true>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s)
+                  : upr::recombine_grad<__nv_bfloat16, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
+    }
 }
 
 int upr_scale_clamp_f32(const float* enh, const float* gain_per_image, float* out, int n, int c, int h, int w,

@@ -7,8 +7,10 @@ What is ON the hot path are the two pointwise Retinex lines around the CNN (refe
 
 Both run in one fused sm_100a kernel (upr_retinex_recombine_f32) at inference (``torch.no_grad()`` / no input requires a
 gradient); the enhance drivers go one step further and hand the two CNN outputs ``forward_maps(x) = (illu, e)`` straight to
-``native.retinex_clahe`` (recombination fused into the CLAHE histogram kernel).  With autograd enabled the same two lines are
-evaluated by stock torch ops so that training back-propagates through them.
+``native.retinex_clahe`` (recombination fused into the CLAHE histogram kernel).  Under autograd (training) they run as one
+``torch.autograd.Function`` on a fused forward and a fused gradient kernel (upr_retinex_recombine_maps / _grad), with the maps
+in f32 or, under autocast, fp16 / bf16; outputs and gradients equal torch autograd through the stock expressions bit for bit.
+Other operands (CPU tensors, mixed map dtypes, other shapes) keep the stock expressions.
 
 The CNN itself (illumination U-Net with residual / pre-activation blocks and an optional ASPP bottleneck, three feature-
 aggregation branches, :11-403) is dense convolution work that cuDNN already covers and is OUT OF SCOPE for hand-written
@@ -35,10 +37,67 @@ EPSILON = 1e-6   # models/model.py:411
 # ---------------------------------------------------------------------------------------------------
 # the two lines on the hot path
 # ---------------------------------------------------------------------------------------------------
+def _fused_autograd(x: torch.Tensor, illu: torch.Tensor, e=None) -> bool:
+    """Whether _RetinexFn takes the operands: CUDA tensors on one device, x [N,3,H,W] f32, illu [N,1,H,W] and e [N,3,H,W]
+    (or None) in one map dtype (f32, fp16, bf16)."""
+    if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and x.shape[1] == 3):
+        return False
+    n, _, h, w = x.shape
+    if illu.device != x.device or illu.dtype not in native.MAP_DTYPES or illu.shape != (n, 1, h, w):
+        return False
+    return e is None or (e.device == x.device and e.dtype == illu.dtype and e.shape == x.shape)
+
+
+def _retinex_grad_ops(x, illu, e, g_refl, g_enh, autocast, need):
+    """The gradient kernel's formulas as differentiable torch ops, for backward(create_graph=True): what autograd computes
+    through the stock expressions, in its accumulation order (include/upretinex_b200.h, upr_retinex_recombine_grad)."""
+    with torch.autocast("cuda", enabled=False):
+        d = illu + EPSILON
+        r = x / d
+        g, ge = g_refl, None
+        if g_enh is not None:
+            ef = e.float() if autocast else e     # autocast evaluates e**2 and its gradient in f32
+            t = -(g_enh * (ef * ef))
+            g = (t if g_refl is None else t + g_refl) + g_enh * e
+            gc = g_enh * (1 - r)
+            if not autocast:
+                gc = gc.to(e.dtype)
+            ge = (g_enh * r).to(e.dtype) + (gc * (2 * ef)).to(e.dtype) if need[2] else None
+        gx = g / d if need[0] else None
+        gi = (-g * ((x / d) / d)).sum(1, keepdim=True).to(illu.dtype) if need[1] else None
+    return gx, gi, ge
+
+
+class _RetinexFn(torch.autograd.Function):
+    """reflectance = x / (illu + 1e-6) and, with e, enhanced = R*e + (1-R)*e**2 on the fused kernels.  Saves only its inputs
+    (the gradient kernel recomputes illu + eps, R and e**2) and forms only the gradients that are needed.  Outputs and
+    gradients equal torch autograd through the stock expressions, also under CUDA autocast (read at forward time)."""
+
+    @staticmethod
+    def forward(ctx, x, illu, e):
+        ctx.set_materialize_grads(False)
+        ctx.autocast = torch.is_autocast_enabled("cuda")
+        refl, enh = native.retinex_recombine_maps(x, illu, e, autocast=ctx.autocast, eps=EPSILON)
+        ctx.save_for_backward(x, illu, e)
+        return refl if e is None else (refl, enh)
+
+    @staticmethod
+    def backward(ctx, g_refl, g_enh=None):
+        x, illu, e = ctx.saved_tensors
+        if g_refl is None and g_enh is None:
+            return None, None, None
+        need = (ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2] and g_enh is not None)
+        if torch.is_grad_enabled():   # backward(create_graph=True): the gradient must itself be differentiable
+            return _retinex_grad_ops(x, illu, e, g_refl, g_enh, ctx.autocast, need)
+        return native.retinex_recombine_grad(x, illu, e, g_enh, g_refl, want=need, autocast=ctx.autocast, eps=EPSILON)
+
+
 def retinex_decompose(x: torch.Tensor, illu: torch.Tensor) -> torch.Tensor:
-    """R = x / (illu + 1e-6).  Inference: the sm_100a kernel (CUDA tensors required -- there is no CPU path).
-    Only when autograd must flow through the line (training) is it left to stock torch ops."""
+    """R = x / (illu + 1e-6).  Inference: the sm_100a kernel (CUDA tensors required -- there is no CPU path).  When autograd
+    must flow through the line (training): _RetinexFn for the operands it takes, the stock torch expression otherwise."""
     if torch.is_grad_enabled() and (x.requires_grad or illu.requires_grad):
+        if _fused_autograd(x, illu):
+            return _RetinexFn.apply(x, illu, None)
         return x / (illu + EPSILON)
     return native.retinex_decompose(x, illu, EPSILON)
 
@@ -46,7 +105,9 @@ def retinex_decompose(x: torch.Tensor, illu: torch.Tensor) -> torch.Tensor:
 def retinex_recombine(x: torch.Tensor, illu: torch.Tensor, enhancement_map: torch.Tensor):
     """(reflectance, enhanced) of models/model.py:412 and :442."""
     needs_grad = torch.is_grad_enabled() and (x.requires_grad or illu.requires_grad or enhancement_map.requires_grad)
-    if needs_grad:   # training: autograd through the two lines, stock torch ops
+    if needs_grad and _fused_autograd(x, illu, enhancement_map):   # training: fused forward + gradient kernels
+        return _RetinexFn.apply(x, illu, enhancement_map)
+    if needs_grad:   # training on other operands: autograd through the stock torch ops
         reflectance = x / (illu + EPSILON)
         return reflectance, reflectance * enhancement_map + (1 - reflectance) * (enhancement_map ** 2)
     return native.retinex_recombine(x, illu, enhancement_map, want_reflectance=True, eps=EPSILON)
@@ -259,7 +320,9 @@ def accelerate_reference_model(model: nn.Module) -> nn.Module:
     checkpoints) through the kernels: ``retinex_decompose`` and ``forward`` take the fused sm_100a path at inference, and the
     instance gains ``forward_maps(x) -> (illu, enhancement_map)`` -- its own ``ie_net`` plus the convolution / fusion / sigmoid
     part of its ``multi_scale_enhance`` (:419-440) -- which is what ``AdaptiveParameterAdjuster.apply_adaptive_enhancement``
-    needs to reach ``upr_retinex_clahe_f32``.  With autograd enabled the instance behaves exactly as before."""
+    needs to reach ``upr_retinex_clahe_f32``.  With autograd enabled (training) ``forward`` and ``retinex_decompose`` run the
+    fused forward and gradient kernels of ``_RetinexFn``, whose outputs and gradients equal the instance's own stock arithmetic
+    bit for bit, and keep that arithmetic for operands the kernels do not take (CPU tensors, mixed map dtypes)."""
     for name in ("ie_net", "scale1", "scale2", "scale3", "fusion", "output_layer"):
         if not hasattr(model, name):
             raise TypeError(f"accelerate_reference_model: not a UP_Retinex-like module (no attribute {name!r})")

@@ -93,6 +93,10 @@ def _declare(lib):
     lib.upr_retinex_recombine_f32.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_decompose_f32.restype = i32
     lib.upr_retinex_decompose_f32.argtypes = [vp, vp, vp, i32, i32, i32, f32, vp]
+    lib.upr_retinex_recombine_maps.restype = i32
+    lib.upr_retinex_recombine_maps.argtypes = [vp, vp, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
+    lib.upr_retinex_recombine_grad.restype = i32
+    lib.upr_retinex_recombine_grad.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_letterbox_f32.restype = i32
     lib.upr_letterbox_f32.argtypes = [vp, vp] + [i32] * 10 + [vp, vp]
     lib.upr_letterbox_u8_f32.restype = i32
@@ -204,14 +208,15 @@ def _dev(device):
     return torch.cuda.device(idx)
 
 
-def _cuda(t: torch.Tensor, name: str, dtype: torch.dtype = torch.float32, shape=None, device=None) -> torch.Tensor:
-    """`t` made contiguous, after checks that cost attribute reads only: RuntimeError off the GPU, TypeError for another dtype,
-    ValueError for another shape (None in `shape` = any size) or for a device other than `device`."""
+def _cuda(t: torch.Tensor, name: str, dtype=torch.float32, shape=None, device=None) -> torch.Tensor:
+    """`t` made contiguous, after checks that cost attribute reads only: RuntimeError off the GPU, TypeError for another dtype
+    (`dtype`: one dtype, or a tuple of the accepted ones), ValueError for another shape (None in `shape` = any size) or for a
+    device other than `device`."""
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor")
     if not t.is_cuda:
         raise RuntimeError(f"{name} must live on a CUDA device (upretinex-b200 has no CPU path)")
-    if t.dtype != dtype:
+    if t.dtype not in (dtype if isinstance(dtype, tuple) else (dtype,)):
         raise TypeError(f"{name} must be {dtype}, got {t.dtype}")
     if shape is not None and (t.dim() != len(shape) or any(s is not None and s != d for s, d in zip(shape, t.shape))):
         raise ValueError(f"{name} must have shape {tuple('*' if s is None else s for s in shape)}, got {tuple(t.shape)}")
@@ -634,6 +639,59 @@ def retinex_decompose(x: torch.Tensor, illu: torch.Tensor, eps: float = 1e-6) ->
     with _dev(x.device):
         _run("upr_retinex_decompose_f32", x.data_ptr(), illu.data_ptr(), refl.data_ptr(), n, h, w, float(eps))
     return refl
+
+
+# storage dtypes of the illumination / enhancement maps that the training entries take (UPR_DT_* of the C ABI)
+MAP_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
+
+def _maps(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor]):
+    """The checked operands of the two training entries: x [N,3,H,W] f32, illu [N,1,H,W] and e [N,3,H,W] (or None) in one map
+    dtype on x's device."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
+    n, _, h, w = x.shape
+    illu = _cuda(illu, "illu", tuple(MAP_DTYPES), shape=(n, 1, h, w), device=x.device)
+    if e is not None:
+        e = _cuda(e, "e", illu.dtype, shape=x.shape, device=x.device)
+    return x, illu, e
+
+
+def retinex_recombine_maps(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], autocast: bool = False,
+                           want_reflectance: bool = True, eps: float = 1e-6):
+    """(reflectance | None, enhanced | None) of models/model.py:412 and :442 with the maps illu [N,1,H,W] and e [N,3,H,W] in
+    f32, fp16 or bf16 (upr_retinex_recombine_maps), equal to torch eager on the same operands; e None = decompose only.
+    autocast: e**2 as CUDA autocast evaluates it (in f32) instead of in the maps' dtype."""
+    x, illu, e = _maps(x, illu, e)
+    n, _, h, w = x.shape
+    refl = torch.empty_like(x) if want_reflectance or e is None else None
+    enh = torch.empty_like(x) if e is not None else None
+    with _dev(x.device):
+        _run("upr_retinex_recombine_maps", x.data_ptr(), illu.data_ptr(), e.data_ptr() if e is not None else None,
+             MAP_DTYPES[illu.dtype], int(bool(autocast)), refl.data_ptr() if refl is not None else None,
+             enh.data_ptr() if enh is not None else None, n, h, w, float(eps))
+    return refl, enh
+
+
+def retinex_recombine_grad(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], g_enh: Optional[torch.Tensor],
+                           g_refl: Optional[torch.Tensor], want=(True, True, True), autocast: bool = False, eps: float = 1e-6):
+    """(grad x | None, grad illu | None, grad e | None) -- what torch autograd back-propagates through
+    retinex_recombine_maps(x, illu, e, autocast) from the upstream gradients g_enh and g_refl (f32, either None) in one pass
+    (upr_retinex_recombine_grad).  want: which of the three to form; grad illu and grad e have the maps' dtype."""
+    x, illu, e = _maps(x, illu, e)
+    n, _, h, w = x.shape
+    g_enh = _cuda(g_enh, "g_enh", shape=x.shape, device=x.device) if g_enh is not None else None
+    g_refl = _cuda(g_refl, "g_refl", shape=x.shape, device=x.device) if g_refl is not None else None
+    gx = torch.empty_like(x) if want[0] else None
+    gi = torch.empty_like(illu) if want[1] else None
+    ge = torch.empty_like(e) if want[2] and e is not None else None
+
+    def ptr(t):
+        return t.data_ptr() if t is not None else None
+
+    with _dev(x.device):
+        _run("upr_retinex_recombine_grad", x.data_ptr(), illu.data_ptr(), ptr(e), MAP_DTYPES[illu.dtype], int(bool(autocast)),
+             ptr(g_enh), ptr(g_refl), ptr(gx), ptr(gi), ptr(ge), n, h, w, float(eps))
+    return gx, gi, ge
 
 
 # ------------------------------------------------------------------------------------------------
