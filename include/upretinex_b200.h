@@ -86,12 +86,10 @@ UPR_API int upr_retinex_clahe_f32(const float* x_nchw, const float* illu_n1hw, c
                                   void* workspace, size_t workspace_bytes, upr_stream_t stream);
 /* Same, writing the packed u8 RGB (HWC) frame that save_image (enhancers/simple_enhance.py:65-100) would store: what the
  * batch driver sends back over PCIe (3 instead of 12 bytes per pixel).  Bit-identical to upr_retinex_clahe_f32 followed by
- * the truncating cast.  Ragged shapes (no vector path) need `enhanced_scratch`, an f32 [n][3][h][w] frame for the
- * recombination; with a NULL scratch they return UPR_E_WORKSPACE. */
+ * the truncating cast. */
 UPR_API int upr_retinex_clahe_f32_u8(const float* x_nchw, const float* illu_n1hw, const float* e_nchw,
-                                     unsigned char* out_nhwc_rgb, float* enhanced_scratch, int n, int h, int w, float eps,
-                                     double clip_limit, int tiles_x, int tiles_y, void* workspace, size_t workspace_bytes,
-                                     upr_stream_t stream);
+                                     unsigned char* out_nhwc_rgb, int n, int h, int w, float eps, double clip_limit,
+                                     int tiles_x, int tiles_y, void* workspace, size_t workspace_bytes, upr_stream_t stream);
 /* Profiling hook: runs only the selected stages of upr_clahe_lab_f32 on a workspace that a full call has
  * already populated.  stage_mask bit 0 = K1 (quantise + Lab + tile histograms + clip/LUT), bit 1 = K3
  * (bilinear LUT map + Lab->RGB); bench.py uses it to time each kernel with CUDA events. */

@@ -655,6 +655,8 @@ k_hist_lab_vec3(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t*
 // K1 generic path: any size (including OpenCV's reflect-101 padding quirk, Appendix A.3 step 1).
 // One CTA per (frame, tile); per-warp shared histograms with atomics.  Correctness path for
 // ragged shapes -- the named workloads all take the vector path.
+//   kFused: as in k_hist_lab_vec3, the input is the Retinex recombination of x, illu and e, evaluated per (reflected)
+//           pixel with recombine_px.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ int reflect101(int p, int len)
 {
@@ -663,11 +665,12 @@ __device__ __forceinline__ int reflect101(int p, int len)
     return p;
 }
 
-template <bool kU8In>
+template <bool kU8In, bool kFused>
 __global__ void __launch_bounds__(256)
 k_hist_lab_generic(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t* __restrict__ hist_g,
-                   uint8_t* __restrict__ lut_g, const ClaheGeom g)
+                   uint8_t* __restrict__ lut_g, const ClaheGeom g, const RetinexIn rx)
 {
+    static_assert(!(kU8In && kFused), "the fused Retinex prologue reads f32 planes");
     __shared__ int s_hist[8][256];
     __shared__ uint16_t s_gamma[UPR_TAB_GAMMA_LEN];
     __shared__ uint16_t s_cbrt[UPR_TAB_CBRT_LEN];
@@ -696,6 +699,14 @@ k_hist_lab_generic(const void* __restrict__ in, uint8_t* __restrict__ lab, int32
         int qr, qg, qb;
         if constexpr (kU8In) {
             qr = in8[3 * off + 0]; qg = in8[3 * off + 1]; qb = in8[3 * off + 2];
+        } else if constexpr (kFused) {
+            const float* eR = rx.e + size_t(f) * 3 * plane;
+            const float d = __fadd_rn(ld_stream_f1(rx.illu + size_t(f) * plane + off, pol_stream), rx.eps);
+            float refl, o[3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c)
+                recombine_px(ld_stream_f1(inR + c * plane + off, pol_stream), d, ld_stream_f1(eR + c * plane + off, pol_stream), refl, o[c]);
+            qr = quantize_u8(o[0]); qg = quantize_u8(o[1]); qb = quantize_u8(o[2]);
         } else {
             qr = quantize_u8(ld_stream_f1(inR + off, pol_stream));
             qg = quantize_u8(ld_stream_f1(inR + plane + off, pol_stream));
@@ -1053,8 +1064,6 @@ static inline int raw_tile(int p, float inv)
 }
 
 // stage_mask: bit 0 = K1 (Lab + histograms + LUTs), bit 1 = K3 (map); 3 = the whole op
-constexpr int kNeedUnfused = -100;   // internal: the fused Retinex prologue exists on the vector path only
-
 // in_u8 / out_u8: the frame on that side is packed u8 RGB (HWC) instead of planar f32 (NCHW)
 static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double clip_limit, int tiles_x, int tiles_y,
                      void* ws, size_t ws_bytes, cudaStream_t stream, int stage_mask = 3, const RetinexIn* rx = nullptr,
@@ -1137,13 +1146,13 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
         }
     }
 
-    if (rx && !fast) return kNeedUnfused;
     const int ntiles = tiles_x * tiles_y;
     // a frame index rides in gridDim.y (<= 65535): run long batches in slices
     for (int f0 = 0; f0 < n; f0 += 65535) {
         const int nf = std::min(n - f0, 65535);
         const size_t fplane = size_t(f0) * 3 * h * w;
         const size_t ftile = size_t(f0) * ntiles;
+        const RetinexIn rxf = rx ? RetinexIn{rx->illu + size_t(f0) * h * w, rx->e + fplane, rx->eps} : RetinexIn{nullptr, nullptr, 0.0f};
         if (fast) {
             // K1: byte counters allow <= 255 pixels per thread between flushes -> <= 63 items/thread
             const int tw4 = g.tw / 4;
@@ -1170,7 +1179,6 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
             const size_t smem1 = size_t(256) * kK1Threads + UPR_TAB_GAMMA_LEN * 4 + UPR_TAB_CBRT_LEN * 2;
             if (stage_mask & 1) {
                 const dim3 grid1(ntiles * g.nstrips, nf);
-                const RetinexIn rxf = rx ? RetinexIn{rx->illu + size_t(f0) * h * w, rx->e + fplane, rx->eps} : RetinexIn{nullptr, nullptr, 0.0f};
                 if (in_u8) {
                     UPR_CUDA_TRY(ensure_dynamic_smem(k_hist_lab_vec3<true, false>, smem1, g_smem_mask[0]));
                     k_hist_lab_vec3<true, false><<<grid1, kK1Threads, smem1, stream>>>(
@@ -1222,8 +1230,10 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
             g.nstrips = 1; g.strip_rows = g.th;
             if (stage_mask & 1) {
                 const void* inf = static_cast<const char*>(in_v) + fplane * in_es;
-                if (in_u8) k_hist_lab_generic<true><<<dim3(ntiles, nf), 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g);
-                else k_hist_lab_generic<false><<<dim3(ntiles, nf), 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g);
+                const dim3 grid1(ntiles, nf);
+                if (in_u8) k_hist_lab_generic<true, false><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
+                else if (rx) k_hist_lab_generic<false, true><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
+                else k_hist_lab_generic<false, false><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
                 UPR_LAUNCH_CHECK();
             }
             const size_t plane = size_t(h) * w;
@@ -1265,31 +1275,18 @@ int upr_retinex_clahe_f32(const float* x, const float* illu, const float* e, flo
 {
     if (!x || !illu || !e) return (n == 0 && upr::valid_shape(n, h, w, tiles_x, tiles_y)) ? UPR_OK : UPR_E_NULL;
     const upr::RetinexIn rx{illu, e, eps};
-    int rc = upr::clahe_run(x, out_nchw, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
-                            static_cast<cudaStream_t>(stream), 3, &rx);
-    if (rc != upr::kNeedUnfused) return rc;
-    // ragged shapes: the two ops back to back (recombination into `out`, CLAHE in place) -- same results
-    rc = upr_retinex_recombine_f32(x, illu, e, nullptr, out_nchw, n, h, w, eps, stream);
-    if (rc) return rc;
-    return upr::clahe_run(out_nchw, out_nchw, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
-                          static_cast<cudaStream_t>(stream));
+    return upr::clahe_run(x, out_nchw, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
+                          static_cast<cudaStream_t>(stream), 3, &rx);
 }
 
-int upr_retinex_clahe_f32_u8(const float* x, const float* illu, const float* e, unsigned char* out_nhwc, float* enhanced_scratch,
-                             int n, int h, int w, float eps, double clip_limit, int tiles_x, int tiles_y, void* workspace,
-                             size_t workspace_bytes, upr_stream_t stream)
+int upr_retinex_clahe_f32_u8(const float* x, const float* illu, const float* e, unsigned char* out_nhwc, int n, int h, int w,
+                             float eps, double clip_limit, int tiles_x, int tiles_y, void* workspace, size_t workspace_bytes,
+                             upr_stream_t stream)
 {
     if (!x || !illu || !e) return (n == 0 && upr::valid_shape(n, h, w, tiles_x, tiles_y)) ? UPR_OK : UPR_E_NULL;
     const upr::RetinexIn rx{illu, e, eps};
-    int rc = upr::clahe_run(x, out_nhwc, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
-                            static_cast<cudaStream_t>(stream), 3, &rx, false, true);
-    if (rc != upr::kNeedUnfused) return rc;
-    // ragged shapes: recombination into the caller's scratch frame, then CLAHE f32 -> u8
-    if (!enhanced_scratch) return UPR_E_WORKSPACE;
-    rc = upr_retinex_recombine_f32(x, illu, e, nullptr, enhanced_scratch, n, h, w, eps, stream);
-    if (rc) return rc;
-    return upr::clahe_run(enhanced_scratch, out_nhwc, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
-                          static_cast<cudaStream_t>(stream), 3, nullptr, false, true);
+    return upr::clahe_run(x, out_nhwc, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
+                          static_cast<cudaStream_t>(stream), 3, &rx, false, true);
 }
 
 int upr_clahe_lab_u8(const unsigned char* in_nhwc, unsigned char* out_nhwc, int n, int h, int w, double clip_limit, int tiles_x,

@@ -1,6 +1,7 @@
 // upr_common.cuh -- shared device/host helpers for the sm_100a kernels.
 #pragma once
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <mutex>
 #include <atomic>
 #include <cstdint>
@@ -39,15 +40,44 @@ SidePool* side_pool();          // nullptr when the streams cannot be created (t
 // frames per chunk of the chunked schedules (~25 Mpx: 3 x 4K, 12 x 1080p)
 inline int chunk_frames(long long plane) { return int(plane >= 25000000LL ? 1 : 25000000LL / plane); }
 
+// The chunked two-stream schedule: launch(f0, nf, stream) enqueues the work of frames [f0, f0 + nf).  With at least two chunks
+// of `chunk` frames and a side pool, consecutive chunks go to the two side streams, which fork from s and join back into it
+// (graph-capturable); otherwise one launch(0, n, s).  Stops at the first failed launch and returns its status.
+template <typename Launch>
+int run_chunked(cudaStream_t s, int n, int chunk, Launch&& launch)
+{
+    if (n >= 2 * chunk) {
+        std::lock_guard<std::mutex> guard(side_pool_mutex());
+        if (SidePool* pool = side_pool()) {
+            UPR_CUDA_TRY(cudaEventRecord(pool->fork, s));
+            for (int i = 0; i < 2; ++i) UPR_CUDA_TRY(cudaStreamWaitEvent(pool->s[i], pool->fork, 0));
+            int rc = UPR_OK;
+            for (int f0 = 0, k = 0; f0 < n && rc == UPR_OK; f0 += chunk, ++k)
+                rc = launch(f0, std::min(chunk, n - f0), pool->s[k & 1]);
+            for (int i = 0; i < 2; ++i) {      // always join, also after a failed launch: the caller's stream must not run ahead
+                UPR_CUDA_TRY(cudaEventRecord(pool->join[i], pool->s[i]));
+                UPR_CUDA_TRY(cudaStreamWaitEvent(s, pool->join[i], 0));
+            }
+            return rc;
+        }
+    }
+    return launch(0, n, s);
+}
+
 // upr_pointwise.cu: out = clamp(enh * gain[frame], 0, 1) on stream s (the kernel behind upr_scale_clamp_f32)
 int scale_clamp_launch(const float* enh, const float* gain, float* out, int n, int c, int h, int w, cudaStream_t s);
 
-// upr_multiscale.cu: launches the streaming statistics kernel for frames [f0, f0 + nf) of a batch of n_total frames on stream s
-// (x, means3, gain already point at frame f0; the workspace is the whole batch's).  Returns UPR_OK, an error, or
-// kMsNotStreamable when the shape needs the generic multi-kernel path (the caller then runs upr_multiscale_stats_f32 itself).
-constexpr int kMsNotStreamable = 1000001;
-int ms_stream_launch_range(const float* x, int nf, int h, int w, void* ms_ws, size_t ms_ws_bytes, int n_total, int f0,
-                           float* means3, float* gain, cudaStream_t s);
+// upr_multiscale.cu: the streaming statistics kernel.  ms_stream_geometry decides once per call whether it serves h x w frames
+// at x (h, w multiples of 4 and at least 8, x 16-byte aligned, at most kMsMaxParts row segments x column bands per frame) and
+// fills in its band count and segment height; false means the generic multi-kernel path (upr_multiscale_stats_f32).
+// ms_stream_launch_range launches it with that geometry for frames [f0, f0 + nf) of a batch of n_total frames on stream s
+// (x, means3, gain already point at frame f0; the workspace is the whole batch's).
+struct MsStreamGeom {
+    int bands, seg_rows;
+};
+bool ms_stream_geometry(int h, int w, const float* x, MsStreamGeom* geo);
+int ms_stream_launch_range(const float* x, int nf, int h, int w, const MsStreamGeom& geo, void* ms_ws, size_t ms_ws_bytes,
+                           int n_total, int f0, float* means3, float* gain, cudaStream_t s);
 
 __host__ __device__ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }

@@ -455,17 +455,9 @@ static int ms_parts(int n, long long px)
     return int(std::max<long long>(1, std::min<long long>(std::min(by_work, by_fill), kMsMaxParts)));
 }
 
-int ms_stream_launch_range(const float* x, int nf, int h, int w, void* ms_ws, size_t ms_ws_bytes, int n_total, int f0,
-                           float* means3, float* gain, cudaStream_t s)
+bool ms_stream_geometry(int h, int w, const float* x, MsStreamGeom* geo)
 {
-    if (nf <= 0 || f0 < 0 || f0 + nf > n_total || n_total > 65535 || h <= 0 || w <= 0) return UPR_E_SHAPE;
-    if (!(h % 4 == 0 && w % 4 == 0 && h / 4 >= 2 && w / 4 >= 2 && aligned16(x))) return kMsNotStreamable;
-    if (!x || !ms_ws || !means3 || !gain) return UPR_E_NULL;
-    const MsLayout lay = ms_layout(n_total, h, w);
-    if (ms_ws_bytes < lay.total || (reinterpret_cast<uintptr_t>(ms_ws) & 255u)) return UPR_E_WORKSPACE;
-    auto* base = static_cast<unsigned char*>(ms_ws);
-    auto* partial = reinterpret_cast<double*>(base + lay.off_partial) + size_t(f0) * kMsMaxParts * 3;
-    auto* tickets = reinterpret_cast<unsigned*>(base + lay.off_tickets) + f0;
+    if (!(h % 4 == 0 && w % 4 == 0 && h / 4 >= 2 && w / 4 >= 2 && aligned16(x))) return false;
     // one warp per (band, row segment, frame)
     const int bands = (w + kMsBandCols - 1) / kMsBandCols;
     // 64-row segments whatever the batch: odd segments walk upwards, and the direction of a row must not depend on nf
@@ -473,9 +465,23 @@ int ms_stream_launch_range(const float* x, int nf, int h, int w, void* ms_ws, si
     int seg_rows = 64;
     // (very wide frames: longer segments keep the per-frame partial count inside the workspace)
     while ((long long)bands * ((h + seg_rows - 1) / seg_rows) > kMsMaxParts && seg_rows < h) seg_rows *= 2;
-    const int segs = (h + seg_rows - 1) / seg_rows;
-    if ((long long)bands * segs > kMsMaxParts) return kMsNotStreamable;
-    k_ms_stream<<<dim3(bands * segs, nf), 32, 0, s>>>(x, h, w, bands, seg_rows, partial, tickets, means3, gain);
+    if ((long long)bands * ((h + seg_rows - 1) / seg_rows) > kMsMaxParts) return false;
+    *geo = MsStreamGeom{bands, seg_rows};
+    return true;
+}
+
+int ms_stream_launch_range(const float* x, int nf, int h, int w, const MsStreamGeom& geo, void* ms_ws, size_t ms_ws_bytes,
+                           int n_total, int f0, float* means3, float* gain, cudaStream_t s)
+{
+    if (nf <= 0 || f0 < 0 || f0 + nf > n_total || n_total > 65535 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    if (!x || !ms_ws || !means3 || !gain) return UPR_E_NULL;
+    const MsLayout lay = ms_layout(n_total, h, w);
+    if (ms_ws_bytes < lay.total || (reinterpret_cast<uintptr_t>(ms_ws) & 255u)) return UPR_E_WORKSPACE;
+    auto* base = static_cast<unsigned char*>(ms_ws);
+    auto* partial = reinterpret_cast<double*>(base + lay.off_partial) + size_t(f0) * kMsMaxParts * 3;
+    auto* tickets = reinterpret_cast<unsigned*>(base + lay.off_tickets) + f0;
+    const int segs = (h + geo.seg_rows - 1) / geo.seg_rows;
+    k_ms_stream<<<dim3(geo.bands * segs, nf), 32, 0, s>>>(x, h, w, geo.bands, geo.seg_rows, partial, tickets, means3, gain);
     UPR_LAUNCH_CHECK();
     return UPR_OK;
 }
@@ -498,10 +504,9 @@ static int ms_run(const float* x, int n, int h, int w, float* means, float* gain
     if (want_feat && !(f1 && f2 && f3)) return UPR_E_NULL;
     if (!want_feat && (!means || !gain)) return UPR_E_NULL;
 
-    if (allow_fused && !want_feat) {
-        const int rc = ms_stream_launch_range(x, n, h, w, ws, ws_bytes, n, 0, means, gain, s);
-        if (rc != kMsNotStreamable) return rc;
-    }
+    MsStreamGeom geo{};
+    if (allow_fused && !want_feat && ms_stream_geometry(h, w, x, &geo))
+        return ms_stream_launch_range(x, n, h, w, geo, ws, ws_bytes, n, 0, means, gain, s);
     // generic: down-sample, then one feature kernel per scale
     {
         const long long t2 = (long long)n * 3 * lay.oh2 * lay.ow2, t4 = (long long)n * 3 * lay.oh4 * lay.ow4;
@@ -569,34 +574,22 @@ int upr_multiscale_enhance_f32(const float* x_nchw, const float* enh_nchw, float
     if (n == 0) return UPR_OK;
     if (!x_nchw || !enh_nchw || !out_nchw || !means_n_by_3 || !gain_per_image || !workspace) return UPR_E_NULL;
     auto s = static_cast<cudaStream_t>(stream);
-    const long long plane = (long long)h * w;
-    const int chunk = chunk_frames(plane);
+    MsStreamGeom geo{};
+    if (!ms_stream_geometry(h, w, x_nchw, &geo)) {
+        const int rc = upr_multiscale_stats_f32(x_nchw, n, h, w, means_n_by_3, gain_per_image, workspace, workspace_bytes, 0, stream);
+        if (rc) return rc;
+        return scale_clamp_launch(enh_nchw, gain_per_image, out_nchw, n, 3, h, w, s);
+    }
     // Chunks of ~25 Mpx, statistics then gain pass of a chunk on one of two side streams: the latency-bound statistics kernel of
     // chunk i + 1 runs under the bandwidth-bound gain pass of chunk i (16 x 4K: 0.82 ms back to back -> 0.79 ms; the frames are
     // independent, so the results do not depend on the schedule).
-    if (n >= 2 * chunk && h % 4 == 0 && w % 4 == 0 && h / 4 >= 2 && w / 4 >= 2 && aligned16(x_nchw)) {
-        std::lock_guard<std::mutex> guard(side_pool_mutex());
-        if (SidePool* pool = side_pool()) {
-            UPR_CUDA_TRY(cudaEventRecord(pool->fork, s));
-            for (int i = 0; i < 2; ++i) UPR_CUDA_TRY(cudaStreamWaitEvent(pool->s[i], pool->fork, 0));
-            int rc = UPR_OK;
-            for (int f0 = 0, k = 0; f0 < n && rc == UPR_OK; f0 += chunk, ++k) {
-                const int nf = std::min(chunk, n - f0);
-                rc = ms_stream_launch_range(x_nchw + f0 * 3 * plane, nf, h, w, workspace, workspace_bytes, n, f0, means_n_by_3 + 3 * f0,
-                                            gain_per_image + f0, pool->s[k & 1]);
-                if (rc == UPR_OK)
-                    rc = scale_clamp_launch(enh_nchw + f0 * 3 * plane, gain_per_image + f0, out_nchw + f0 * 3 * plane, nf, 3, h, w, pool->s[k & 1]);
-            }
-            for (int i = 0; i < 2; ++i) {      // always join, also after a failed launch: the caller's stream must not run ahead
-                UPR_CUDA_TRY(cudaEventRecord(pool->join[i], pool->s[i]));
-                UPR_CUDA_TRY(cudaStreamWaitEvent(s, pool->join[i], 0));
-            }
-            if (rc != kMsNotStreamable) return rc;
-        }
-    }
-    const int rc = upr_multiscale_stats_f32(x_nchw, n, h, w, means_n_by_3, gain_per_image, workspace, workspace_bytes, 0, stream);
-    if (rc) return rc;
-    return scale_clamp_launch(enh_nchw, gain_per_image, out_nchw, n, 3, h, w, s);
+    const long long plane = (long long)h * w;
+    return run_chunked(s, n, chunk_frames(plane), [&](int f0, int nf, cudaStream_t cs) {
+        const int rc = ms_stream_launch_range(x_nchw + f0 * 3 * plane, nf, h, w, geo, workspace, workspace_bytes, n, f0,
+                                              means_n_by_3 + 3 * f0, gain_per_image + f0, cs);
+        if (rc) return rc;
+        return scale_clamp_launch(enh_nchw + f0 * 3 * plane, gain_per_image + f0, out_nchw + f0 * 3 * plane, nf, 3, h, w, cs);
+    });
 }
 
 }  // extern "C"

@@ -865,6 +865,7 @@ static int sal_launch(int mode, const float* x, int n, int h, int w, float* out,
 // chunk runs on the chunk's stream ahead of its blur kernel, so its issue-bound pass overlaps the memory-bound passes of the
 // neighbouring chunk instead of running alone over the whole batch first.
 struct MsJob {
+    MsStreamGeom geo;
     void* ws;
     size_t ws_bytes;
     float* means3;      // [n][3]
@@ -894,36 +895,19 @@ static int sal_run(int mode, const float* x, int n, int h, int w, float* out, vo
     // alternating streams.  The 4-8 B/px intermediate of a chunk (~100-200 MB) is then re-read while part of it is still in L2, and
     // the passes of neighbouring chunks overlap.  Measured on 16 x 4K / 64 x 1080p: 1.39 -> 1.28-1.30 ms (profiles/r4_content_aware.md;
     // single-frame chunks lose more to short kernels than they gain).  Results do not depend on the schedule: every frame is
-    // normalised on its own.
-    const int chunk = chunk_frames(plane);
+    // normalised on its own.  An in-place apply (!lum_ok) runs as one chunk.
+    const int chunk = (mode != 2 || lum_ok) ? chunk_frames(plane) : n;
     const long long step_x = 3 * plane, step_p = plane;
-    if (n >= 2 * chunk && (mode != 2 || lum_ok)) {
-        std::lock_guard<std::mutex> guard(side_pool_mutex());
-        if (SidePool* pool = side_pool()) {
-            UPR_CUDA_TRY(cudaEventRecord(pool->fork, s));
-            for (int i = 0; i < 2; ++i) UPR_CUDA_TRY(cudaStreamWaitEvent(pool->s[i], pool->fork, 0));
-            int rc = UPR_OK;
-            for (int f0 = 0, k = 0; f0 < n && rc == UPR_OK; f0 += chunk, ++k) {
-                const int nf = std::min(chunk, n - f0);
-                if (ms) rc = ms_stream_launch_range(x + f0 * step_x, nf, h, w, ms->ws, ms->ws_bytes, n, f0, ms->means3 + 3 * f0, ms->gain + f0,
-                                                    pool->s[k & 1]);
-                if (rc != UPR_OK) break;
-                rc = sal_launch(mode, x + f0 * step_x, nf, h, w, out + f0 * (mode == 2 ? step_x : step_p), mm + f0, blur + f0 * step_p,
-                                pool->s[k & 1], enh ? enh + f0 * step_x : nullptr, att_out ? att_out + f0 * step_p : nullptr,
-                                ms_gain ? ms_gain + f0 : nullptr, lum_ok);
-            }
-            for (int i = 0; i < 2; ++i) {      // always join, also after a failed launch: the caller's stream must not run ahead
-                UPR_CUDA_TRY(cudaEventRecord(pool->join[i], pool->s[i]));
-                UPR_CUDA_TRY(cudaStreamWaitEvent(s, pool->join[i], 0));
-            }
-            return rc;
+    return run_chunked(s, n, chunk, [&](int f0, int nf, cudaStream_t cs) {
+        if (ms) {
+            const int rc = ms_stream_launch_range(x + f0 * step_x, nf, h, w, ms->geo, ms->ws, ms->ws_bytes, n, f0, ms->means3 + 3 * f0,
+                                                  ms->gain + f0, cs);
+            if (rc != UPR_OK) return rc;
         }
-    }
-    if (ms) {
-        const int rc = ms_stream_launch_range(x, n, h, w, ms->ws, ms->ws_bytes, n, 0, ms->means3, ms->gain, s);
-        if (rc != UPR_OK) return rc;
-    }
-    return sal_launch(mode, x, n, h, w, out, mm, blur, s, enh, att_out, ms_gain, lum_ok);
+        return sal_launch(mode, x + f0 * step_x, nf, h, w, out + f0 * (mode == 2 ? step_x : step_p), mm + f0, blur + f0 * step_p, cs,
+                          enh ? enh + f0 * step_x : nullptr, att_out ? att_out + f0 * step_p : nullptr, ms_gain ? ms_gain + f0 : nullptr,
+                          lum_ok);
+    });
 }
 
 }  // namespace upr
@@ -961,18 +945,15 @@ int upr_content_multiscale_f32(const float* x_nchw, const float* enh_nchw, float
 {
     if (n > 0 && (!means_n_by_3 || !gain_per_image || !ms_workspace)) return UPR_E_NULL;
     auto s = static_cast<cudaStream_t>(stream);
+    upr::MsStreamGeom geo{};
     // shapes the streaming statistics kernel does not serve: the generic statistics path over the whole batch first
-    if (n > 0 && !(h % 4 == 0 && w % 4 == 0 && h / 4 >= 2 && w / 4 >= 2 && upr::aligned16(x_nchw))) {
+    if (n > 0 && !upr::ms_stream_geometry(h, w, x_nchw, &geo)) {
         const int rc = upr_multiscale_stats_f32(x_nchw, n, h, w, means_n_by_3, gain_per_image, ms_workspace, ms_workspace_bytes, 0, stream);
         if (rc) return rc;
         return upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, s, enh_nchw, att_n1hw, gain_per_image);
     }
-    const upr::MsJob job{ms_workspace, ms_workspace_bytes, means_n_by_3, gain_per_image};
-    const int rc = upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, s, enh_nchw, att_n1hw, gain_per_image, &job);
-    if (rc != upr::kMsNotStreamable) return rc;
-    const int rc2 = upr_multiscale_stats_f32(x_nchw, n, h, w, means_n_by_3, gain_per_image, ms_workspace, ms_workspace_bytes, 0, stream);
-    if (rc2) return rc2;
-    return upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, s, enh_nchw, att_n1hw, gain_per_image);
+    const upr::MsJob job{geo, ms_workspace, ms_workspace_bytes, means_n_by_3, gain_per_image};
+    return upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, s, enh_nchw, att_n1hw, gain_per_image, &job);
 }
 
 int upr_content_multiscale_apply_f32(const float* x_nchw, const float* enh_nchw, const float* ms_gain_per_image, float* out_nchw,

@@ -46,7 +46,7 @@ def _declare(lib):
     lib.upr_retinex_clahe_f32.restype = i32
     lib.upr_retinex_clahe_f32.argtypes = [vp, vp, vp, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
     lib.upr_retinex_clahe_f32_u8.restype = i32
-    lib.upr_retinex_clahe_f32_u8.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
+    lib.upr_retinex_clahe_f32_u8.argtypes = [vp, vp, vp, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
     lib.upr_clahe_lab_stages_f32.restype = i32
     lib.upr_clahe_lab_stages_f32.argtypes = [vp, vp, i32, i32, i32, f64, i32, i32, vp, sz, i32, vp]
     lib.upr_clahe_debug_dump.restype = i32
@@ -312,17 +312,8 @@ def _clahe(entry: str, x: torch.Tensor, clip_limit: float, tiles: Tuple[int, int
         tail = (float(clip_limit), tx, ty, ws.data_ptr(), ws.numel(), *extra)
         if retinex is None:
             _run(entry, x.data_ptr(), out.data_ptr(), n, h, w, *tail)
-        elif not u8_out:
-            _run(entry, x.data_ptr(), illu.data_ptr(), e.data_ptr(), out.data_ptr(), n, h, w, float(eps), *tail)
         else:
-            fn = getattr(lib(), entry)
-            ptrs = (x.data_ptr(), illu.data_ptr(), e.data_ptr(), out.data_ptr())
-            args = (n, h, w, float(eps), *tail, _stream())
-            rc = fn(*ptrs, None, *args)
-            if rc == -3:   # ragged shape: the recombination needs a scratch frame
-                scratch = torch.empty_like(x)
-                rc = fn(*ptrs, scratch.data_ptr(), *args)
-            check(rc, entry)
+            _run(entry, x.data_ptr(), illu.data_ptr(), e.data_ptr(), out.data_ptr(), n, h, w, float(eps), *tail)
     return out
 
 

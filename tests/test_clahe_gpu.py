@@ -159,8 +159,8 @@ def test_persistent_map_kernel_shapes(native, n, h, w, tiles):
 @pytest.mark.parametrize("n,h,w,tiles", [(2, 1080, 1920, (8, 8)), (3, 400, 600, (8, 8)), (1, 403, 601, (8, 8)), (2, 64, 96, (4, 2)),
                                           (1, 2160, 3840, (8, 8))])
 def test_retinex_clahe_fused_equals_composition(native, n, h, w, tiles):
-    """upr_retinex_clahe_f32 == upr_retinex_recombine_f32 -> upr_clahe_lab_f32, bit for bit (vector path, ragged fallback),
-    and == the oracle's recombination + CLAHE on a small case."""
+    """upr_retinex_clahe_f32 == upr_retinex_recombine_f32 -> upr_clahe_lab_f32, bit for bit (vector path; generic path on ragged
+    shapes), also in place (out = x), and == the oracle's recombination + CLAHE on a small case."""
     rng = np.random.default_rng(h + w)
     x = np.concatenate([O.kat_input(800 + i, h, w, ("dark", "uniform")[i % 2]) for i in range(n)])
     e = rng.random((n, 3, h, w), dtype=np.float32)
@@ -170,6 +170,9 @@ def test_retinex_clahe_fused_equals_composition(native, n, h, w, tiles):
     ref = native.clahe_lab(enh, 2.0, tiles)
     got = native.retinex_clahe(xd, id_, ed, 2.0, tiles)
     assert torch.equal(got, ref)
+    inplace = xd.clone()
+    native.retinex_clahe(inplace, id_, ed, 2.0, tiles, out=inplace)
+    assert torch.equal(inplace, ref)
     if h * w <= 400 * 600:
         _, e_ref = O.retinex_recombine(x[:1], illu[:1], e[:1])
         assert np.array_equal(got[:1].cpu().numpy(), O.clahe_lab(e_ref, 2.0, tiles))
@@ -199,8 +202,8 @@ def test_column_passes_and_partial_occupancy(native, n, h, w, tiles):
 
 
 def test_retinex_clahe_u8_output(native):
-    """upr_retinex_clahe_f32_u8 == upr_retinex_clahe_f32 followed by save_image's truncating cast (vector path; ragged shapes
-    through the caller's scratch frame)."""
+    """upr_retinex_clahe_f32_u8 == upr_retinex_clahe_f32 followed by save_image's truncating cast (vector path; generic path on
+    ragged shapes)."""
     rng = np.random.default_rng(77)
     for n, h, w in ((2, 1080, 1920), (3, 400, 600), (1, 403, 601)):
         x = np.concatenate([O.kat_input(840 + i, h, w, ("dark", "uniform")[i % 2]) for i in range(n)])
@@ -210,6 +213,31 @@ def test_retinex_clahe_u8_output(native):
         ref = native.retinex_clahe(xd, id_, ed)
         want = (ref.clamp(0, 1) * 255).to(torch.uint8).permute(0, 2, 3, 1).contiguous()
         assert torch.equal(native.retinex_clahe_u8(xd, id_, ed), want)
+
+
+def misaligned(t):
+    """A contiguous copy of t whose data starts one element past a 16-byte boundary."""
+    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
+    view = buf[1:].view(t.shape)
+    view.copy_(t)
+    return view
+
+
+@pytest.mark.parametrize("which", ["x", "illu", "e"])
+@pytest.mark.parametrize("h,w", [(1080, 1920), (400, 600)])
+def test_retinex_clahe_misaligned_operand(native, h, w, which):
+    """One operand one float past 16-byte alignment: the fused call runs the generic histogram kernel on a shape of the vector
+    path.  f32 and u8 outputs bit-identical to upr_retinex_recombine_f32 -> upr_clahe_lab_f32 / upr_clahe_lab_f32_u8."""
+    rng = np.random.default_rng(h * w)
+    x = np.concatenate([O.kat_input(860 + i, h, w, ("dark", "uniform")[i % 2]) for i in range(2)])
+    ops = {"x": x, "e": rng.random((2, 3, h, w), dtype=np.float32),
+           "illu": (rng.random((2, 1, h, w), dtype=np.float32) * 0.9 + 0.05).astype(np.float32)}
+    ops = {k: torch.from_numpy(a).cuda() for k, a in ops.items()}
+    ops[which] = misaligned(ops[which])
+    assert ops[which].data_ptr() % 16 == 4
+    _, enh = native.retinex_recombine(ops["x"], ops["illu"], ops["e"], want_reflectance=False)
+    assert torch.equal(native.retinex_clahe(ops["x"], ops["illu"], ops["e"]), native.clahe_lab(enh))
+    assert torch.equal(native.retinex_clahe_u8(ops["x"], ops["illu"], ops["e"]), native.clahe_lab_f32_u8(enh))
 
 
 def test_second_device_same_process(native):

@@ -435,6 +435,23 @@ def test_content_multiscale_chain(native):
             np.testing.assert_allclose(out[i:i + 1].cpu().numpy(), want, rtol=0, atol=2e-6)
 
 
+@pytest.mark.parametrize("n,h,w,shift", [(2, 1080, 1920, 1), (1, 16, 491640, 0)])
+def test_multiscale_chains_on_the_generic_statistics_path(native, n, h, w, shift):
+    """multiscale_enhance and content_multiscale_apply on inputs the streaming statistics kernel does not serve: x one float past
+    16-byte alignment, and 4097 column bands of 120 px (more than the per-frame partial slots even with one row segment).  Same bits
+    as the generic statistics followed by the gain pass / the content-aware passes."""
+    g = torch.Generator(device="cuda").manual_seed(h + w)
+    buf = torch.rand((n * 3 * h * w + shift,), device="cuda", generator=g) * 0.8
+    x = buf[shift:].view(n, 3, h, w)
+    assert (x.data_ptr() % 16 != 0) == (shift != 0)
+    enh = torch.rand((n, 3, h, w), device="cuda", generator=g) * 1.2
+    means, gain = native.multiscale_stats(x, force_generic=True)
+    out, means2, gain2 = native.multiscale_enhance(x, enh)
+    assert torch.equal(out, native.scale_clamp(enh, gain)) and torch.equal(means2, means) and torch.equal(gain2, gain)
+    chain, gain3 = native.content_multiscale_apply(x, enh)
+    assert torch.equal(chain, native.scale_clamp(native.content_aware_apply(x, enh), gain)) and torch.equal(gain3, gain)
+
+
 def test_fused_peer_allreduce_two_gpus():
     """upr_texture_weight_peer_f32 under torchrun on two GPUs: bit-equal to statistics kernel + NCCL all-reduce + weight kernel on
     every rank, every step (unequal local batches included; beyond two ranks NCCL's summation order differs from the kernel's
