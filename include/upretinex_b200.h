@@ -90,6 +90,22 @@ UPR_API int upr_retinex_clahe_f32(const float* x_nchw, const float* illu_n1hw, c
 UPR_API int upr_retinex_clahe_f32_u8(const float* x_nchw, const float* illu_n1hw, const float* e_nchw,
                                      unsigned char* out_nhwc_rgb, int n, int h, int w, float eps, double clip_limit,
                                      int tiles_x, int tiles_y, void* workspace, size_t workspace_bytes, upr_stream_t stream);
+/* The same two fused calls with the maps in the dtypes the CNN emits under autocast (enum UPR_DT_* and UPR_RETINEX_AUTOCAST
+ * below): illu in illu_dtype, e in e_dtype, with e_dtype one of F32 / F16 / BF16 and illu_dtype either F32 or e_dtype.  The
+ * real network under CUDA autocast emits (F32, F16 / BF16): its illumination head adds an f32 scalar.  flags is 0 or
+ * UPR_RETINEX_AUTOCAST; anything else returns UPR_E_PARAM.  x stays f32.  With f(.) widening to f32, TI(.) / TE(.) rounding
+ * to illu's / e's dtype and every step one IEEE f32 operation:
+ *   d = TI(f(illu) + eps);  R = x / f(d);  c = f(e)*f(e), rounded to TE unless UPR_RETINEX_AUTOCAST;  enh = R*f(e) + (1-R)*f(c)
+ * (d is not rounded when illu is F32), i.e. torch eager of the two lines under torch.autocast("cuda", enabled=flags), followed
+ * by upr_clahe_lab_f32 resp. upr_clahe_lab_f32_u8 of enh, bit for bit.  F32 / F32 is upr_retinex_clahe_f32 / _f32_u8 (the flag
+ * is moot).  fp16 / bf16 maps read 2 B/px per map channel instead of 4.  NULL, n == 0, workspace and in-place rules as for the
+ * f32 entries. */
+UPR_API int upr_retinex_clahe_typed_f32(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                        int flags, float* out_nchw, int n, int h, int w, float eps, double clip_limit, int tiles_x,
+                                        int tiles_y, void* workspace, size_t workspace_bytes, upr_stream_t stream);
+UPR_API int upr_retinex_clahe_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                       int flags, unsigned char* out_nhwc_rgb, int n, int h, int w, float eps, double clip_limit,
+                                       int tiles_x, int tiles_y, void* workspace, size_t workspace_bytes, upr_stream_t stream);
 /* Profiling hook: runs only the selected stages of upr_clahe_lab_f32 on a workspace that a full call has
  * already populated.  stage_mask bit 0 = K1 (quantise + Lab + tile histograms + clip/LUT), bit 1 = K3
  * (bilinear LUT map + Lab->RGB); bench.py uses it to time each kernel with CUDA events. */
@@ -223,6 +239,11 @@ enum { UPR_DT_F32 = 0, UPR_DT_F16 = 1, UPR_DT_BF16 = 2 };
 enum { UPR_RETINEX_AUTOCAST = 1 };
 UPR_API int upr_retinex_recombine_maps(const float* x, const void* illu, const void* e, int map_dtype, int flags,
                                        float* refl, float* enh, int n, int h, int w, float eps, upr_stream_t stream);
+/* The forward of upr_retinex_recombine_maps with illu and e in separate dtypes: illu_dtype, e_dtype, flags and the arithmetic
+ * as for upr_retinex_clahe_typed_f32 (d is rounded to illu's dtype, c to e's); the NULL rules of upr_retinex_recombine_maps
+ * (e or refl may be NULL).  upr_retinex_recombine_maps is this entry with illu_dtype == e_dtype. */
+UPR_API int upr_retinex_recombine_typed(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                                        float* refl, float* enh, int n, int h, int w, float eps, upr_stream_t stream);
 UPR_API int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
                                        const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e,
                                        int n, int h, int w, float eps, upr_stream_t stream);

@@ -32,10 +32,10 @@ def main_enhance(args):
         raise SystemExit(f"错误: 输入路径 '{args.input_path}' 不存在")
     if os.path.isdir(args.input_path):
         enhance_batch_images(args.input_path, args.output_dir, device, args.max_size, args.multi_scale, args.content_aware,
-                             model=_model(device, args.use_preact, args.use_aspp))
+                             model=_model(device, args.use_preact, args.use_aspp), amp=args.amp)
     else:
         enhance_single_image(_model(device, args.use_preact, args.use_aspp), args.input_path, args.output_dir, device,
-                             args.max_size, args.multi_scale, args.content_aware, adjuster=AdaptiveParameterAdjuster())
+                             args.max_size, args.multi_scale, args.content_aware, adjuster=AdaptiveParameterAdjuster(), amp=args.amp)
 
 
 def main_predict(args):
@@ -57,9 +57,9 @@ def main_predict(args):
     model = model.to(device).eval()
     print("模型加载完成")
     if os.path.isdir(args.input_path):
-        P.predict_batch(model, args.input_path, args.output_dir, device, args.max_size, not args.no_comparison)
+        P.predict_batch(model, args.input_path, args.output_dir, device, args.max_size, not args.no_comparison, amp=args.amp)
     else:
-        P.predict_single_image(model, args.input_path, args.output_dir, device, args.max_size, not args.no_comparison)
+        P.predict_single_image(model, args.input_path, args.output_dir, device, args.max_size, not args.no_comparison, amp=args.amp)
     return 0
 
 
@@ -77,6 +77,7 @@ def build_main_parser():
     p.add_argument("--use_preact", action="store_true")
     p.add_argument("--use_aspp", action="store_true")
     p.add_argument("--no_comparison", action="store_true")
+    p.add_argument("--amp", type=str, default=None, choices=["bf16", "fp16"], help="run the CNN under CUDA autocast")
     return p
 
 
@@ -96,7 +97,8 @@ def simple_enhance_main(argv=None):
     p.add_argument("--device", type=str, default=None)
     p.add_argument("--multi_scale", action="store_true")
     p.add_argument("--content_aware", action="store_true")     # parsed AND forwarded (the reference drops it, :70-77)
+    p.add_argument("--amp", type=str, default=None, choices=["bf16", "fp16"], help="run the CNN under CUDA autocast")
     a = p.parse_args(argv)
     ns = argparse.Namespace(input_path=a.input, output_dir=a.output, max_size=a.max_size, device=a.device,
-                            multi_scale=a.multi_scale, content_aware=a.content_aware, use_preact=False, use_aspp=False)
+                            multi_scale=a.multi_scale, content_aware=a.content_aware, use_preact=False, use_aspp=False, amp=a.amp)
     return main_enhance(ns)

@@ -27,6 +27,7 @@
 #include <cstring>
 
 #include "upr_common.cuh"
+#include "upr_maps.cuh"
 #include "upr_tables_gen.h"
 
 namespace upr {
@@ -421,17 +422,12 @@ __device__ __forceinline__ void k1_core(const float (&R)[4], const float (&G)[4]
 
 // kFused: the CLAHE input is the Retinex recombination of the CNN outputs (models/model.py:405-413,442 followed by
 // adaptive_params.py:195): enhanced = R*e + (1-R)*e^2 with R = x / (illu + eps), evaluated in registers with exactly the
-// arithmetic of k_recombine_vec (IEEE division, separately rounded products) -- the 12 B/px `enhanced` frame is never
-// written nor re-read (x 12 + illu 4 + e 12 B/px are read instead).
-__device__ __forceinline__ void recombine_px(float x, float d, float e, float& r, float& o)
-{
-    r = __fdiv_rn(x, d);
-    o = __fadd_rn(__fmul_rn(r, e), __fmul_rn(__fsub_rn(1.0f, r), __fmul_rn(e, e)));
-}
-
+// arithmetic of k_recombine_vec (upr_maps.cuh: IEEE division, separately rounded products, the roundings of the map dtypes) --
+// the 12 B/px `enhanced` frame is never written nor re-read (x 12 + illu 4 + e 12 B/px are read instead, less for fp16 / bf16
+// maps).  The pointers have the kernel's map types TI (illu) and TE (e).
 struct RetinexIn {
-    const float* illu;   // [n][1][h][w]
-    const float* e;      // [n][3][h][w]
+    const void* illu;    // [n][1][h][w]
+    const void* e;       // [n][3][h][w]
     float eps;
 };
 
@@ -447,11 +443,13 @@ struct RetinexIn {
 //   kU8In : the frame is packed u8 RGB (HWC, upr_clahe_lab_u8): a 4-pixel group is 12 contiguous bytes, three 32-bit
 //           loads; the bytes index the gamma table directly (no quantisation).
 //   kFused: the CLAHE input is the Retinex recombination of the CNN outputs (models/model.py:405-413,442 followed by
-//           adaptive_params.py:195), evaluated in registers (recombine_px) from x, illu and e: 28 B/px read instead of a
-//           12 B/px `enhanced` frame written by one kernel and re-read by this one.  One raw register set (7 float4)
-//           requested one iteration ahead; two CTAs per SM (128 registers) instead of three.
+//           adaptive_params.py:195), evaluated in registers (recombine1) from x, illu and e: 28 B/px read (f32 maps)
+//           instead of a 12 B/px `enhanced` frame written by one kernel and re-read by this one.  One raw register set
+//           requested one iteration ahead (f32 maps: 7 float4; fp16 / bf16 e: 8 bytes per 4 pixels and channel, kept packed
+//           until use); two CTAs per SM (128 registers) instead of three.  TI / TE / kAutocast: the maps' dtypes and
+//           autocast semantics of e**2 (upr_maps.cuh).
 // ---------------------------------------------------------------------------------------------
-template <bool kU8In, bool kFused>
+template <bool kU8In, bool kFused, typename TI = float, typename TE = float, bool kAutocast = false>
 __global__ void __launch_bounds__(kK1Threads, kFused ? 2 : 3)
 k_hist_lab_vec3(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t* __restrict__ hist_g,
                 uint8_t* __restrict__ lut_g, unsigned* __restrict__ tickets, const ClaheGeom g, const RetinexIn rx)
@@ -534,28 +532,33 @@ k_hist_lab_vec3(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t*
     const int row_pf = row1 - kPf * rpi;            // row < row_pf: there is an iteration kPf ahead to prefetch
 
     if constexpr (kFused) {
-        const float4* eR = opaque_ptr(reinterpret_cast<const float4*>(rx.e) + (size_t(f) * 3 * plane4 + col));
-        const float4* eG = opaque_ptr(eR + plane4);
-        const float4* eB = opaque_ptr(eG + plane4);
-        const float4* ilp = opaque_ptr(reinterpret_cast<const float4*>(rx.illu) + (size_t(f) * plane4 + col));
-        float4 X0, X1, X2, E0, E1, E2, IL;
+        using RawE = typename MapIO<TE>::Raw4;
+        using RawI = typename MapIO<TI>::Raw4;
+        const RawE* eR = opaque_ptr(reinterpret_cast<const RawE*>(rx.e) + (size_t(f) * 3 * plane4 + col));
+        const RawE* eG = opaque_ptr(eR + plane4);
+        const RawE* eB = opaque_ptr(eG + plane4);
+        const RawI* ilp = opaque_ptr(reinterpret_cast<const RawI*>(rx.illu) + (size_t(f) * plane4 + col));
+        float4 X0, X1, X2;
+        RawE E0, E1, E2;
+        RawI IL;
         auto load7 = [&](uint32_t oo) {
             X0 = ld_nc_f4(inR + oo); X1 = ld_nc_f4(inG + oo); X2 = ld_nc_f4(inB + oo);
-            E0 = ld_nc_f4(eR + oo); E1 = ld_nc_f4(eG + oo); E2 = ld_nc_f4(eB + oo);
-            IL = ld_nc_f4(ilp + oo);
+            E0 = MapIO<TE>::ld4nc(eR + oo); E1 = MapIO<TE>::ld4nc(eG + oo); E2 = MapIO<TE>::ld4nc(eB + oo);
+            IL = MapIO<TI>::ld4nc(ilp + oo);
         };
         auto prefetch7 = [&](uint32_t oo) {
             prefetch_l2(inR + oo); prefetch_l2(inG + oo); prefetch_l2(inB + oo);
             prefetch_l2(eR + oo); prefetch_l2(eG + oo); prefetch_l2(eB + oo);
             prefetch_l2(ilp + oo);
         };
-        auto recombine4 = [&](const float4 xv, const float4 ev, const float d[4]) {
+        auto recombine4 = [&](const float4 xv, const RawE raw, const float d[4]) {
+            const float4 ev = MapIO<TE>::wide4(raw);
             float4 r;
             float refl;
-            recombine_px(xv.x, d[0], ev.x, refl, r.x);
-            recombine_px(xv.y, d[1], ev.y, refl, r.y);
-            recombine_px(xv.z, d[2], ev.z, refl, r.z);
-            recombine_px(xv.w, d[3], ev.w, refl, r.w);
+            recombine1<TE, kAutocast>(xv.x, d[0], ev.x, refl, r.x);
+            recombine1<TE, kAutocast>(xv.y, d[1], ev.y, refl, r.y);
+            recombine1<TE, kAutocast>(xv.z, d[2], ev.z, refl, r.z);
+            recombine1<TE, kAutocast>(xv.w, d[3], ev.w, refl, r.w);
             return r;
         };
         if (row < row1) {
@@ -565,7 +568,9 @@ k_hist_lab_vec3(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t*
                 if (row + k * rpi < row1) prefetch7(o + uint32_t(k) * step);
         }
         while (row < row1) {
-            const float d[4] = {__fadd_rn(IL.x, rx.eps), __fadd_rn(IL.y, rx.eps), __fadd_rn(IL.z, rx.eps), __fadd_rn(IL.w, rx.eps)};
+            const float4 il = MapIO<TI>::wide4(IL);
+            const float d[4] = {illu_eps<TI>(il.x, rx.eps), illu_eps<TI>(il.y, rx.eps), illu_eps<TI>(il.z, rx.eps),
+                                illu_eps<TI>(il.w, rx.eps)};
             const float4 er = recombine4(X0, E0, d), eg = recombine4(X1, E1, d), eb = recombine4(X2, E2, d);
             if (row < row_ld) load7(o + step);
             if (row < row_pf) prefetch7(o + pfo);
@@ -655,8 +660,8 @@ k_hist_lab_vec3(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t*
 // K1 generic path: any size (including OpenCV's reflect-101 padding quirk, Appendix A.3 step 1).
 // One CTA per (frame, tile); per-warp shared histograms with atomics.  Correctness path for
 // ragged shapes -- the named workloads all take the vector path.
-//   kFused: as in k_hist_lab_vec3, the input is the Retinex recombination of x, illu and e, evaluated per (reflected)
-//           pixel with recombine_px.
+//   kFused: as in k_hist_lab_vec3, the input is the Retinex recombination of x, illu (TI) and e (TE), evaluated per
+//           (reflected) pixel with recombine1; each map value is widened where it is loaded.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ int reflect101(int p, int len)
 {
@@ -665,7 +670,7 @@ __device__ __forceinline__ int reflect101(int p, int len)
     return p;
 }
 
-template <bool kU8In, bool kFused>
+template <bool kU8In, bool kFused, typename TI = float, typename TE = float, bool kAutocast = false>
 __global__ void __launch_bounds__(256)
 k_hist_lab_generic(const void* __restrict__ in, uint8_t* __restrict__ lab, int32_t* __restrict__ hist_g,
                    uint8_t* __restrict__ lut_g, const ClaheGeom g, const RetinexIn rx)
@@ -700,12 +705,13 @@ k_hist_lab_generic(const void* __restrict__ in, uint8_t* __restrict__ lab, int32
         if constexpr (kU8In) {
             qr = in8[3 * off + 0]; qg = in8[3 * off + 1]; qb = in8[3 * off + 2];
         } else if constexpr (kFused) {
-            const float* eR = rx.e + size_t(f) * 3 * plane;
-            const float d = __fadd_rn(ld_stream_f1(rx.illu + size_t(f) * plane + off, pol_stream), rx.eps);
+            const TE* eR = static_cast<const TE*>(rx.e) + size_t(f) * 3 * plane;
+            const float d = illu_eps<TI>(MapIO<TI>::ld1(static_cast<const TI*>(rx.illu) + size_t(f) * plane + off, pol_stream), rx.eps);
             float refl, o[3];
 #pragma unroll
             for (int c = 0; c < 3; ++c)
-                recombine_px(ld_stream_f1(inR + c * plane + off, pol_stream), d, ld_stream_f1(eR + c * plane + off, pol_stream), refl, o[c]);
+                recombine1<TE, kAutocast>(ld_stream_f1(inR + c * plane + off, pol_stream), d, MapIO<TE>::ld1(eR + c * plane + off, pol_stream),
+                                          refl, o[c]);
             qr = quantize_u8(o[0]); qg = quantize_u8(o[1]); qb = quantize_u8(o[2]);
         } else {
             qr = quantize_u8(ld_stream_f1(inR + off, pol_stream));
@@ -1053,7 +1059,28 @@ static bool valid_shape(int n, int h, int w, int tiles_x, int tiles_y)
 // cudaFuncAttributeMaxDynamicSharedMemorySize bookkeeping, one word per kernel instantiation, one bit per device ordinal.
 // Written without a lock on purpose: concurrent callers can only both see "not set yet" and both issue the (idempotent)
 // cudaFuncSetAttribute call; the words are atomics so that the race is a defined one.
-static std::atomic<unsigned long long> g_smem_mask[5];
+static std::atomic<unsigned long long> g_smem_mask[4];
+
+// storage dtypes (UPR_DT_*) and flags of the Retinex maps of a fused call; valid_map_dtypes() holds
+struct MapDtypes {
+    int illu = UPR_DT_F32, e = UPR_DT_F32, flags = 0;
+};
+static size_t map_bytes(int dt) { return dt == UPR_DT_F32 ? sizeof(float) : 2; }
+
+// K1 with the fused Retinex prologue on maps (TI, TE): the vector kernel when `fast`, the generic one otherwise
+template <typename TI, typename TE, bool AC>
+static int k1_fused_launch(bool fast, dim3 grid, size_t smem, cudaStream_t stream, const float* in, uint8_t* lab, int32_t* hist,
+                           uint8_t* lut, unsigned* tickets, const ClaheGeom& g, const RetinexIn& rx)
+{
+    if (fast) {
+        static std::atomic<unsigned long long> smem_mask{0};   // one per instantiation, as g_smem_mask
+        UPR_CUDA_TRY(ensure_dynamic_smem(k_hist_lab_vec3<false, true, TI, TE, AC>, smem, smem_mask));
+        k_hist_lab_vec3<false, true, TI, TE, AC><<<grid, kK1Threads, smem, stream>>>(in, lab, hist, lut, tickets, g, rx);
+    } else {
+        k_hist_lab_generic<false, true, TI, TE, AC><<<grid, 256, 0, stream>>>(in, lab, hist, lut, g, rx);
+    }
+    return UPR_OK;
+}
 
 // raw tile coordinate of OpenCV's interpolation: floor(p * inv - 0.5f), fp32, separately rounded
 static inline int raw_tile(int p, float inv)
@@ -1065,9 +1092,10 @@ static inline int raw_tile(int p, float inv)
 
 // stage_mask: bit 0 = K1 (Lab + histograms + LUTs), bit 1 = K3 (map); 3 = the whole op
 // in_u8 / out_u8: the frame on that side is packed u8 RGB (HWC) instead of planar f32 (NCHW)
+// rx: the fused Retinex prologue on maps of the dtypes `dt`
 static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double clip_limit, int tiles_x, int tiles_y,
                      void* ws, size_t ws_bytes, cudaStream_t stream, int stage_mask = 3, const RetinexIn* rx = nullptr,
-                     bool in_u8 = false, bool out_u8 = false)
+                     bool in_u8 = false, bool out_u8 = false, MapDtypes dt = {})
 {
     if (!valid_shape(n, h, w, tiles_x, tiles_y)) return UPR_E_SHAPE;
     if (n == 0) return UPR_OK;
@@ -1107,7 +1135,9 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
     bool fast = !padded && tiles_x <= kMaxTiles && tiles_y <= kMaxTiles && (g.tw % 4 == 0) && g.tw / 4 <= 63 * kK1Threads &&
                 (in_u8 ? (reinterpret_cast<uintptr_t>(in_v) & 3u) == 0 : aligned16(in_v)) &&
                 (out_u8 ? (reinterpret_cast<uintptr_t>(out_v) & 3u) == 0 : aligned16(out_v)) &&
-                size_t(h) * w * 3 < (size_t(1) << 32) && (!rx || (aligned16(rx->illu) && aligned16(rx->e)));
+                size_t(h) * w * 3 < (size_t(1) << 32) &&
+                (!rx || ((reinterpret_cast<uintptr_t>(rx->illu) & (4 * map_bytes(dt.illu) - 1)) == 0 &&
+                         (reinterpret_cast<uintptr_t>(rx->e) & (4 * map_bytes(dt.e) - 1)) == 0));   // 4 pixels of each map
     if (fast) {
         m.ay_bias = 0u - 0x4B400000u * 128u;
         m.n = n; m.h = h; m.w = w; m.tiles_x = tiles_x; m.tiles_y = tiles_y; m.inv_tw = inv_tw; m.inv_th = inv_th;
@@ -1152,7 +1182,15 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
         const int nf = std::min(n - f0, 65535);
         const size_t fplane = size_t(f0) * 3 * h * w;
         const size_t ftile = size_t(f0) * ntiles;
-        const RetinexIn rxf = rx ? RetinexIn{rx->illu + size_t(f0) * h * w, rx->e + fplane, rx->eps} : RetinexIn{nullptr, nullptr, 0.0f};
+        const RetinexIn rxf = rx ? RetinexIn{static_cast<const char*>(rx->illu) + size_t(f0) * h * w * map_bytes(dt.illu),
+                                             static_cast<const char*>(rx->e) + fplane * map_bytes(dt.e), rx->eps}
+                                 : RetinexIn{nullptr, nullptr, 0.0f};
+        auto k1_fused = [&](bool vec, dim3 grid1, size_t smem1) {
+            return with_map_types(dt.illu, dt.e, dt.flags, [&](auto ti, auto te, auto ac) {
+                return k1_fused_launch<typename decltype(ti)::type, typename decltype(te)::type, decltype(ac)::value>(
+                    vec, grid1, smem1, stream, in + fplane, lab + fplane, hist + ftile * 256, lut + ftile * 256, tickets + ftile, g, rxf);
+            });
+        };
         if (fast) {
             // K1: byte counters allow <= 255 pixels per thread between flushes -> <= 63 items/thread
             const int tw4 = g.tw / 4;
@@ -1184,11 +1222,10 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
                     k_hist_lab_vec3<true, false><<<grid1, kK1Threads, smem1, stream>>>(
                         static_cast<const uint8_t*>(in_v) + fplane, lab + fplane, hist + ftile * 256, lut + ftile * 256, tickets + ftile, g, rxf);
                 } else if (rx) {
-                    UPR_CUDA_TRY(ensure_dynamic_smem(k_hist_lab_vec3<false, true>, smem1, g_smem_mask[1]));
-                    k_hist_lab_vec3<false, true><<<grid1, kK1Threads, smem1, stream>>>(
-                        in + fplane, lab + fplane, hist + ftile * 256, lut + ftile * 256, tickets + ftile, g, rxf);
+                    const int rc = k1_fused(true, grid1, smem1);
+                    if (rc != UPR_OK) return rc;
                 } else {
-                    UPR_CUDA_TRY(ensure_dynamic_smem(k_hist_lab_vec3<false, false>, smem1, g_smem_mask[2]));
+                    UPR_CUDA_TRY(ensure_dynamic_smem(k_hist_lab_vec3<false, false>, smem1, g_smem_mask[1]));
                     k_hist_lab_vec3<false, false><<<grid1, kK1Threads, smem1, stream>>>(
                         in + fplane, lab + fplane, hist + ftile * 256, lut + ftile * 256, tickets + ftile, g, rxf);
                 }
@@ -1217,10 +1254,10 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
                     const dim3 grid5(unsigned(std::min<long long>(nitems, resident)));
                     void* outf = static_cast<char*>(out_v) + fplane * out_es;
                     if (out_u8) {
-                        UPR_CUDA_TRY(ensure_dynamic_smem(k_map_vec5<true, true>, smem5, g_smem_mask[3]));
+                        UPR_CUDA_TRY(ensure_dynamic_smem(k_map_vec5<true, true>, smem5, g_smem_mask[2]));
                         k_map_vec5<true, true><<<grid5, nthr, smem5, stream>>>(lab + fplane, lut + ftile * 256, outf, m, work, int(nitems));
                     } else {
-                        UPR_CUDA_TRY(ensure_dynamic_smem(k_map_vec5<true, false>, smem5, g_smem_mask[4]));
+                        UPR_CUDA_TRY(ensure_dynamic_smem(k_map_vec5<true, false>, smem5, g_smem_mask[3]));
                         k_map_vec5<true, false><<<grid5, nthr, smem5, stream>>>(lab + fplane, lut + ftile * 256, outf, m, work, int(nitems));
                     }
                 }
@@ -1232,8 +1269,10 @@ static int clahe_run(const void* in_v, void* out_v, int n, int h, int w, double 
                 const void* inf = static_cast<const char*>(in_v) + fplane * in_es;
                 const dim3 grid1(ntiles, nf);
                 if (in_u8) k_hist_lab_generic<true, false><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
-                else if (rx) k_hist_lab_generic<false, true><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
-                else k_hist_lab_generic<false, false><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
+                else if (rx) {
+                    const int rc = k1_fused(false, grid1, 0);
+                    if (rc != UPR_OK) return rc;
+                } else k_hist_lab_generic<false, false><<<grid1, 256, 0, stream>>>(inf, lab + fplane, hist + ftile * 256, lut + ftile * 256, g, rxf);
                 UPR_LAUNCH_CHECK();
             }
             const size_t plane = size_t(h) * w;
@@ -1287,6 +1326,40 @@ int upr_retinex_clahe_f32_u8(const float* x, const float* illu, const float* e, 
     const upr::RetinexIn rx{illu, e, eps};
     return upr::clahe_run(x, out_nhwc, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes,
                           static_cast<cudaStream_t>(stream), 3, &rx, false, true);
+}
+
+// the typed entries: the checks of the f32 ones (shape, then the dtypes and flags, then n == 0, then NULL) before clahe_run
+static int retinex_clahe_typed(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags, void* out,
+                               bool out_u8, int n, int h, int w, float eps, double clip_limit, int tiles_x, int tiles_y,
+                               void* workspace, size_t workspace_bytes, cudaStream_t stream)
+{
+    if (!upr::valid_shape(n, h, w, tiles_x, tiles_y)) return UPR_E_SHAPE;
+    if (!upr::valid_map_dtypes(illu_dtype, e_dtype, flags)) return UPR_E_PARAM;
+    if (n == 0) return UPR_OK;
+    if (!x || !illu || !e) return UPR_E_NULL;
+    const upr::RetinexIn rx{illu, e, eps};
+    upr::MapDtypes dt;
+    dt.illu = illu_dtype;
+    dt.e = e_dtype;
+    dt.flags = flags;
+    return upr::clahe_run(x, out, n, h, w, clip_limit, tiles_x, tiles_y, workspace, workspace_bytes, stream, 3, &rx, false, out_u8,
+                          dt);
+}
+
+int upr_retinex_clahe_typed_f32(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                                float* out_nchw, int n, int h, int w, float eps, double clip_limit, int tiles_x, int tiles_y,
+                                void* workspace, size_t workspace_bytes, upr_stream_t stream)
+{
+    return retinex_clahe_typed(x, illu, illu_dtype, e, e_dtype, flags, out_nchw, false, n, h, w, eps, clip_limit, tiles_x, tiles_y,
+                               workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int upr_retinex_clahe_typed_u8(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                               unsigned char* out_nhwc_rgb, int n, int h, int w, float eps, double clip_limit, int tiles_x,
+                               int tiles_y, void* workspace, size_t workspace_bytes, upr_stream_t stream)
+{
+    return retinex_clahe_typed(x, illu, illu_dtype, e, e_dtype, flags, out_nhwc_rgb, true, n, h, w, eps, clip_limit, tiles_x,
+                               tiles_y, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 int upr_clahe_lab_u8(const unsigned char* in_nhwc, unsigned char* out_nhwc, int n, int h, int w, double clip_limit, int tiles_x,

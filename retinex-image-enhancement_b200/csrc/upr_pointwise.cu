@@ -12,10 +12,7 @@
 // frame-major index space.  Every product/sum is an explicitly rounded fp32 operation
 // (__fmul_rn/__fadd_rn/__fdiv_rn): torch eager evaluates each Python operator as its own
 // kernel, so there is no FMA contraction in the reference and none here -> bit-exact.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-
-#include "upr_common.cuh"
+#include "upr_maps.cuh"
 
 namespace upr {
 
@@ -28,77 +25,12 @@ __device__ __forceinline__ float clamp01_keep_nan(float v)
     return v < 0.0f ? 0.0f : (v > 1.0f ? 1.0f : v);
 }
 
-// ---- map storage -------------------------------------------------------------------------
-// The CNN's illumination and enhancement maps are f32, or fp16 / bf16 when the model runs under autocast.  Every map value
-// is widened to f32 on load; rnd<T>(v) = f(T(v)) is the rounding torch applies when an op's result has the map's dtype.
-template <typename T> struct MapIO;
-
-template <> struct MapIO<float> {
-    using Raw4 = float4;   // 4 pixels as loaded
-    static __device__ __forceinline__ float wide(float v) { return v; }
-    static __device__ __forceinline__ float narrow(float v) { return v; }
-    static __device__ __forceinline__ float4 ld4raw(const float* p, uint64_t pol) { return ld_stream_f4(p, pol); }
-    static __device__ __forceinline__ float4 wide4(float4 v) { return v; }
-    static __device__ __forceinline__ float4 ld4(const float* p, uint64_t pol) { return ld_stream_f4(p, pol); }
-    static __device__ __forceinline__ void st4(float* p, float4 v, uint64_t pol) { st_stream_f4(p, v, pol); }
-};
-
-__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
-__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
-__device__ __forceinline__ __half from_f32(float v, const __half*) { return __float2half_rn(v); }
-__device__ __forceinline__ __nv_bfloat16 from_f32(float v, const __nv_bfloat16*) { return __float2bfloat16_rn(v); }
-__device__ __forceinline__ __half from_bits(uint32_t b, const __half*) { return __ushort_as_half((unsigned short)b); }
-__device__ __forceinline__ __nv_bfloat16 from_bits(uint32_t b, const __nv_bfloat16*) { return __ushort_as_bfloat16((unsigned short)b); }
-__device__ __forceinline__ uint32_t to_bits(__half v) { return __half_as_ushort(v); }
-__device__ __forceinline__ uint32_t to_bits(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
-
-template <typename H> struct MapIO16 {   // H = __half or __nv_bfloat16
-    using Raw4 = uint2;    // kept packed until use: fewer registers live across the division slow path
-    static __device__ __forceinline__ float wide(H v) { return to_f32(v); }
-    static __device__ __forceinline__ H narrow(float v) { return from_f32(v, (const H*)nullptr); }
-    static __device__ __forceinline__ float lo(uint32_t u) { return to_f32(from_bits(u & 0xffffu, (const H*)nullptr)); }
-    static __device__ __forceinline__ float hi(uint32_t u) { return to_f32(from_bits(u >> 16, (const H*)nullptr)); }
-    static __device__ __forceinline__ uint32_t pack(float a, float b) { return to_bits(narrow(a)) | (to_bits(narrow(b)) << 16); }
-    // 4 pixels = 8 bytes: one 64-bit streaming access
-    static __device__ __forceinline__ uint2 ld4raw(const H* p, uint64_t pol)
-    {
-        uint2 v;
-        asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.u32 {%0,%1}, [%2], %3;" : "=r"(v.x), "=r"(v.y) : "l"(p), "l"(pol));
-        return v;
-    }
-    static __device__ __forceinline__ float4 wide4(uint2 v) { return make_float4(lo(v.x), hi(v.x), lo(v.y), hi(v.y)); }
-    static __device__ __forceinline__ float4 ld4(const H* p, uint64_t pol) { return wide4(ld4raw(p, pol)); }
-    static __device__ __forceinline__ void st4(H* p, float4 v, uint64_t pol)
-    {
-        asm volatile("st.global.L1::no_allocate.L2::cache_hint.v2.u32 [%0], {%1,%2}, %3;" ::"l"(p), "r"(pack(v.x, v.y)),
-                     "r"(pack(v.z, v.w)), "l"(pol)
-                     : "memory");
-    }
-};
-template <> struct MapIO<__half> : MapIO16<__half> {};
-template <> struct MapIO<__nv_bfloat16> : MapIO16<__nv_bfloat16> {};
-
-template <typename T> __device__ __forceinline__ float rnd(float v) { return MapIO<T>::wide(MapIO<T>::narrow(v)); }
-
-// e^2 with the map dtype T: torch rounds pow's result to T, except under CUDA autocast, where pow runs in fp32
-template <typename T, bool kAutocast> __device__ __forceinline__ float square(float e)
-{
-    return kAutocast ? __fmul_rn(e, e) : rnd<T>(__fmul_rn(e, e));
-}
-
-template <typename T, bool kAutocast>
-__device__ __forceinline__ void recombine1(float x, float d, float e, float& r, float& o)
-{
-    r = __fdiv_rn(x, d);
-    o = __fadd_rn(__fmul_rn(r, e), __fmul_rn(__fsub_rn(1.0f, r), square<T, kAutocast>(e)));
-}
-
 // ---- a8 ---------------------------------------------------------------------------------
-// plane4 = H*W/4 ; one work item = 4 consecutive pixels of one frame (all three channels).  T = map storage type; d = illu + eps
-// is rounded to T (torch adds the scalar in fp32 and stores a T tensor), R and enhanced are f32 (type promotion).
-template <typename T, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
+// plane4 = H*W/4 ; one work item = 4 consecutive pixels of one frame (all three channels).  TI / TE = storage types of illu / e
+// (upr_maps.cuh); d = illu + eps is rounded to TI, R and enhanced are f32 (type promotion).
+template <typename TI, typename TE, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
 __global__ void __launch_bounds__(kPwThreads)
-k_recombine_vec(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+k_recombine_vec(const float* __restrict__ x, const TI* __restrict__ illu, const TE* __restrict__ e,
                 float* __restrict__ refl, float* __restrict__ enh, long long plane4, long long items, float eps)
 {
     const uint64_t pol = policy_evict_first();
@@ -106,25 +38,24 @@ k_recombine_vec(const float* __restrict__ x, const T* __restrict__ illu, const T
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane4, p = it - f * plane4;
         const long long o3 = (f * 3 * plane4 + p) * 4, o1 = (f * plane4 + p) * 4;
-        const float4 il = MapIO<T>::ld4(illu + o1, pol);
-        const float d[4] = {rnd<T>(__fadd_rn(il.x, eps)), rnd<T>(__fadd_rn(il.y, eps)), rnd<T>(__fadd_rn(il.z, eps)),
-                            rnd<T>(__fadd_rn(il.w, eps))};
+        const float4 il = MapIO<TI>::ld4(illu + o1, pol);
+        const float d[4] = {illu_eps<TI>(il.x, eps), illu_eps<TI>(il.y, eps), illu_eps<TI>(il.z, eps), illu_eps<TI>(il.w, eps)};
         float4 xv[3];
-        typename MapIO<T>::Raw4 ev[3];
+        typename MapIO<TE>::Raw4 ev[3];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             xv[c] = ld_stream_f4(x + o3 + c * plane4 * 4, pol);
-            if (kWriteEnh) ev[c] = MapIO<T>::ld4raw(e + o3 + c * plane4 * 4, pol);
+            if (kWriteEnh) ev[c] = MapIO<TE>::ld4raw(e + o3 + c * plane4 * 4, pol);
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             float4 r, o;
             if (kWriteEnh) {
-                const float4 ef = MapIO<T>::wide4(ev[c]);
-                recombine1<T, kAutocast>(xv[c].x, d[0], ef.x, r.x, o.x);
-                recombine1<T, kAutocast>(xv[c].y, d[1], ef.y, r.y, o.y);
-                recombine1<T, kAutocast>(xv[c].z, d[2], ef.z, r.z, o.z);
-                recombine1<T, kAutocast>(xv[c].w, d[3], ef.w, r.w, o.w);
+                const float4 ef = MapIO<TE>::wide4(ev[c]);
+                recombine1<TE, kAutocast>(xv[c].x, d[0], ef.x, r.x, o.x);
+                recombine1<TE, kAutocast>(xv[c].y, d[1], ef.y, r.y, o.y);
+                recombine1<TE, kAutocast>(xv[c].z, d[2], ef.z, r.z, o.z);
+                recombine1<TE, kAutocast>(xv[c].w, d[3], ef.w, r.w, o.w);
                 st_stream_f4(enh + o3 + c * plane4 * 4, o, pol);
             } else {
                 r.x = __fdiv_rn(xv[c].x, d[0]);
@@ -137,21 +68,21 @@ k_recombine_vec(const float* __restrict__ x, const T* __restrict__ illu, const T
     }
 }
 
-template <typename T, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
+template <typename TI, typename TE, bool kAutocast, bool kWriteRefl, bool kWriteEnh>
 __global__ void __launch_bounds__(kPwThreads)
-k_recombine_scalar(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+k_recombine_scalar(const float* __restrict__ x, const TI* __restrict__ illu, const TE* __restrict__ e,
                    float* __restrict__ refl, float* __restrict__ enh, long long plane, long long items, float eps)
 {
     const long long stride = (long long)gridDim.x * kPwThreads;
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane, p = it - f * plane;
-        const float d = rnd<T>(__fadd_rn(MapIO<T>::wide(illu[it]), eps));
+        const float d = illu_eps<TI>(MapIO<TI>::wide(illu[it]), eps);
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const long long o = (f * 3 + c) * plane + p;
             float r, v;
             if (kWriteEnh) {
-                recombine1<T, kAutocast>(x[o], d, MapIO<T>::wide(e[o]), r, v);
+                recombine1<TE, kAutocast>(x[o], d, MapIO<TE>::wide(e[o]), r, v);
                 enh[o] = v;
             } else {
                 r = __fdiv_rn(x[o], d);
@@ -324,13 +255,8 @@ static inline int pw_grid(long long items)
     return int(std::max<long long>(1, std::min<long long>(want, (long long)kNumSMsB200 * kPwCtasPerSm)));
 }
 
-template <typename T> static inline bool aligned4px(const T* p)
-{
-    return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0;
-}
-
-template <typename T, bool AC, bool R, bool E>
-static int recombine_launch(const float* x, const T* illu, const T* e, float* refl, float* enh, int n, int h, int w,
+template <typename TI, typename TE, bool AC, bool R, bool E>
+static int recombine_launch(const float* x, const TI* illu, const TE* e, float* refl, float* enh, int n, int h, int w,
                             float eps, cudaStream_t s)
 {
     const long long plane = (long long)h * w;
@@ -338,26 +264,37 @@ static int recombine_launch(const float* x, const T* illu, const T* e, float* re
                      (!R || aligned16(refl));
     if (vec) {
         const long long items = (long long)n * (plane / 4);
-        k_recombine_vec<T, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane / 4, items, eps);
+        k_recombine_vec<TI, TE, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane / 4, items, eps);
     } else {
         const long long items = (long long)n * plane;
-        k_recombine_scalar<T, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane, items, eps);
+        k_recombine_scalar<TI, TE, AC, R, E><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, refl, enh, plane, items, eps);
     }
     UPR_LAUNCH_CHECK();
     return UPR_OK;
 }
 
-// upr_retinex_recombine_maps on map type T; the arguments are checked (refl or enh is given; enh only with e).  Without e,
-// or without enh, only R is formed, and the flag is moot.
-template <typename T, bool AC>
+// upr_retinex_recombine_maps / _typed on map types (TI, TE); the arguments are checked (refl or enh is given; enh only with e).
+// Without e, or without enh, only R is formed, and e's dtype and the flag are moot.
+template <typename TI, typename TE, bool AC>
 static int recombine_maps(const float* x, const void* illu_v, const void* e_v, float* refl, float* enh, int n, int h,
                           int w, float eps, cudaStream_t s)
 {
-    const T* illu = static_cast<const T*>(illu_v);
-    const T* e = static_cast<const T*>(e_v);
-    if (!e || !enh) return recombine_launch<T, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps, s);
-    return refl ? recombine_launch<T, AC, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
-                : recombine_launch<T, AC, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
+    const TI* illu = static_cast<const TI*>(illu_v);
+    const TE* e = static_cast<const TE*>(e_v);
+    if (!e || !enh)
+        return recombine_launch<TI, TI, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps, s);
+    return refl ? recombine_launch<TI, TE, AC, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                : recombine_launch<TI, TE, AC, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
+}
+
+// the checked arguments of upr_retinex_recombine_maps / _typed, dispatched on (illu dtype, e dtype, autocast)
+static int recombine_typed(const float* x, const void* illu, int illu_dt, const void* e, int e_dt, int flags, float* refl,
+                           float* enh, int n, int h, int w, float eps, cudaStream_t s)
+{
+    return with_map_types(illu_dt, e_dt, flags, [&](auto ti, auto te, auto ac) {
+        return recombine_maps<typename decltype(ti)::type, typename decltype(te)::type, decltype(ac)::value>(x, illu, e, refl, enh,
+                                                                                                              n, h, w, eps, s);
+    });
 }
 
 template <typename T, bool AC>
@@ -482,8 +419,8 @@ int upr_retinex_recombine_f32(const float* x, const float* illu, const float* e,
     if (n == 0) return UPR_OK;
     if (!x || !illu || !e || !enh) return UPR_E_NULL;
     auto s = static_cast<cudaStream_t>(stream);
-    return refl ? upr::recombine_launch<float, false, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
-                : upr::recombine_launch<float, false, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
+    return refl ? upr::recombine_launch<float, float, false, true, true>(x, illu, e, refl, enh, n, h, w, eps, s)
+                : upr::recombine_launch<float, float, false, false, true>(x, illu, e, nullptr, enh, n, h, w, eps, s);
 }
 
 int upr_retinex_decompose_f32(const float* x, const float* illu, float* refl, int n, int h, int w, float eps,
@@ -492,8 +429,8 @@ int upr_retinex_decompose_f32(const float* x, const float* illu, float* refl, in
     if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
     if (n == 0) return UPR_OK;
     if (!x || !illu || !refl) return UPR_E_NULL;
-    return upr::recombine_launch<float, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps,
-                                                            static_cast<cudaStream_t>(stream));
+    return upr::recombine_launch<float, float, false, true, false>(x, illu, nullptr, refl, nullptr, n, h, w, eps,
+                                                                   static_cast<cudaStream_t>(stream));
 }
 
 int upr_retinex_recombine_maps(const float* x, const void* illu, const void* e, int map_dtype, int flags, float* refl,
@@ -503,17 +440,17 @@ int upr_retinex_recombine_maps(const float* x, const void* illu, const void* e, 
     if (map_dtype < UPR_DT_F32 || map_dtype > UPR_DT_BF16 || (flags & ~UPR_RETINEX_AUTOCAST)) return UPR_E_PARAM;
     if (n == 0) return UPR_OK;
     if (!x || !illu || (!refl && !enh) || (!e && enh)) return UPR_E_NULL;
-    auto s = static_cast<cudaStream_t>(stream);
-    const bool ac = flags & UPR_RETINEX_AUTOCAST;
-    switch (map_dtype) {
-    case UPR_DT_F32: return upr::recombine_maps<float, false>(x, illu, e, refl, enh, n, h, w, eps, s);
-    case UPR_DT_F16:
-        return ac ? upr::recombine_maps<__half, true>(x, illu, e, refl, enh, n, h, w, eps, s)
-                  : upr::recombine_maps<__half, false>(x, illu, e, refl, enh, n, h, w, eps, s);
-    default:
-        return ac ? upr::recombine_maps<__nv_bfloat16, true>(x, illu, e, refl, enh, n, h, w, eps, s)
-                  : upr::recombine_maps<__nv_bfloat16, false>(x, illu, e, refl, enh, n, h, w, eps, s);
-    }
+    return upr::recombine_typed(x, illu, map_dtype, e, map_dtype, flags, refl, enh, n, h, w, eps, static_cast<cudaStream_t>(stream));
+}
+
+int upr_retinex_recombine_typed(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                                float* refl, float* enh, int n, int h, int w, float eps, upr_stream_t stream)
+{
+    if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    if (!upr::valid_map_dtypes(illu_dtype, e_dtype, flags)) return UPR_E_PARAM;
+    if (n == 0) return UPR_OK;
+    if (!x || !illu || (!refl && !enh) || (!e && enh)) return UPR_E_NULL;
+    return upr::recombine_typed(x, illu, illu_dtype, e, e_dtype, flags, refl, enh, n, h, w, eps, static_cast<cudaStream_t>(stream));
 }
 
 int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,

@@ -121,8 +121,9 @@ class AdaptiveParameterAdjuster:
                 # recombination (models/model.py:405-413,442) fused into the CLAHE histogram kernel: the `enhanced` frame
                 # is never materialised; bit-identical to model(x)[0] -> apply_clahe_enhancement
                 illu_map, e_map = model.forward_maps(image_tensor)
+                # (maps from a CNN under the caller's torch.autocast: fp16 / bf16 e, with e**2 evaluated as autocast does)
                 enhanced_img = native.retinex_clahe(image_tensor.contiguous(), illu_map.contiguous(), e_map.contiguous(),
-                                                    self.CLIP_LIMIT, self.TILE_GRID)
+                                                    self.CLIP_LIMIT, self.TILE_GRID, autocast=torch.is_autocast_enabled("cuda"))
                 return enhanced_img, illu_map
             enhanced_img, _reflectance, illu_map = model(image_tensor)
         enhanced_img = native.clahe_lab(enhanced_img, self.CLIP_LIMIT, self.TILE_GRID)

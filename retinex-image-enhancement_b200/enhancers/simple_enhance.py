@@ -17,11 +17,14 @@ B200-first differences:
     silently drops them at :240) and, launched with one process per GPU (torchrun), shards the file list by rank and binds
     each rank to cuda:LOCAL_RANK -- frames are independent, there is no collective;
   * ``enhance_single_image`` accepts ``adjuster=`` (the reference's main.py:246 passes it and crashes on the missing
-    parameter).
+    parameter);
+  * ``amp="fp16"`` / ``"bf16"`` runs the CNN and the fused Retinex + CLAHE dispatch under ``torch.autocast("cuda")``; the
+    fp16 / bf16 maps go straight into the fused kernels (default None: f32, the reference's behaviour).
 File decoding / PNG encoding themselves stay PIL (an nvJPEG decode would not be bit-identical to the reference's).
 """
 from __future__ import annotations
 
+import contextlib
 import os
 import time
 from collections import deque
@@ -36,6 +39,16 @@ from .content_aware import ContentAwareEnhancer
 from .multi_scale import MultiScaleEnhancer
 
 VALID_EXTENSIONS = {".jpg", ".jpeg", ".png", ".bmp", ".tif", ".tiff"}
+AMP_DTYPES = {"fp16": torch.float16, "bf16": torch.bfloat16}
+
+
+def amp_context(amp):
+    """torch.autocast("cuda") in the dtype that ``amp`` names ("fp16" / "bf16"); no context for None."""
+    if amp is None:
+        return contextlib.nullcontext()
+    if amp not in AMP_DTYPES:
+        raise ValueError(f"amp must be None, 'fp16' or 'bf16', got {amp!r}")
+    return torch.autocast("cuda", dtype=AMP_DTYPES[amp])
 
 
 def bind_rank_to_gpu() -> str:
@@ -156,14 +169,15 @@ def enhance_frames_u8(model, low, enable_multi_scale=False, enable_content_aware
             if hasattr(model, "forward_maps") and not getattr(model, "training", False):
                 illu, e_map = model.forward_maps(low)
                 enh8 = native.retinex_clahe_u8(low.contiguous(), illu.contiguous(), e_map.contiguous(), adj.CLIP_LIMIT, adj.TILE_GRID,
-                                               out=out_enh)
+                                               out=out_enh, autocast=torch.is_autocast_enabled("cuda"))
             else:
                 enhanced, _refl, illu = model(low)
                 enh8 = native.clahe_lab_f32_u8(enhanced.contiguous(), adj.CLIP_LIMIT, adj.TILE_GRID, out=out_enh)
         else:
             enhanced, illu = _enhance_tensor(model, low, low.device, enable_multi_scale, enable_content_aware)
             enh8 = native.quantize_u8(enhanced.contiguous(), out=out_enh)
-        illu8 = native.quantize_u8(illu.contiguous(), out=out_illu)
+        # a map from a CNN under autocast is widened first, as _to_u8_hwc does
+        illu8 = native.quantize_u8(illu.to(torch.float32).contiguous(), out=out_illu)
     return enh8, illu8
 
 
@@ -252,12 +266,13 @@ def _write_outputs(img_low, img_enhanced, illu_map, image_path, output_dir, pool
 
 
 def enhance_single_image(model, image_path, output_dir, device, max_size=None, enable_multi_scale=False,
-                         enable_content_aware=False, adjuster=None):
+                         enable_content_aware=False, adjuster=None, amp=None):
     print(f"正在处理: {os.path.basename(image_path)}")
     device = resolve_device(device)
     img_low, _original_size = load_image(image_path, max_size, device=device)
     start = time.time()
-    img_enhanced, illu_map = _enhance_tensor(model, img_low, device, enable_multi_scale, enable_content_aware, adjuster)
+    with amp_context(amp):
+        img_enhanced, illu_map = _enhance_tensor(model, img_low, device, enable_multi_scale, enable_content_aware, adjuster)
     if img_enhanced.is_cuda:
         torch.cuda.synchronize(img_enhanced.device)
     print(f"增强耗时: {time.time() - start:.4f}s")
@@ -393,8 +408,9 @@ def run_batch_pipeline(files, output_dir, device, max_size, batch_size, frame_fn
 
 
 def enhance_batch_images(input_dir, output_dir, device, max_size=None, enable_multi_scale=False,
-                         enable_content_aware=False, batch_size=16, model=None, decode_workers=None, encode_workers=None):
+                         enable_content_aware=False, batch_size=16, model=None, decode_workers=None, encode_workers=None, amp=None):
     device = resolve_device(device)
+    amp_context(amp)   # an unknown amp fails before any file is read
     print("正在加载模型...")
     if model is None:
         model = UP_Retinex().to(device).eval()
@@ -415,12 +431,16 @@ def enhance_batch_images(input_dir, output_dir, device, max_size=None, enable_mu
         low = torch.from_numpy(arr).permute(2, 0, 1).to(torch.float32).div(255.0).unsqueeze(0)
         if max_size is not None:
             low = letterbox_tensor(low[0], new_shape=max_size, auto=True, scaleup=False)[0].unsqueeze(0)
-        enhanced, illu = _enhance_tensor(model, low, device, enable_multi_scale, enable_content_aware)
+        with amp_context(amp):
+            enhanced, illu = _enhance_tensor(model, low, device, enable_multi_scale, enable_content_aware)
         _write_outputs(low, enhanced, illu, path, output_dir)
 
-    run_batch_pipeline(mine, output_dir, device, max_size, batch_size,
-                       lambda low: enhance_frames_u8(model, low, enable_multi_scale, enable_content_aware), write_files, host_fn,
-                       decode_workers, encode_workers)
+    def frame_fn(low):
+        with amp_context(amp):   # entered by the thread that runs the batch (autocast state is per thread)
+            return enhance_frames_u8(model, low, enable_multi_scale, enable_content_aware)
+
+    run_batch_pipeline(mine, output_dir, device, max_size, batch_size, frame_fn, write_files, host_fn, decode_workers,
+                       encode_workers)
     total = time.time() - t0
     print("=" * 50)
     print(f"总共处理了 {len(mine)} 张图像")

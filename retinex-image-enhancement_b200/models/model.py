@@ -99,6 +99,8 @@ def retinex_decompose(x: torch.Tensor, illu: torch.Tensor) -> torch.Tensor:
         if _fused_autograd(x, illu):
             return _RetinexFn.apply(x, illu, None)
         return x / (illu + EPSILON)
+    if illu.dtype != torch.float32:   # a map from a CNN under autocast
+        return native.retinex_recombine_typed(x, illu, None, eps=EPSILON)[0]
     return native.retinex_decompose(x, illu, EPSILON)
 
 
@@ -110,6 +112,8 @@ def retinex_recombine(x: torch.Tensor, illu: torch.Tensor, enhancement_map: torc
     if needs_grad:   # training on other operands: autograd through the stock torch ops
         reflectance = x / (illu + EPSILON)
         return reflectance, reflectance * enhancement_map + (1 - reflectance) * (enhancement_map ** 2)
+    if illu.dtype != torch.float32 or enhancement_map.dtype != torch.float32:   # the maps of a CNN under autocast
+        return native.retinex_recombine_typed(x, illu, enhancement_map, autocast=torch.is_autocast_enabled("cuda"), eps=EPSILON)
     return native.retinex_recombine(x, illu, enhancement_map, want_reflectance=True, eps=EPSILON)
 
 

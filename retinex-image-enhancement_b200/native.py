@@ -47,6 +47,10 @@ def _declare(lib):
     lib.upr_retinex_clahe_f32.argtypes = [vp, vp, vp, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
     lib.upr_retinex_clahe_f32_u8.restype = i32
     lib.upr_retinex_clahe_f32_u8.argtypes = [vp, vp, vp, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
+    lib.upr_retinex_clahe_typed_f32.restype = i32
+    lib.upr_retinex_clahe_typed_f32.argtypes = [vp, vp, i32, vp, i32, i32, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
+    lib.upr_retinex_clahe_typed_u8.restype = i32
+    lib.upr_retinex_clahe_typed_u8.argtypes = [vp, vp, i32, vp, i32, i32, vp, i32, i32, i32, C.c_float, f64, i32, i32, vp, sz, vp]
     lib.upr_clahe_lab_stages_f32.restype = i32
     lib.upr_clahe_lab_stages_f32.argtypes = [vp, vp, i32, i32, i32, f64, i32, i32, vp, sz, i32, vp]
     lib.upr_clahe_debug_dump.restype = i32
@@ -95,6 +99,8 @@ def _declare(lib):
     lib.upr_retinex_decompose_f32.argtypes = [vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_recombine_maps.restype = i32
     lib.upr_retinex_recombine_maps.argtypes = [vp, vp, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
+    lib.upr_retinex_recombine_typed.restype = i32
+    lib.upr_retinex_recombine_typed.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_recombine_grad.restype = i32
     lib.upr_retinex_recombine_grad.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_letterbox_f32.restype = i32
@@ -288,8 +294,9 @@ def release_workspaces() -> None:
 def _clahe(entry: str, x: torch.Tensor, clip_limit: float, tiles: Tuple[int, int], out: Optional[torch.Tensor],
            u8_in: bool = False, u8_out: bool = False, retinex=None, extra=()) -> torch.Tensor:
     """The body of the CLAHE family.  x: [N,3,H,W] f32, or with u8_in [N,H,W,3] uint8 (packed RGB); out: [N,3,H,W] f32, or
-    with u8_out [N,H,W,3] uint8.  retinex = (illu, e, eps): CLAHE of the Retinex recombination of x, e and illu (the
-    upr_retinex_clahe_* entries).  extra: arguments of `entry` between the workspace and the stream."""
+    with u8_out [N,H,W,3] uint8.  retinex = (illu, e, eps, autocast): CLAHE of the Retinex recombination of x, e and illu (the
+    upr_retinex_clahe_* entries; `entry` is then the pair (f32 entry, _typed entry), the latter for maps that are not both
+    f32).  extra: arguments of `entry` between the workspace and the stream."""
     if u8_in:
         x = _cuda(x, "x", torch.uint8)
         if x.dim() != 4 or x.shape[3] != 3:      # a planar u8 tensor is not the decoded file this entry reads
@@ -301,19 +308,26 @@ def _clahe(entry: str, x: torch.Tensor, clip_limit: float, tiles: Tuple[int, int
     dev = x.device
     out = _out(out, (n, h, w, 3), torch.uint8, dev) if u8_out else _out(out, x.shape, torch.float32, dev)
     if retinex is not None:
-        illu, e, eps = retinex
-        illu = _cuda(illu, "illu", device=dev)
-        e = _cuda(e, "e", shape=x.shape, device=dev)
+        illu, e, eps, autocast = retinex
+        illu = _cuda(illu, "illu", tuple(MAP_DTYPES), device=dev)
+        e = _cuda(e, "e", tuple(MAP_DTYPES), shape=x.shape, device=dev)
         if illu.numel() != n * h * w:
             raise ValueError(f"illu must be [N,1,H,W], got {tuple(illu.shape)}")
+        typed = not (illu.dtype == e.dtype == torch.float32)
+        if typed:
+            _typed_map_dtypes(illu, e)
+        entry = entry[1] if typed else entry[0]
     tx, ty = int(tiles[0]), int(tiles[1])
     with _dev(dev):
         ws = _ws("upr_clahe_workspace_bytes", (n, h, w, tx, ty), dev)
         tail = (float(clip_limit), tx, ty, ws.data_ptr(), ws.numel(), *extra)
         if retinex is None:
             _run(entry, x.data_ptr(), out.data_ptr(), n, h, w, *tail)
-        else:
+        elif not typed:
             _run(entry, x.data_ptr(), illu.data_ptr(), e.data_ptr(), out.data_ptr(), n, h, w, float(eps), *tail)
+        else:
+            _run(entry, x.data_ptr(), illu.data_ptr(), MAP_DTYPES[illu.dtype], e.data_ptr(), MAP_DTYPES[e.dtype], int(bool(autocast)),
+                 out.data_ptr(), n, h, w, float(eps), *tail)
     return out
 
 
@@ -498,16 +512,22 @@ def scale_clamp(enh: torch.Tensor, gain: torch.Tensor, out: Optional[torch.Tenso
 
 
 def retinex_clahe(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, clip_limit: float = 2.0,
-                  tiles: Tuple[int, int] = (8, 8), eps: float = 1e-6, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                  tiles: Tuple[int, int] = (8, 8), eps: float = 1e-6, out: Optional[torch.Tensor] = None,
+                  autocast: bool = False) -> torch.Tensor:
     """CLAHE-in-Lab of the Retinex recombination R*e + (1-R)*e^2, R = x/(illu+eps), in one call (upr_retinex_clahe_f32):
-    the recombined frame is never materialised.  Bit-identical to retinex_recombine(...)[1] -> clahe_lab(...)."""
-    return _clahe("upr_retinex_clahe_f32", x, clip_limit, tiles, out, retinex=(illu, e, eps))
+    the recombined frame is never materialised.  Bit-identical to retinex_recombine(...)[1] -> clahe_lab(...).
+    The maps may also be what the CNN emits under autocast: e fp16 / bf16 and illu f32 or e's dtype
+    (upr_retinex_clahe_typed_f32), equal to the two lines in torch eager under torch.autocast("cuda", enabled=autocast)
+    followed by clahe_lab().  autocast: e**2 in f32 (as CUDA autocast runs pow) instead of in e's dtype."""
+    return _clahe(("upr_retinex_clahe_f32", "upr_retinex_clahe_typed_f32"), x, clip_limit, tiles, out, retinex=(illu, e, eps, autocast))
 
 
 def retinex_clahe_u8(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, clip_limit: float = 2.0,
-                     tiles: Tuple[int, int] = (8, 8), eps: float = 1e-6, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """retinex_clahe() emitting the packed u8 RGB frame [N,H,W,3] that save_image would store (upr_retinex_clahe_f32_u8)."""
-    return _clahe("upr_retinex_clahe_f32_u8", x, clip_limit, tiles, out, u8_out=True, retinex=(illu, e, eps))
+                     tiles: Tuple[int, int] = (8, 8), eps: float = 1e-6, out: Optional[torch.Tensor] = None,
+                     autocast: bool = False) -> torch.Tensor:
+    """retinex_clahe() emitting the packed u8 RGB frame [N,H,W,3] that save_image would store (upr_retinex_clahe_f32_u8, or
+    upr_retinex_clahe_typed_u8 for fp16 / bf16 maps)."""
+    return _clahe(("upr_retinex_clahe_f32_u8", "upr_retinex_clahe_typed_u8"), x, clip_limit, tiles, out, u8_out=True, retinex=(illu, e, eps, autocast))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -660,6 +680,33 @@ def retinex_recombine_maps(x: torch.Tensor, illu: torch.Tensor, e: Optional[torc
         _run("upr_retinex_recombine_maps", x.data_ptr(), illu.data_ptr(), e.data_ptr() if e is not None else None,
              MAP_DTYPES[illu.dtype], int(bool(autocast)), refl.data_ptr() if refl is not None else None,
              enh.data_ptr() if enh is not None else None, n, h, w, float(eps))
+    return refl, enh
+
+
+def _typed_map_dtypes(illu: torch.Tensor, e: Optional[torch.Tensor]) -> None:
+    """TypeError unless (illu, e) is a pair of map dtypes that the _typed entries take: e fp16 / bf16 (or f32) and illu f32 or
+    e's dtype."""
+    if e is not None and not (illu.dtype in (torch.float32, e.dtype)):
+        raise TypeError(f"illu must be float32 or e's dtype {e.dtype}, got {illu.dtype}")
+
+
+def retinex_recombine_typed(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], autocast: bool = False,
+                            want_reflectance: bool = True, eps: float = 1e-6):
+    """retinex_recombine_maps() with illu and e in their own dtypes, as the CNN emits them under autocast: e f32 / fp16 / bf16
+    and illu f32 or e's dtype (upr_retinex_recombine_typed); d = illu + eps is rounded to illu's dtype, e**2 to e's unless
+    autocast.  Forward only; e None = decompose only."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
+    n, _, h, w = x.shape
+    illu = _cuda(illu, "illu", tuple(MAP_DTYPES), shape=(n, 1, h, w), device=x.device)
+    if e is not None:
+        e = _cuda(e, "e", tuple(MAP_DTYPES), shape=x.shape, device=x.device)
+    _typed_map_dtypes(illu, e)
+    refl = torch.empty_like(x) if want_reflectance or e is None else None
+    enh = torch.empty_like(x) if e is not None else None
+    with _dev(x.device):
+        _run("upr_retinex_recombine_typed", x.data_ptr(), illu.data_ptr(), MAP_DTYPES[illu.dtype],
+             e.data_ptr() if e is not None else None, MAP_DTYPES[e.dtype if e is not None else illu.dtype], int(bool(autocast)),
+             refl.data_ptr() if refl is not None else None, enh.data_ptr() if enh is not None else None, n, h, w, float(eps))
     return refl, enh
 
 

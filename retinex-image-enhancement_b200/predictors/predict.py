@@ -13,7 +13,7 @@ import time
 import numpy as np
 import torch
 
-from ..enhancers.simple_enhance import _to_u8_hwc, list_images, load_image, save_image, shard_for_rank
+from ..enhancers.simple_enhance import AMP_DTYPES, _to_u8_hwc, amp_context, list_images, load_image, save_image, shard_for_rank
 from ..models.model import UP_Retinex
 
 
@@ -24,11 +24,12 @@ def create_comparison(img_low, img_enhanced, illu_map, save_path):
     print(f"Saved comparison: {save_path}")
 
 
-def predict_single_image(model, image_path, output_dir, device, max_size=None, save_comparison=True):
+def predict_single_image(model, image_path, output_dir, device, max_size=None, save_comparison=True, amp=None):
+    """amp: "fp16" / "bf16" runs the model under torch.autocast("cuda") (None: f32)."""
     img_low, _ = load_image(image_path, max_size, device=device)
     img_low = img_low.to(device)
     start = time.time()
-    with torch.no_grad():
+    with torch.no_grad(), amp_context(amp):
         img_enhanced, _reflectance, illu_map = model(img_low)
     if img_enhanced.is_cuda:
         torch.cuda.synchronize(img_enhanced.device)
@@ -41,12 +42,13 @@ def predict_single_image(model, image_path, output_dir, device, max_size=None, s
         create_comparison(img_low, img_enhanced, illu_map, os.path.join(output_dir, f"{stem}_comparison.png"))
 
 
-def predict_batch(model, input_dir, output_dir, device, max_size=None, save_comparison=True, batch_size=16):
+def predict_batch(model, input_dir, output_dir, device, max_size=None, save_comparison=True, batch_size=16, amp=None):
     """predict.py:186-235 over the batch pipeline of enhancers/simple_enhance.py (SURVEY 8f row N1): files are decoded ahead of
     the GPU, same-shaped frames run as one device batch (uint8 up, uint8 enhanced + illumination down), PNGs are encoded on a
     thread pool.  Same three files per image as predict_single_image."""
     from ..enhancers.simple_enhance import resolve_device, run_batch_pipeline
     from .. import native
+    amp_context(amp)   # an unknown amp fails before any file is read
     files = [f for f in list_images(input_dir) if os.path.splitext(f)[1].lower() in {".jpg", ".jpeg", ".png", ".bmp"}]
     if not files:
         print(f"No images found in {input_dir}")
@@ -57,9 +59,10 @@ def predict_batch(model, input_dir, output_dir, device, max_size=None, save_comp
     t0 = time.time()
 
     def frame_fn(low):
-        with torch.no_grad():
+        with torch.no_grad(), amp_context(amp):
             enhanced, _reflectance, illu = model(low)
-        return native.quantize_u8(enhanced.contiguous()), native.quantize_u8(illu.contiguous())
+        # a map from a CNN under autocast is widened first, as _to_u8_hwc does
+        return native.quantize_u8(enhanced.contiguous()), native.quantize_u8(illu.to(torch.float32).contiguous())
 
     def write_files(stem, low8, enh8, illu8):
         save_image(enh8, os.path.join(output_dir, f"{stem}_enhanced.png"))
@@ -68,7 +71,7 @@ def predict_batch(model, input_dir, output_dir, device, max_size=None, save_comp
             create_comparison(low8, enh8, illu8, os.path.join(output_dir, f"{stem}_comparison.png"))
 
     def host_fn(path, _arr):
-        predict_single_image(model, path, output_dir, device, max_size, save_comparison)
+        predict_single_image(model, path, output_dir, device, max_size, save_comparison, amp)
 
     run_batch_pipeline(mine, output_dir, device, max_size, batch_size, frame_fn, write_files, host_fn)
     total = time.time() - t0
@@ -106,6 +109,7 @@ def main(argv=None):
     p.add_argument("--max_size", type=int, default=None)
     p.add_argument("--no_comparison", action="store_true")
     p.add_argument("--device", type=str, default=None)
+    p.add_argument("--amp", type=str, default=None, choices=sorted(AMP_DTYPES), help="run the CNN under CUDA autocast")
     args = p.parse_args(argv)
     from ..enhancers.simple_enhance import bind_rank_to_gpu
     device = args.device or ("cuda" if torch.cuda.is_available() else "cpu")
@@ -117,9 +121,9 @@ def main(argv=None):
     if not os.path.exists(args.input):
         raise ValueError(f"Invalid input path: {args.input}")
     if os.path.isdir(args.input):
-        predict_batch(model, args.input, args.output, device, args.max_size, not args.no_comparison)
+        predict_batch(model, args.input, args.output, device, args.max_size, not args.no_comparison, amp=args.amp)
     else:
-        predict_single_image(model, args.input, args.output, device, args.max_size, not args.no_comparison)
+        predict_single_image(model, args.input, args.output, device, args.max_size, not args.no_comparison, amp=args.amp)
 
 
 if __name__ == "__main__":
