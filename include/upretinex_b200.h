@@ -248,6 +248,41 @@ UPR_API int upr_retinex_recombine_grad(const float* x, const void* illu, const v
                                        const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e,
                                        int n, int h, int w, float eps, upr_stream_t stream);
 
+/* ---- a5 / a7 / predict from the CNN maps -----------------------------------------------------------------------------------
+ * The content-aware, multi-scale and predict inference modes straight from the two CNN outputs: enh = R*f(e) + (1-R)*f(c) of
+ * upr_retinex_clahe_typed_f32 (same x, illu / illu_dtype, e / e_dtype, flags and eps; F32 / F32 included) is formed in registers
+ * inside the last pass of each mode, so neither R nor enh is written.  Status rules: UPR_E_SHAPE first, then UPR_E_PARAM for a
+ * dtype pair or flag the typed entries reject, then UPR_OK for n == 0, then UPR_E_NULL, then UPR_E_WORKSPACE.  The u8 results
+ * are what upr_quantize_u8_f32 makes of the f32 result: out_nhwc [n][h][w][3]; illu_nhw1 [n][h][w][1] (may be NULL) receives
+ * the quantised illumination map f(illu), the second frame the drivers store.  u8 outputs must not overlap an input.
+ *
+ * Content-aware (content_aware.py:105-120): out = clamp(enh * (1 + 0.2 att(x)), 0, 1), bit-identical to
+ * upr_retinex_recombine_typed followed by upr_content_aware_apply_f32.  workspace = upr_saliency_workspace_bytes(n, h, w);
+ * n <= 65535.  The f32 entry may run in place (out_nchw == x_nchw). */
+UPR_API int upr_retinex_content_aware_typed_f32(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw,
+                                                int e_dtype, int flags, float* out_nchw, int n, int h, int w, float eps,
+                                                void* workspace, size_t workspace_bytes, upr_stream_t stream);
+UPR_API int upr_retinex_content_aware_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw,
+                                               int e_dtype, int flags, unsigned char* out_nhwc, unsigned char* illu_nhw1, int n,
+                                               int h, int w, float eps, void* workspace, size_t workspace_bytes, upr_stream_t stream);
+/* Multi-scale (multi_scale.py:62-100 after the CNN): out = clamp(enh * gain[frame], 0, 1) with the statistics of x, means [n][3]
+ * and gain [n] written as by upr_multiscale_enhance_f32, whose schedule and workspace (upr_multiscale_workspace_bytes, zero-filled
+ * once) it shares.  Bit-identical to upr_retinex_recombine_typed followed by upr_multiscale_enhance_f32.  n <= 65535; h and w
+ * at least 4.  The f32 entry may run in place. */
+UPR_API int upr_retinex_multiscale_typed_f32(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw,
+                                             int e_dtype, int flags, float* out_nchw, float* means_n_by_3, float* gain_per_image,
+                                             int n, int h, int w, float eps, void* workspace, size_t workspace_bytes,
+                                             upr_stream_t stream);
+UPR_API int upr_retinex_multiscale_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw,
+                                            int e_dtype, int flags, unsigned char* out_nhwc, unsigned char* illu_nhw1,
+                                            float* means_n_by_3, float* gain_per_image, int n, int h, int w, float eps,
+                                            void* workspace, size_t workspace_bytes, upr_stream_t stream);
+/* Predict's stored pair (predictors/predict.py): enh_nhwc = quantise(enh), illu_nhw1 = quantise(f(illu)) in one pass,
+ * bit-identical to upr_retinex_recombine_typed followed by upr_quantize_u8_f32 of enh and of the widened illu. */
+UPR_API int upr_retinex_quantize_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw,
+                                          int e_dtype, int flags, unsigned char* enh_nhwc, unsigned char* illu_nhw1, int n, int h,
+                                          int w, float eps, upr_stream_t stream);
+
 /* ---- a9/a10: texture complexity and the dynamic smoothness weight ------------------------
  * losses/loss.py:523-583: per_image[i] = mean|dx| + mean|dy| ('tv') or the fraction of pixels whose Sobel
  * magnitude exceeds 1.5x its mean ('edge_density').  batch_stats2 (nullable) receives

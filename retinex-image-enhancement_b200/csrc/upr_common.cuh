@@ -176,6 +176,26 @@ __device__ __forceinline__ int quantize_u8(float x)
     return i & 0xff;
 }
 
+// ---------------------------------------------------------------------------------------
+// save_image's quantiser (enhancers/simple_enhance.py:65-100): (clip(v, 0, 1) * 255).astype(uint8) -- fp32 product,
+// truncation.  NaN clips to NaN and casts to 0 on the host; fmaxf(NaN, 0) = 0 gives the same byte here.  One definition for
+// upr_quantize_u8_f32 and every epilogue that emits the stored frame itself.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned save_u8(float v)
+{
+    return unsigned(__float2int_rz(__fmul_rn(fminf(fmaxf(v, 0.0f), 1.0f), 255.0f)));
+}
+// four bytes of four consecutive pixels of one plane, little-endian
+__device__ __forceinline__ unsigned pack4_u8(const unsigned (&q)[4]) { return q[0] | (q[1] << 8) | (q[2] << 16) | (q[3] << 24); }
+// four RGB pixels, q[channel][pixel], as the 12 interleaved bytes R0 G0 B0 R1 | G1 B1 R2 G2 | B2 R3 G3 B3 at a 4-byte aligned o
+__device__ __forceinline__ void st_rgb4_u8(unsigned char* o, const unsigned (&q)[3][4])
+{
+    unsigned* o32 = reinterpret_cast<unsigned*>(o);
+    o32[0] = q[0][0] | (q[1][0] << 8) | (q[2][0] << 16) | (q[0][1] << 24);
+    o32[1] = q[1][1] | (q[2][1] << 8) | (q[0][2] << 16) | (q[1][2] << 24);
+    o32[2] = q[2][2] | (q[0][3] << 8) | (q[1][3] << 16) | (q[2][3] << 24);
+}
+
 // u8 -> f32 without the (slower) conversion pipe: 0x4B000000 | b is 2^23 + b.
 __device__ __forceinline__ float byte_to_float(uint32_t word, int k)
 {

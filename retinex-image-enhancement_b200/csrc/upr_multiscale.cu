@@ -17,7 +17,7 @@
 // partials in index order (deterministic) and writes the three means and the gain.
 #include <algorithm>
 
-#include "upr_common.cuh"
+#include "upr_maps.cuh"
 #include <type_traits>
 
 namespace upr {
@@ -540,9 +540,48 @@ static int ms_run(const float* x, int n, int h, int w, float* means, float* gain
     return UPR_OK;
 }
 
+// upr_retinex_multiscale_typed_*: the schedule of upr_multiscale_enhance_f32 with the map epilogue in place of the gain pass
+static int ms_maps_run(const MapsArgs& m, float* means, float* gain, int n, int h, int w, void* ws, size_t ws_bytes, cudaStream_t s)
+{
+    if (n < 0 || n > 65535 || h <= 0 || w <= 0 || int(h * 0.25) < 1 || int(w * 0.25) < 1) return UPR_E_SHAPE;
+    bool done;
+    const int rc = maps_check(m, n, &done);
+    if (done) return rc;
+    if (!means || !gain || !ws) return UPR_E_NULL;
+    MsStreamGeom geo{};
+    if (!ms_stream_geometry(h, w, m.x, &geo)) {
+        const int rs = ms_run(m.x, n, h, w, means, gain, nullptr, nullptr, nullptr, ws, ws_bytes, s, true);
+        if (rs) return rs;
+        return maps_epilogue(m, n, h, w, FrameGain{gain}, s);
+    }
+    const long long plane = (long long)h * w;
+    return run_chunked(s, n, chunk_frames(plane), [&](int f0, int nf, cudaStream_t cs) {
+        const int rs = ms_stream_launch_range(m.x + f0 * 3 * plane, nf, h, w, geo, ws, ws_bytes, n, f0, means + 3 * f0, gain + f0, cs);
+        if (rs) return rs;
+        return maps_epilogue(m.at(f0, plane), nf, h, w, FrameGain{gain + f0}, cs);
+    });
+}
+
 }  // namespace upr
 
 extern "C" {
+
+int upr_retinex_multiscale_typed_f32(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                     int flags, float* out_nchw, float* means_n_by_3, float* gain_per_image, int n, int h, int w,
+                                     float eps, void* workspace, size_t workspace_bytes, upr_stream_t stream)
+{
+    const upr::MapsArgs m{x_nchw, illu_n1hw, illu_dtype, e_nchw, e_dtype, flags, eps, out_nchw, nullptr, nullptr};
+    return upr::ms_maps_run(m, means_n_by_3, gain_per_image, n, h, w, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int upr_retinex_multiscale_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                    int flags, unsigned char* out_nhwc, unsigned char* illu_nhw1, float* means_n_by_3,
+                                    float* gain_per_image, int n, int h, int w, float eps, void* workspace, size_t workspace_bytes,
+                                    upr_stream_t stream)
+{
+    const upr::MapsArgs m{x_nchw, illu_n1hw, illu_dtype, e_nchw, e_dtype, flags, eps, nullptr, out_nhwc, illu_nhw1};
+    return upr::ms_maps_run(m, means_n_by_3, gain_per_image, n, h, w, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
 
 size_t upr_multiscale_workspace_bytes(int n, int h, int w)
 {

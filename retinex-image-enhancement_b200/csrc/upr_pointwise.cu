@@ -19,12 +19,6 @@ namespace upr {
 constexpr int kPwThreads = 256;
 constexpr int kPwCtasPerSm = 8;
 
-__device__ __forceinline__ float clamp01_keep_nan(float v)
-{
-    // torch.clamp propagates NaN; fminf/fmaxf would not
-    return v < 0.0f ? 0.0f : (v > 1.0f ? 1.0f : v);
-}
-
 // ---- a8 ---------------------------------------------------------------------------------
 // plane4 = H*W/4 ; one work item = 4 consecutive pixels of one frame (all three channels).  TI / TE = storage types of illu / e
 // (upr_maps.cuh); d = illu + eps is rounded to TI, R and enhanced are f32 (type promotion).
@@ -344,8 +338,7 @@ int scale_clamp_launch(const float* enh, const float* gain, float* out, int n, i
 }
 
 // ---- save_image quantiser (enhancers/simple_enhance.py:65-100) -----------------------------------
-// [n][c][h][w] f32 -> [n][h][w][c] u8 with (clip(x, 0, 1) * 255).astype(uint8): fp32 product, truncation.  NaN clips to NaN and
-// casts to 0 on the host; fmaxf(NaN, 0) = 0 gives the same byte here.  c = 1 (illumination maps) or 3 (frames).  One thread
+// [n][c][h][w] f32 -> [n][h][w][c] u8 with save_u8 (upr_common.cuh).  c = 1 (illumination maps) or 3 (frames).  One thread
 // per 4 pixels: c 128-bit loads, 4c contiguous bytes stored.
 template <int C>
 __global__ void __launch_bounds__(kPwThreads)
@@ -361,17 +354,11 @@ k_quantize_u8(const float* __restrict__ x, unsigned char* __restrict__ out, long
             const float4 v = __ldcs(reinterpret_cast<const float4*>(x + (f * C + c) * plane) + p);
             const float a[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-            for (int k = 0; k < 4; ++k) q[c][k] = unsigned(__float2int_rz(__fmul_rn(fminf(fmaxf(a[k], 0.0f), 1.0f), 255.0f)));
+            for (int k = 0; k < 4; ++k) q[c][k] = save_u8(a[k]);
         }
         unsigned char* o = out + (f * plane + p * 4) * C;
-        if (C == 1) {
-            *reinterpret_cast<unsigned*>(o) = q[0][0] | (q[0][1] << 8) | (q[0][2] << 16) | (q[0][3] << 24);
-        } else {
-            unsigned* o32 = reinterpret_cast<unsigned*>(o);   // 12 bytes: R0 G0 B0 R1 | G1 B1 R2 G2 | B2 R3 G3 B3
-            o32[0] = q[0][0] | (q[1][0] << 8) | (q[2][0] << 16) | (q[0][1] << 24);
-            o32[1] = q[1][1] | (q[2][1] << 8) | (q[0][2] << 16) | (q[1][2] << 24);
-            o32[2] = q[2][2] | (q[0][3] << 8) | (q[1][3] << 16) | (q[2][3] << 24);
-        }
+        if constexpr (C == 1) *reinterpret_cast<unsigned*>(o) = pack4_u8(q[0]);
+        else st_rgb4_u8(o, q);
     }
 }
 
@@ -384,7 +371,7 @@ k_quantize_u8_scalar(const float* __restrict__ x, unsigned char* __restrict__ ou
         const long long f = it / plane, p = it - f * plane;
 #pragma unroll
         for (int c = 0; c < C; ++c)
-            out[it * C + c] = (unsigned char)__float2int_rz(__fmul_rn(fminf(fmaxf(x[(f * C + c) * plane + p], 0.0f), 1.0f), 255.0f));
+            out[it * C + c] = (unsigned char)save_u8(x[(f * C + c) * plane + p]);
     }
 }
 
@@ -410,6 +397,18 @@ int upr_quantize_u8_f32(const float* x_nchw, unsigned char* out_nhwc, int n, int
     }
     UPR_LAUNCH_CHECK();
     return UPR_OK;
+}
+
+int upr_retinex_quantize_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                  int flags, unsigned char* enh_nhwc, unsigned char* illu_nhw1, int n, int h, int w, float eps,
+                                  upr_stream_t stream)
+{
+    if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    const upr::MapsArgs m{x_nchw, illu_n1hw, illu_dtype, e_nchw, e_dtype, flags, eps, nullptr, enh_nhwc, illu_nhw1};
+    bool done;
+    const int rc = upr::maps_check(m, n, &done);
+    if (done) return rc;
+    return upr::maps_epilogue(m, n, h, w, upr::NoGain{}, static_cast<cudaStream_t>(stream));
 }
 
 int upr_retinex_recombine_f32(const float* x, const float* illu, const float* e, float* refl, float* enh, int n, int h,

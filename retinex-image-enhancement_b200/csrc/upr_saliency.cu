@@ -20,7 +20,7 @@
 
 #include <cuda_fp16.h>
 
-#include "upr_common.cuh"
+#include "upr_maps.cuh"
 
 namespace upr {
 
@@ -768,6 +768,30 @@ k_att_gain(const float* __restrict__ raw, const float* __restrict__ enh, float* 
     }
 }
 
+// The attention gain of the map epilogue: the k_att_gain<false, false> arithmetic over the raw attention plane and its min/max
+struct AttGain {
+    const float* raw;
+    const SalMinMax* mm;
+    long long plane;
+    static constexpr bool kApply = true;
+    struct Frame {
+        const float* r;
+        float mn, inv;
+        __device__ float gain(float a) const { return __fadd_rn(1.0f, __fmul_rn(0.2f, __fmul_rn(__fsub_rn(a, mn), inv))); }
+        __device__ float4 g4(long long q) const
+        {
+            const float4 t = __ldcs(reinterpret_cast<const float4*>(r) + q);
+            return make_float4(gain(t.x), gain(t.y), gain(t.z), gain(t.w));
+        }
+        __device__ float g1(long long p) const { return gain(r[p]); }
+    };
+    __device__ Frame frame(int f) const
+    {
+        const float mn = key_flt(mm[f].att_min), mx = key_flt(mm[f].att_max);
+        return {raw + f * plane, mn, att_inv_range(mn, mx)};
+    }
+};
+
 static GaussTapsF sal_taps_f()
 {
     // cv2.getGaussianKernel(15, sigma=0.3*((15-1)*0.5-1)+0.8 = 2.6) in fp64, rounded to fp32; t[d] = weight at distance d
@@ -788,8 +812,9 @@ static size_t sal_ws_bytes(int n, int h, int w)
 // mode 2: out = clamp(enh * (1 + 0.2 attention), 0, 1) with the attention map optional (att_out)
 // The passes of one (sub-)batch of n frames on stream s.  mm / blur: the min-max records and the intermediate plane of these frames.
 // lum_ok: the result frame may serve as luma scratch (mode 2, no aliasing with the inputs).
+// maps (mode 2): the result is the map epilogue of these frames (out is maps->out, enh is unused).
 static int sal_launch(int mode, const float* x, int n, int h, int w, float* out, SalMinMax* mm, float* blur, cudaStream_t s,
-                      const float* enh, float* att_out, const float* ms_gain, bool lum_ok)
+                      const float* enh, float* att_out, const float* ms_gain, bool lum_ok, const MapsArgs* maps)
 {
     const long long plane = (long long)h * w;
     k_sal_reset<<<(n + 127) / 128, 128, 0, s>>>(mm, n);
@@ -837,6 +862,7 @@ static int sal_launch(int mode, const float* x, int n, int h, int w, float* out,
         else if (v4) k_sal_normalize<true, 4><<<dim3(parts, n), kSalThreads, 0, s>>>(blur, x, blur, plane, mm);
         else k_sal_normalize<true, 1><<<dim3(parts, n), kSalThreads, 0, s>>>(blur, x, blur, plane, mm);
         UPR_LAUNCH_CHECK();
+        if (maps) return maps_epilogue(*maps, n, h, w, AttGain{blur, mm, plane}, s);
         const dim3 grid(parts, n);
 #define UPR_ATT_GAIN(A, G)                                                                                                     \
     do {                                                                                                                       \
@@ -872,31 +898,42 @@ struct MsJob {
     float* gain;        // [n]
 };
 
+// maps (mode 2): the content-aware result of the CNN maps -- pass 3 is the map epilogue with the attention gain; out must be
+// maps->out (NULL for the u8 result) and enh NULL.
 static int sal_run(int mode, const float* x, int n, int h, int w, float* out, void* ws, size_t ws_bytes, cudaStream_t s,
-                   const float* enh = nullptr, float* att_out = nullptr, const float* ms_gain = nullptr, const MsJob* ms = nullptr)
+                   const float* enh = nullptr, float* att_out = nullptr, const float* ms_gain = nullptr, const MsJob* ms = nullptr,
+                   const MapsArgs* maps = nullptr)
 {
     if (n < 0 || n > 65535 || h <= 0 || w <= 0) return UPR_E_SHAPE;
     if (n == 0) return UPR_OK;
-    if (!x || !out || !ws || (mode == 2 && !enh)) return UPR_E_NULL;
+    if (!x || !(out || maps) || !ws || (mode == 2 && !enh && !maps)) return UPR_E_NULL;
     if (ws_bytes < sal_ws_bytes(n, h, w) || (reinterpret_cast<uintptr_t>(ws) & 255u)) return UPR_E_WORKSPACE;
     auto* mm = static_cast<SalMinMax*>(ws);
     auto* blur = reinterpret_cast<float*>(static_cast<unsigned char*>(ws) + align_up(size_t(n) * sizeof(SalMinMax), 256));
     const long long plane = (long long)h * w;
-    bool lum_ok = false;
-    if (mode == 2) {    // the result frame is luma scratch between the passes unless it aliases an input (in-place apply)
-        const char *o0 = reinterpret_cast<const char*>(out), *o1 = o0 + size_t(n) * 3 * plane * sizeof(float);
-        auto overlaps = [&](const void* q) {
+    // lum_ok: the f32 result frame is luma scratch between the passes, which it may be unless it aliases an input (in-place
+    // apply).  chunk_ok: the frames may run chunk by chunk on the side streams.  A u8 result cannot hold luma (3 < 4 B/px) and
+    // aliases no f32 input, so it chunks without the scratch.
+    bool lum_ok = false, chunk_ok = true;
+    if (mode == 2 && out) {
+        const size_t frame_bytes = size_t(n) * 3 * plane * sizeof(float);
+        const char *o0 = reinterpret_cast<const char*>(out), *o1 = o0 + frame_bytes;
+        auto overlaps = [&](const void* q, size_t bytes) {
             const char* q0 = reinterpret_cast<const char*>(q);
-            return q0 < o1 && q0 + size_t(n) * 3 * plane * sizeof(float) > o0;
+            return q0 < o1 && q0 + bytes > o0;
         };
-        lum_ok = !overlaps(enh) && !overlaps(x);
+        lum_ok = !overlaps(x, frame_bytes) &&
+                 (maps ? !overlaps(maps->illu, size_t(n) * plane * map_dtype_bytes(maps->illu_dt)) &&
+                             !overlaps(maps->e, frame_bytes / sizeof(float) * map_dtype_bytes(maps->e_dt))
+                       : !overlaps(enh, frame_bytes));
+        chunk_ok = lum_ok;
     }
     // Chunked schedule: the three passes of a chunk of ~25 Mpx run back to back on one of two side streams, consecutive chunks on
     // alternating streams.  The 4-8 B/px intermediate of a chunk (~100-200 MB) is then re-read while part of it is still in L2, and
     // the passes of neighbouring chunks overlap.  Measured on 16 x 4K / 64 x 1080p: 1.39 -> 1.28-1.30 ms (profiles/r4_content_aware.md;
     // single-frame chunks lose more to short kernels than they gain).  Results do not depend on the schedule: every frame is
-    // normalised on its own.  An in-place apply (!lum_ok) runs as one chunk.
-    const int chunk = (mode != 2 || lum_ok) ? chunk_frames(plane) : n;
+    // normalised on its own.  An in-place apply (!chunk_ok) runs as one chunk.
+    const int chunk = chunk_ok ? chunk_frames(plane) : n;
     const long long step_x = 3 * plane, step_p = plane;
     return run_chunked(s, n, chunk, [&](int f0, int nf, cudaStream_t cs) {
         if (ms) {
@@ -904,9 +941,10 @@ static int sal_run(int mode, const float* x, int n, int h, int w, float* out, vo
                                                   ms->gain + f0, cs);
             if (rc != UPR_OK) return rc;
         }
-        return sal_launch(mode, x + f0 * step_x, nf, h, w, out + f0 * (mode == 2 ? step_x : step_p), mm + f0, blur + f0 * step_p, cs,
-                          enh ? enh + f0 * step_x : nullptr, att_out ? att_out + f0 * step_p : nullptr, ms_gain ? ms_gain + f0 : nullptr,
-                          lum_ok);
+        const MapsArgs mf = maps ? maps->at(f0, plane) : MapsArgs{};
+        return sal_launch(mode, x + f0 * step_x, nf, h, w, out ? out + f0 * (mode == 2 ? step_x : step_p) : nullptr, mm + f0,
+                          blur + f0 * step_p, cs, enh ? enh + f0 * step_x : nullptr, att_out ? att_out + f0 * step_p : nullptr,
+                          ms_gain ? ms_gain + f0 : nullptr, lum_ok, maps ? &mf : nullptr);
     });
 }
 
@@ -954,6 +992,32 @@ int upr_content_multiscale_f32(const float* x_nchw, const float* enh_nchw, float
     }
     const upr::MsJob job{geo, ms_workspace, ms_workspace_bytes, means_n_by_3, gain_per_image};
     return upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, s, enh_nchw, att_n1hw, gain_per_image, &job);
+}
+
+int upr_retinex_content_aware_typed_f32(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                        int flags, float* out_nchw, int n, int h, int w, float eps, void* workspace,
+                                        size_t workspace_bytes, upr_stream_t stream)
+{
+    if (n < 0 || n > 65535 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    const upr::MapsArgs m{x_nchw, illu_n1hw, illu_dtype, e_nchw, e_dtype, flags, eps, out_nchw, nullptr, nullptr};
+    bool done;
+    const int rc = upr::maps_check(m, n, &done);
+    if (done) return rc;
+    return upr::sal_run(2, x_nchw, n, h, w, out_nchw, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), nullptr, nullptr,
+                        nullptr, nullptr, &m);
+}
+
+int upr_retinex_content_aware_typed_u8(const float* x_nchw, const void* illu_n1hw, int illu_dtype, const void* e_nchw, int e_dtype,
+                                       int flags, unsigned char* out_nhwc, unsigned char* illu_nhw1, int n, int h, int w, float eps,
+                                       void* workspace, size_t workspace_bytes, upr_stream_t stream)
+{
+    if (n < 0 || n > 65535 || h <= 0 || w <= 0) return UPR_E_SHAPE;
+    const upr::MapsArgs m{x_nchw, illu_n1hw, illu_dtype, e_nchw, e_dtype, flags, eps, nullptr, out_nhwc, illu_nhw1};
+    bool done;
+    const int rc = upr::maps_check(m, n, &done);
+    if (done) return rc;
+    return upr::sal_run(2, x_nchw, n, h, w, nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), nullptr, nullptr,
+                        nullptr, nullptr, &m);
 }
 
 int upr_content_multiscale_apply_f32(const float* x_nchw, const float* enh_nchw, const float* ms_gain_per_image, float* out_nchw,

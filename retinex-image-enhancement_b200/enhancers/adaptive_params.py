@@ -41,6 +41,16 @@ def _to_device(image_tensor: torch.Tensor, device=None) -> torch.Tensor:
     return image_tensor.detach().to(device=dev, dtype=torch.float32, non_blocking=True)
 
 
+def cnn_maps(model, image_tensor: torch.Tensor):
+    """(illu, e) = model.forward_maps(x) for the inference modes that take the CNN maps straight into their last pass: a model
+    with forward_maps that is not training, a CUDA input, and maps the native *_typed entries accept.  None otherwise, and the
+    caller runs model(x) as before (for maps in a pair those entries do not take, that is a second forward pass)."""
+    if not (image_tensor.is_cuda and hasattr(model, "forward_maps") and not getattr(model, "training", False)):
+        return None
+    illu, e = model.forward_maps(image_tensor)
+    return (illu.contiguous(), e.contiguous()) if native.maps_supported(image_tensor, illu, e) else None
+
+
 class AdaptiveParameterAdjuster:
     """Image-statistics driven parameter selection plus the CLAHE-in-Lab post-enhancer."""
 

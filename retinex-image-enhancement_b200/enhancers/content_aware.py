@@ -17,7 +17,7 @@ from __future__ import annotations
 import torch
 
 from .. import native
-from .adaptive_params import _as_batch, _to_device
+from .adaptive_params import _as_batch, _to_device, cnn_maps
 
 
 class ContentAwareEnhancer:
@@ -35,6 +35,13 @@ class ContentAwareEnhancer:
     def apply_content_aware_enhancement(self, model, image_tensor, device):
         image_tensor = _to_device(_as_batch(image_tensor), device)
         with torch.no_grad():
+            maps = cnn_maps(model, image_tensor)
+            if maps is not None:
+                # the Retinex recombination formed in the attention pass: R and enhanced are never written; bit-identical to
+                # model(x)[0] -> content_aware_apply (under the caller's torch.autocast too)
+                illu_map, e_map = maps
+                return native.retinex_content_aware(image_tensor.contiguous(), illu_map, e_map,
+                                                    autocast=torch.is_autocast_enabled("cuda")), illu_map
             enhanced_img, _reflectance, illu_map = model(image_tensor)
         # attention map + gain + clamp in three passes over the frame (the map itself is not materialised)
         return native.content_aware_apply(image_tensor, enhanced_img.contiguous()), illu_map

@@ -15,7 +15,7 @@ from __future__ import annotations
 import torch
 
 from .. import native
-from .adaptive_params import _as_batch, _to_device
+from .adaptive_params import _as_batch, _to_device, cnn_maps
 
 
 class MultiScaleEnhancer:
@@ -37,6 +37,13 @@ class MultiScaleEnhancer:
     def apply_multi_scale_enhancement(self, model, image_tensor, device):
         image_tensor = _to_device(_as_batch(image_tensor), device)
         with torch.no_grad():
+            maps = cnn_maps(model, image_tensor)
+            if maps is not None:
+                # the Retinex recombination formed in the gain pass; bit-identical to model(x)[0] -> multiscale_enhance
+                illu_map, e_map = maps
+                out, _means, _gain = native.retinex_multiscale(image_tensor.contiguous(), illu_map, e_map,
+                                                               autocast=torch.is_autocast_enabled("cuda"))
+                return out, illu_map
             enhanced_img, _reflectance, illu_map = model(image_tensor)
         # statistics of the input + gain/clamp of the CNN output in one call (chunked on two streams for large batches)
         out, _means, _gain = native.multiscale_enhance(image_tensor, enhanced_img.contiguous())

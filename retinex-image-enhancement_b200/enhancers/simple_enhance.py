@@ -34,7 +34,7 @@ import torch
 
 from ..models.model import UP_Retinex
 from ..utils.letterbox import letterbox_geometry, letterbox_tensor
-from .adaptive_params import AdaptiveParameterAdjuster
+from .adaptive_params import AdaptiveParameterAdjuster, cnn_maps
 from .content_aware import ContentAwareEnhancer
 from .multi_scale import MultiScaleEnhancer
 
@@ -174,6 +174,12 @@ def enhance_frames_u8(model, low, enable_multi_scale=False, enable_content_aware
                 enhanced, _refl, illu = model(low)
                 enh8 = native.clahe_lab_f32_u8(enhanced.contiguous(), adj.CLIP_LIMIT, adj.TILE_GRID, out=out_enh)
         else:
+            maps = cnn_maps(model, low)
+            if maps is not None:
+                # both stored frames from the mode's last pass (content-aware wins when both flags are set, as in
+                # _enhance_tensor); the illumination frame is the widened map quantised, as below
+                fn = native.retinex_content_aware_u8 if enable_content_aware else native.retinex_multiscale_u8
+                return fn(low.contiguous(), *maps, autocast=torch.is_autocast_enabled("cuda"), out=out_enh, out_illu=out_illu)
             enhanced, illu = _enhance_tensor(model, low, low.device, enable_multi_scale, enable_content_aware)
             enh8 = native.quantize_u8(enhanced.contiguous(), out=out_enh)
         # a map from a CNN under autocast is widened first, as _to_u8_hwc does

@@ -101,6 +101,16 @@ def _declare(lib):
     lib.upr_retinex_recombine_maps.argtypes = [vp, vp, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_recombine_typed.restype = i32
     lib.upr_retinex_recombine_typed.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
+    lib.upr_retinex_content_aware_typed_f32.restype = i32
+    lib.upr_retinex_content_aware_typed_f32.argtypes = [vp, vp, i32, vp, i32, i32, vp, i32, i32, i32, f32, vp, sz, vp]
+    lib.upr_retinex_content_aware_typed_u8.restype = i32
+    lib.upr_retinex_content_aware_typed_u8.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp, sz, vp]
+    lib.upr_retinex_multiscale_typed_f32.restype = i32
+    lib.upr_retinex_multiscale_typed_f32.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp, i32, i32, i32, f32, vp, sz, vp]
+    lib.upr_retinex_multiscale_typed_u8.restype = i32
+    lib.upr_retinex_multiscale_typed_u8.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, f32, vp, sz, vp]
+    lib.upr_retinex_quantize_typed_u8.restype = i32
+    lib.upr_retinex_quantize_typed_u8.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_recombine_grad.restype = i32
     lib.upr_retinex_recombine_grad.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_letterbox_f32.restype = i32
@@ -708,6 +718,107 @@ def retinex_recombine_typed(x: torch.Tensor, illu: torch.Tensor, e: Optional[tor
              e.data_ptr() if e is not None else None, MAP_DTYPES[e.dtype if e is not None else illu.dtype], int(bool(autocast)),
              refl.data_ptr() if refl is not None else None, enh.data_ptr() if enh is not None else None, n, h, w, float(eps))
     return refl, enh
+
+
+# ------------------------------------------------------------------------------------------------
+# a5 / a7 / predict straight from the CNN maps (x, illu, e): the recombination formed inside the last pass
+# ------------------------------------------------------------------------------------------------
+def maps_supported(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor) -> bool:
+    """Whether the *_maps entries below take these operands: CUDA tensors and a (illu, e) dtype pair of the _typed entries."""
+    return (x.is_cuda and illu.is_cuda and e.is_cuda and x.dtype == torch.float32 and e.dtype in MAP_DTYPES
+            and illu.dtype in (torch.float32, e.dtype))
+
+
+def _typed_maps(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor):
+    """The checked operands of the maps entries: x [N,3,H,W] f32, illu [N,1,H,W], e [N,3,H,W] in a pair of the _typed entries,
+    and the entries' leading dtype arguments."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
+    n, _, h, w = x.shape
+    illu = _cuda(illu, "illu", tuple(MAP_DTYPES), shape=(n, 1, h, w), device=x.device)
+    e = _cuda(e, "e", tuple(MAP_DTYPES), shape=x.shape, device=x.device)
+    _typed_map_dtypes(illu, e)
+    return x, illu, e, (x.data_ptr(), illu.data_ptr(), MAP_DTYPES[illu.dtype], e.data_ptr(), MAP_DTYPES[e.dtype])
+
+
+def _u8_pair(x: torch.Tensor, out: Optional[torch.Tensor], out_illu: Optional[torch.Tensor]):
+    n, _, h, w = x.shape
+    return _out(out, (n, h, w, 3), torch.uint8, x.device), _out(out_illu, (n, h, w, 1), torch.uint8, x.device)
+
+
+def retinex_content_aware(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, autocast: bool = False, eps: float = 1e-6,
+                          out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """clamp(enh * (1 + 0.2 * attention(x)), 0, 1) with enh the Retinex recombination of x, illu and e formed in the attention
+    pass (upr_retinex_content_aware_typed_f32): bit-identical to retinex_recombine_typed(...)[1] -> content_aware_apply().
+    Maps as for retinex_clahe(); out may be x."""
+    x, illu, e, head = _typed_maps(x, illu, e)
+    n, _, h, w = x.shape
+    out = _out(out, x.shape, torch.float32, x.device)
+    with _dev(x.device):
+        ws = _ws("upr_saliency_workspace_bytes", (n, h, w), x.device)
+        _run("upr_retinex_content_aware_typed_f32", *head, int(bool(autocast)), out.data_ptr(), n, h, w, float(eps), ws.data_ptr(),
+             ws.numel())
+    return out
+
+
+def retinex_content_aware_u8(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, autocast: bool = False, eps: float = 1e-6,
+                             out: Optional[torch.Tensor] = None, out_illu: Optional[torch.Tensor] = None):
+    """retinex_content_aware() as the two frames the drivers store: (quantize_u8 of the result [N,H,W,3], quantize_u8 of
+    illu.float() [N,H,W,1]) from one call (upr_retinex_content_aware_typed_u8)."""
+    x, illu, e, head = _typed_maps(x, illu, e)
+    n, _, h, w = x.shape
+    out, out_illu = _u8_pair(x, out, out_illu)
+    with _dev(x.device):
+        ws = _ws("upr_saliency_workspace_bytes", (n, h, w), x.device)
+        _run("upr_retinex_content_aware_typed_u8", *head, int(bool(autocast)), out.data_ptr(), out_illu.data_ptr(), n, h, w,
+             float(eps), ws.data_ptr(), ws.numel())
+    return out, out_illu
+
+
+def _ms_maps(entry: str, x, illu, e, autocast, eps, outs):
+    x, illu, e, head = _typed_maps(x, illu, e)
+    n, _, h, w = x.shape
+    if int(h * 0.25) < 1 or int(w * 0.25) < 1:
+        raise ValueError("image too small for the 1/4 scale")
+    means = torch.empty((n, 3), dtype=torch.float32, device=x.device)
+    gain = torch.empty((n,), dtype=torch.float32, device=x.device)
+    with _dev(x.device):
+        ws = _ws("upr_multiscale_workspace_bytes", (n, h, w), x.device, "ms")
+        _run(entry, *head, int(bool(autocast)), *(o.data_ptr() for o in outs), means.data_ptr(), gain.data_ptr(), n, h, w, float(eps),
+             ws.data_ptr(), ws.numel())
+    return means, gain
+
+
+def retinex_multiscale(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, autocast: bool = False, eps: float = 1e-6,
+                       out: Optional[torch.Tensor] = None):
+    """clamp(enh * gain(x)[frame], 0, 1) with enh the Retinex recombination formed in the gain pass
+    (upr_retinex_multiscale_typed_f32) -> (out, means [N,3], gain [N]): bit-identical to retinex_recombine_typed(...)[1] ->
+    multiscale_enhance().  Maps as for retinex_clahe(); out may be x."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
+    out = _out(out, x.shape, torch.float32, x.device)
+    means, gain = _ms_maps("upr_retinex_multiscale_typed_f32", x, illu, e, autocast, eps, (out,))
+    return out, means, gain
+
+
+def retinex_multiscale_u8(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, autocast: bool = False, eps: float = 1e-6,
+                          out: Optional[torch.Tensor] = None, out_illu: Optional[torch.Tensor] = None):
+    """retinex_multiscale() as the two stored frames (enh8 [N,H,W,3], illu8 [N,H,W,1]) from one call
+    (upr_retinex_multiscale_typed_u8)."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
+    out, out_illu = _u8_pair(x, out, out_illu)
+    _ms_maps("upr_retinex_multiscale_typed_u8", x, illu, e, autocast, eps, (out, out_illu))
+    return out, out_illu
+
+
+def retinex_quantize_u8(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, autocast: bool = False, eps: float = 1e-6,
+                        out: Optional[torch.Tensor] = None, out_illu: Optional[torch.Tensor] = None):
+    """predict's stored pair in one pass (upr_retinex_quantize_typed_u8): (quantize_u8 of the Retinex recombination [N,H,W,3],
+    quantize_u8 of illu.float() [N,H,W,1])."""
+    x, illu, e, head = _typed_maps(x, illu, e)
+    n, _, h, w = x.shape
+    out, out_illu = _u8_pair(x, out, out_illu)
+    with _dev(x.device):
+        _run("upr_retinex_quantize_typed_u8", *head, int(bool(autocast)), out.data_ptr(), out_illu.data_ptr(), n, h, w, float(eps))
+    return out, out_illu
 
 
 def retinex_recombine_grad(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], g_enh: Optional[torch.Tensor],

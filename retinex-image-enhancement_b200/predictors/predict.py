@@ -13,6 +13,7 @@ import time
 import numpy as np
 import torch
 
+from ..enhancers.adaptive_params import cnn_maps
 from ..enhancers.simple_enhance import AMP_DTYPES, _to_u8_hwc, amp_context, list_images, load_image, save_image, shard_for_rank
 from ..models.model import UP_Retinex
 
@@ -60,6 +61,10 @@ def predict_batch(model, input_dir, output_dir, device, max_size=None, save_comp
 
     def frame_fn(low):
         with torch.no_grad(), amp_context(amp):
+            maps = cnn_maps(model, low)
+            if maps is not None:
+                # both stored frames in one pass over x and the maps: R and enhanced are never written
+                return native.retinex_quantize_u8(low.contiguous(), *maps, autocast=torch.is_autocast_enabled("cuda"))
             enhanced, _reflectance, illu = model(low)
         # a map from a CNN under autocast is widened first, as _to_u8_hwc does
         return native.quantize_u8(enhanced.contiguous()), native.quantize_u8(illu.to(torch.float32).contiguous())
