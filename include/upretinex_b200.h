@@ -247,6 +247,17 @@ UPR_API int upr_retinex_recombine_typed(const float* x, const void* illu, int il
 UPR_API int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
                                        const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e,
                                        int n, int h, int w, float eps, upr_stream_t stream);
+/* The gradient of upr_retinex_recombine_typed: illu and e in separate dtypes, with illu_dtype, e_dtype and flags accepted and
+ * rejected (UPR_E_PARAM) as there; NULL and status rules, d, R and c recomputation as for upr_retinex_recombine_grad, which is
+ * this entry with illu_dtype == e_dtype.  g_illu is written in illu's dtype TI, g_e in e's dtype TE.  With illu f32 and e
+ * fp16 / bf16 (the maps of the CNN under CUDA autocast) the formulas above read, nothing on the illumination side rounded:
+ *   forward   d = f(illu) + eps;  R = x / d;  c = f(e)*f(e) (f32 under UPR_RETINEX_AUTOCAST, else TE(.));  enh = R*f(e) + (1-R)*c
+ *   gradient  gRt as above;  g_x = gRt / d;  g_illu = ((0 + gd0) + gd1) + gd2 in f32
+ *             g_e = TE(f(TE(gE*R)) + f(TE(gc * 2*f(e))))  with gc = gE*(1-R) in f32 under UPR_RETINEX_AUTOCAST;
+ *                   without the flag gc and 2*f(e) are rounded to TE and their product to TE as for upr_retinex_recombine_grad */
+UPR_API int upr_retinex_recombine_grad_typed(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                                             const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e,
+                                             int n, int h, int w, float eps, upr_stream_t stream);
 
 /* ---- a5 / a7 / predict from the CNN maps -----------------------------------------------------------------------------------
  * The content-aware, multi-scale and predict inference modes straight from the two CNN outputs: enh = R*f(e) + (1-R)*f(c) of

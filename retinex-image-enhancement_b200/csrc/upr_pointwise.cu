@@ -90,14 +90,15 @@ k_recombine_scalar(const float* __restrict__ x, const TI* __restrict__ illu, con
 // What torch autograd computes for the two lines, recomputing d, R and e^2 from the inputs (nothing is saved by the forward).
 // gRt, the gradient reaching R, accumulates in the order the autograd engine adds its parts: g_refl (from R's consumers, which
 // run first) onto -(gE*c) (rsub), then gE*e (the R*e product, created first, runs last).  The e gradient sums the R*e
-// branch, rounded to T, and the e^2 branch, rounded to T once (in T arithmetic without autocast; by the fp32 cast's backward
-// under autocast).  The illu gradient is the channel sum of div's "other" gradient in f32 (torch's sum starts from 0),
-// then rounded to T.
+// branch, rounded to TE, and the e^2 branch, rounded to TE once (in TE arithmetic without autocast; by the fp32 cast's
+// backward under autocast).  The illu gradient is the channel sum of div's "other" gradient in f32 (torch's sum starts from
+// 0), then rounded to TI (not at all for the f32 illumination map the network emits under autocast).  grad1 sees the
+// illumination side only through d, so it is typed on e's dtype alone.
 struct GradPx {
     float gx, ge, gd;
 };
 
-template <typename T, bool kAutocast>
+template <typename TE, bool kAutocast>
 __device__ __forceinline__ GradPx grad1(float x, float d, float e, float gE, float gR, bool has_gE, bool has_gR)
 {
     const float r = __fdiv_rn(x, d);
@@ -106,13 +107,13 @@ __device__ __forceinline__ GradPx grad1(float x, float d, float e, float gE, flo
     GradPx o;
     o.ge = 0.0f;
     if (has_gE) {
-        const float c = square<T, kAutocast>(e);
+        const float c = square<TE, kAutocast>(e);
         const float t = -__fmul_rn(gE, c);
         g = __fadd_rn(has_gR ? __fadd_rn(t, gR) : t, __fmul_rn(gE, e));
         float gc = __fmul_rn(gE, __fsub_rn(1.0f, r));
-        if (!kAutocast) gc = rnd<T>(gc);
-        const float two_e = kAutocast ? __fmul_rn(2.0f, e) : rnd<T>(__fmul_rn(2.0f, e));
-        o.ge = __fadd_rn(rnd<T>(__fmul_rn(gE, r)), rnd<T>(__fmul_rn(gc, two_e)));
+        if (!kAutocast) gc = rnd<TE>(gc);
+        const float two_e = kAutocast ? __fmul_rn(2.0f, e) : rnd<TE>(__fmul_rn(2.0f, e));
+        o.ge = __fadd_rn(rnd<TE>(__fmul_rn(gE, r)), rnd<TE>(__fmul_rn(gc, two_e)));
     }
     o.gx = __fdiv_rn(g, d);
     o.gd = __fmul_rn(-g, q);
@@ -125,11 +126,11 @@ __device__ __forceinline__ GradPx grad1(float x, float d, float e, float gE, flo
 // the division slow path; it needs 72 (3 CTAs per SM).  The grid stays pw_grid's 148 x 8 CTAs: the later ones start as earlier
 // ones finish and keep more loads in flight; a one-wave grid of 148 x 3 measured slower (32x3x640^2: 0.32 -> 0.35 ms f32,
 // 0.32 -> 0.37 ms fp16; the same at 16x1080p)
-template <typename T, bool kAutocast>
+template <typename TI, typename TE, bool kAutocast>
 __global__ void __launch_bounds__(kPwThreads, 1)
-k_recombine_grad_vec(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+k_recombine_grad_vec(const float* __restrict__ x, const TI* __restrict__ illu, const TE* __restrict__ e,
                      const float* __restrict__ g_enh, const float* __restrict__ g_refl, float* __restrict__ g_x,
-                     T* __restrict__ g_illu, T* __restrict__ g_e, long long plane4, long long items, float eps)
+                     TI* __restrict__ g_illu, TE* __restrict__ g_e, long long plane4, long long items, float eps)
 {
     const uint64_t pol = policy_evict_first();
     const long long stride = (long long)gridDim.x * kPwThreads;
@@ -138,16 +139,15 @@ k_recombine_grad_vec(const float* __restrict__ x, const T* __restrict__ illu, co
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane4, p = it - f * plane4;
         const long long o3 = (f * 3 * plane4 + p) * 4, o1 = (f * plane4 + p) * 4;
-        const float4 il = MapIO<T>::ld4(illu + o1, pol);
-        const float d[4] = {rnd<T>(__fadd_rn(il.x, eps)), rnd<T>(__fadd_rn(il.y, eps)), rnd<T>(__fadd_rn(il.z, eps)),
-                            rnd<T>(__fadd_rn(il.w, eps))};
+        const float4 il = MapIO<TI>::ld4(illu + o1, pol);
+        const float d[4] = {illu_eps<TI>(il.x, eps), illu_eps<TI>(il.y, eps), illu_eps<TI>(il.z, eps), illu_eps<TI>(il.w, eps)};
         // one channel at a time: what stays live across the division slow path fits the callee-saved registers (no spills)
         float gd[4];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const long long o = o3 + c * plane4 * 4;
             const float4 xv = ld_stream_f4(x + o, pol);
-            const float4 ev = has_gE ? MapIO<T>::ld4(e + o, pol) : zero;
+            const float4 ev = has_gE ? MapIO<TE>::ld4(e + o, pol) : zero;
             const float4 gev = has_gE ? ld_stream_f4(g_enh + o, pol) : zero;
             const float4 grv = has_gR ? ld_stream_f4(g_refl + o, pol) : zero;
             const float xs[4] = {xv.x, xv.y, xv.z, xv.w}, es[4] = {ev.x, ev.y, ev.z, ev.w};
@@ -155,40 +155,40 @@ k_recombine_grad_vec(const float* __restrict__ x, const T* __restrict__ illu, co
             float gx[4], ge[4];
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                const GradPx g = grad1<T, kAutocast>(xs[k], d[k], es[k], gEs[k], gRs[k], has_gE, has_gR);
+                const GradPx g = grad1<TE, kAutocast>(xs[k], d[k], es[k], gEs[k], gRs[k], has_gE, has_gR);
                 gx[k] = g.gx;
                 ge[k] = g.ge;
                 gd[k] = c == 0 ? __fadd_rn(0.0f, g.gd) : __fadd_rn(gd[k], g.gd);
             }
             if (g_x) st_stream_f4(g_x + o, make_float4(gx[0], gx[1], gx[2], gx[3]), pol);
-            if (g_e) MapIO<T>::st4(g_e + o, make_float4(ge[0], ge[1], ge[2], ge[3]), pol);
+            if (g_e) MapIO<TE>::st4(g_e + o, make_float4(ge[0], ge[1], ge[2], ge[3]), pol);
         }
-        if (g_illu) MapIO<T>::st4(g_illu + o1, make_float4(gd[0], gd[1], gd[2], gd[3]), pol);
+        if (g_illu) MapIO<TI>::st4(g_illu + o1, make_float4(gd[0], gd[1], gd[2], gd[3]), pol);
     }
 }
 
-template <typename T, bool kAutocast>
+template <typename TI, typename TE, bool kAutocast>
 __global__ void __launch_bounds__(kPwThreads)
-k_recombine_grad_scalar(const float* __restrict__ x, const T* __restrict__ illu, const T* __restrict__ e,
+k_recombine_grad_scalar(const float* __restrict__ x, const TI* __restrict__ illu, const TE* __restrict__ e,
                         const float* __restrict__ g_enh, const float* __restrict__ g_refl, float* __restrict__ g_x,
-                        T* __restrict__ g_illu, T* __restrict__ g_e, long long plane, long long items, float eps)
+                        TI* __restrict__ g_illu, TE* __restrict__ g_e, long long plane, long long items, float eps)
 {
     const long long stride = (long long)gridDim.x * kPwThreads;
     const bool has_gE = g_enh != nullptr, has_gR = g_refl != nullptr;
     for (long long it = (long long)blockIdx.x * kPwThreads + threadIdx.x; it < items; it += stride) {
         const long long f = it / plane, p = it - f * plane;
-        const float d = rnd<T>(__fadd_rn(MapIO<T>::wide(illu[it]), eps));
+        const float d = illu_eps<TI>(MapIO<TI>::wide(illu[it]), eps);
         float gd = 0.0f;
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const long long o = (f * 3 + c) * plane + p;
-            const GradPx g = grad1<T, kAutocast>(x[o], d, has_gE ? MapIO<T>::wide(e[o]) : 0.0f, has_gE ? g_enh[o] : 0.0f,
-                                                 has_gR ? g_refl[o] : 0.0f, has_gE, has_gR);
+            const GradPx g = grad1<TE, kAutocast>(x[o], d, has_gE ? MapIO<TE>::wide(e[o]) : 0.0f, has_gE ? g_enh[o] : 0.0f,
+                                                  has_gR ? g_refl[o] : 0.0f, has_gE, has_gR);
             gd = __fadd_rn(gd, g.gd);
             if (g_x) g_x[o] = g.gx;
-            if (g_e) g_e[o] = MapIO<T>::narrow(g.ge);
+            if (g_e) g_e[o] = MapIO<TE>::narrow(g.ge);
         }
-        if (g_illu) g_illu[it] = MapIO<T>::narrow(gd);
+        if (g_illu) g_illu[it] = MapIO<TI>::narrow(gd);
     }
 }
 
@@ -291,26 +291,28 @@ static int recombine_typed(const float* x, const void* illu, int illu_dt, const 
     });
 }
 
-template <typename T, bool AC>
+// upr_retinex_recombine_grad_typed on map types (TI, TE), arguments checked.  The vector kernel needs every map operand
+// aligned to 4 pixels of its own dtype (aligned4px), as the forward does.
+template <typename TI, typename TE, bool AC>
 static int recombine_grad(const float* x, const void* illu_v, const void* e_v, const float* g_enh, const float* g_refl,
                           float* g_x, void* g_illu_v, void* g_e_v, int n, int h, int w, float eps, cudaStream_t s)
 {
-    const T* illu = static_cast<const T*>(illu_v);
-    const T* e = static_cast<const T*>(e_v);
-    T* g_illu = static_cast<T*>(g_illu_v);
-    T* g_e = static_cast<T*>(g_e_v);
+    const TI* illu = static_cast<const TI*>(illu_v);
+    const TE* e = static_cast<const TE*>(e_v);
+    TI* g_illu = static_cast<TI*>(g_illu_v);
+    TE* g_e = static_cast<TE*>(g_e_v);
     const long long plane = (long long)h * w;
     const bool vec = plane % 4 == 0 && aligned16(x) && aligned4px(illu) && (!e || aligned4px(e)) &&
                      (!g_enh || aligned16(g_enh)) && (!g_refl || aligned16(g_refl)) && (!g_x || aligned16(g_x)) &&
                      (!g_illu || aligned4px(g_illu)) && (!g_e || aligned4px(g_e));
     if (vec) {
         const long long items = (long long)n * (plane / 4);
-        k_recombine_grad_vec<T, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e,
-                                                                         plane / 4, items, eps);
+        k_recombine_grad_vec<TI, TE, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e,
+                                                                              plane / 4, items, eps);
     } else {
         const long long items = (long long)n * plane;
-        k_recombine_grad_scalar<T, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e,
-                                                                            plane, items, eps);
+        k_recombine_grad_scalar<TI, TE, AC><<<pw_grid(items), kPwThreads, 0, s>>>(x, illu, e, g_enh, g_refl, g_x, g_illu,
+                                                                                 g_e, plane, items, eps);
     }
     UPR_LAUNCH_CHECK();
     return UPR_OK;
@@ -452,26 +454,28 @@ int upr_retinex_recombine_typed(const float* x, const void* illu, int illu_dtype
     return upr::recombine_typed(x, illu, illu_dtype, e, e_dtype, flags, refl, enh, n, h, w, eps, static_cast<cudaStream_t>(stream));
 }
 
-int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
-                               const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e, int n, int h,
-                               int w, float eps, upr_stream_t stream)
+int upr_retinex_recombine_grad_typed(const float* x, const void* illu, int illu_dtype, const void* e, int e_dtype, int flags,
+                                     const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e, int n, int h,
+                                     int w, float eps, upr_stream_t stream)
 {
     if (n < 0 || h <= 0 || w <= 0) return UPR_E_SHAPE;
-    if (map_dtype < UPR_DT_F32 || map_dtype > UPR_DT_BF16 || (flags & ~UPR_RETINEX_AUTOCAST)) return UPR_E_PARAM;
+    if (!upr::valid_map_dtypes(illu_dtype, e_dtype, flags)) return UPR_E_PARAM;
     if (n == 0) return UPR_OK;
     if (!x || !illu || (!g_enh && !g_refl) || (!e && (g_enh || g_e))) return UPR_E_NULL;
     if (!g_x && !g_illu && !g_e) return UPR_OK;
     auto s = static_cast<cudaStream_t>(stream);
-    const bool ac = flags & UPR_RETINEX_AUTOCAST;
-    switch (map_dtype) {
-    case UPR_DT_F32: return upr::recombine_grad<float, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
-    case UPR_DT_F16:
-        return ac ? upr::recombine_grad<__half, true>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s)
-                  : upr::recombine_grad<__half, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
-    default:
-        return ac ? upr::recombine_grad<__nv_bfloat16, true>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s)
-                  : upr::recombine_grad<__nv_bfloat16, false>(x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
-    }
+    return upr::with_map_types(illu_dtype, e_dtype, flags, [&](auto ti, auto te, auto ac) {
+        return upr::recombine_grad<typename decltype(ti)::type, typename decltype(te)::type, decltype(ac)::value>(
+            x, illu, e, g_enh, g_refl, g_x, g_illu, g_e, n, h, w, eps, s);
+    });
+}
+
+int upr_retinex_recombine_grad(const float* x, const void* illu, const void* e, int map_dtype, int flags,
+                               const float* g_enh, const float* g_refl, float* g_x, void* g_illu, void* g_e, int n, int h,
+                               int w, float eps, upr_stream_t stream)
+{
+    return upr_retinex_recombine_grad_typed(x, illu, map_dtype, e, map_dtype, flags, g_enh, g_refl, g_x, g_illu, g_e, n, h, w,
+                                            eps, stream);
 }
 
 int upr_scale_clamp_f32(const float* enh, const float* gain_per_image, float* out, int n, int c, int h, int w,

@@ -8,9 +8,10 @@ What is ON the hot path are the two pointwise Retinex lines around the CNN (refe
 Both run in one fused sm_100a kernel (upr_retinex_recombine_f32) at inference (``torch.no_grad()`` / no input requires a
 gradient); the enhance drivers go one step further and hand the two CNN outputs ``forward_maps(x) = (illu, e)`` straight to
 ``native.retinex_clahe`` (recombination fused into the CLAHE histogram kernel).  Under autograd (training) they run as one
-``torch.autograd.Function`` on a fused forward and a fused gradient kernel (upr_retinex_recombine_maps / _grad), with the maps
-in f32 or, under autocast, fp16 / bf16; outputs and gradients equal torch autograd through the stock expressions bit for bit.
-Other operands (CPU tensors, mixed map dtypes, other shapes) keep the stock expressions.
+``torch.autograd.Function`` on a fused forward and a fused gradient kernel (upr_retinex_recombine_typed / _grad_typed), with
+the maps in f32, both in fp16 / bf16, or -- under CUDA autocast, the pair the network emits there -- illu f32 and e fp16 / bf16;
+outputs and gradients equal torch autograd through the stock expressions bit for bit.  Other operands (CPU tensors, mixed map
+dtypes outside autocast, other shapes) keep the stock expressions.
 
 The CNN itself (illumination U-Net with residual / pre-activation blocks and an optional ASPP bottleneck, three feature-
 aggregation branches, :11-403) is dense convolution work that cuDNN already covers and is OUT OF SCOPE for hand-written
@@ -39,18 +40,24 @@ EPSILON = 1e-6   # models/model.py:411
 # ---------------------------------------------------------------------------------------------------
 def _fused_autograd(x: torch.Tensor, illu: torch.Tensor, e=None) -> bool:
     """Whether _RetinexFn takes the operands: CUDA tensors on one device, x [N,3,H,W] f32, illu [N,1,H,W] and e [N,3,H,W]
-    (or None) in one map dtype (f32, fp16, bf16)."""
+    (or None) in one map dtype (f32, fp16, bf16) or, while CUDA autocast is enabled, illu f32 and e fp16 / bf16: the maps of
+    the network under autocast, whose illumination head adds the f32 mean(x)."""
     if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and x.shape[1] == 3):
         return False
     n, _, h, w = x.shape
     if illu.device != x.device or illu.dtype not in native.MAP_DTYPES or illu.shape != (n, 1, h, w):
         return False
-    return e is None or (e.device == x.device and e.dtype == illu.dtype and e.shape == x.shape)
+    if e is None:
+        return True
+    pair = e.dtype == illu.dtype or (illu.dtype == torch.float32 and e.dtype in native.MAP_DTYPES
+                                     and torch.is_autocast_enabled("cuda"))
+    return pair and e.device == x.device and e.shape == x.shape
 
 
 def _retinex_grad_ops(x, illu, e, g_refl, g_enh, autocast, need):
     """The gradient kernel's formulas as differentiable torch ops, for backward(create_graph=True): what autograd computes
-    through the stock expressions, in its accumulation order (include/upretinex_b200.h, upr_retinex_recombine_grad)."""
+    through the stock expressions, in its accumulation order (include/upretinex_b200.h, upr_retinex_recombine_grad_typed).
+    The illu gradient keeps illu's dtype: f32 (not rounded) for the maps of the network under autocast."""
     with torch.autocast("cuda", enabled=False):
         d = illu + EPSILON
         r = x / d
@@ -77,7 +84,7 @@ class _RetinexFn(torch.autograd.Function):
     def forward(ctx, x, illu, e):
         ctx.set_materialize_grads(False)
         ctx.autocast = torch.is_autocast_enabled("cuda")
-        refl, enh = native.retinex_recombine_maps(x, illu, e, autocast=ctx.autocast, eps=EPSILON)
+        refl, enh = native.retinex_recombine_typed(x, illu, e, autocast=ctx.autocast, eps=EPSILON)
         ctx.save_for_backward(x, illu, e)
         return refl if e is None else (refl, enh)
 
@@ -89,7 +96,7 @@ class _RetinexFn(torch.autograd.Function):
         need = (ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2] and g_enh is not None)
         if torch.is_grad_enabled():   # backward(create_graph=True): the gradient must itself be differentiable
             return _retinex_grad_ops(x, illu, e, g_refl, g_enh, ctx.autocast, need)
-        return native.retinex_recombine_grad(x, illu, e, g_enh, g_refl, want=need, autocast=ctx.autocast, eps=EPSILON)
+        return native.retinex_recombine_grad_typed(x, illu, e, g_enh, g_refl, want=need, autocast=ctx.autocast, eps=EPSILON)
 
 
 def retinex_decompose(x: torch.Tensor, illu: torch.Tensor) -> torch.Tensor:
@@ -326,7 +333,8 @@ def accelerate_reference_model(model: nn.Module) -> nn.Module:
     part of its ``multi_scale_enhance`` (:419-440) -- which is what ``AdaptiveParameterAdjuster.apply_adaptive_enhancement``
     needs to reach ``upr_retinex_clahe_f32``.  With autograd enabled (training) ``forward`` and ``retinex_decompose`` run the
     fused forward and gradient kernels of ``_RetinexFn``, whose outputs and gradients equal the instance's own stock arithmetic
-    bit for bit, and keep that arithmetic for operands the kernels do not take (CPU tensors, mixed map dtypes)."""
+    bit for bit, also under CUDA autocast, and keep that arithmetic for operands the kernels do not take (CPU tensors, mixed
+    map dtypes outside autocast)."""
     for name in ("ie_net", "scale1", "scale2", "scale3", "fusion", "output_layer"):
         if not hasattr(model, name):
             raise TypeError(f"accelerate_reference_model: not a UP_Retinex-like module (no attribute {name!r})")

@@ -113,6 +113,8 @@ def _declare(lib):
     lib.upr_retinex_quantize_typed_u8.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_retinex_recombine_grad.restype = i32
     lib.upr_retinex_recombine_grad.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
+    lib.upr_retinex_recombine_grad_typed.restype = i32
+    lib.upr_retinex_recombine_grad_typed.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp]
     lib.upr_letterbox_f32.restype = i32
     lib.upr_letterbox_f32.argtypes = [vp, vp] + [i32] * 10 + [vp, vp]
     lib.upr_letterbox_u8_f32.restype = i32
@@ -824,10 +826,24 @@ def retinex_quantize_u8(x: torch.Tensor, illu: torch.Tensor, e: torch.Tensor, au
 def retinex_recombine_grad(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], g_enh: Optional[torch.Tensor],
                            g_refl: Optional[torch.Tensor], want=(True, True, True), autocast: bool = False, eps: float = 1e-6):
     """(grad x | None, grad illu | None, grad e | None) -- what torch autograd back-propagates through
-    retinex_recombine_maps(x, illu, e, autocast) from the upstream gradients g_enh and g_refl (f32, either None) in one pass
-    (upr_retinex_recombine_grad).  want: which of the three to form; grad illu and grad e have the maps' dtype."""
+    retinex_recombine_maps(x, illu, e, autocast) from the upstream gradients g_enh and g_refl (f32, either None) in one pass.
+    want: which of the three to form; grad illu and grad e have the maps' dtype.  retinex_recombine_grad_typed() with both
+    maps in one dtype."""
     x, illu, e = _maps(x, illu, e)
+    return retinex_recombine_grad_typed(x, illu, e, g_enh, g_refl, want=want, autocast=autocast, eps=eps)
+
+
+def retinex_recombine_grad_typed(x: torch.Tensor, illu: torch.Tensor, e: Optional[torch.Tensor], g_enh: Optional[torch.Tensor],
+                                 g_refl: Optional[torch.Tensor], want=(True, True, True), autocast: bool = False,
+                                 eps: float = 1e-6):
+    """The gradient of retinex_recombine_typed(x, illu, e, autocast) (upr_retinex_recombine_grad_typed): maps as there, e.g. the
+    f32 illu and fp16 / bf16 e of a CNN under autocast; grad illu has illu's dtype and grad e has e's."""
+    x = _cuda(x, "x", shape=(None, 3, None, None))
     n, _, h, w = x.shape
+    illu = _cuda(illu, "illu", tuple(MAP_DTYPES), shape=(n, 1, h, w), device=x.device)
+    if e is not None:
+        e = _cuda(e, "e", tuple(MAP_DTYPES), shape=x.shape, device=x.device)
+    _typed_map_dtypes(illu, e)
     g_enh = _cuda(g_enh, "g_enh", shape=x.shape, device=x.device) if g_enh is not None else None
     g_refl = _cuda(g_refl, "g_refl", shape=x.shape, device=x.device) if g_refl is not None else None
     gx = torch.empty_like(x) if want[0] else None
@@ -838,8 +854,9 @@ def retinex_recombine_grad(x: torch.Tensor, illu: torch.Tensor, e: Optional[torc
         return t.data_ptr() if t is not None else None
 
     with _dev(x.device):
-        _run("upr_retinex_recombine_grad", x.data_ptr(), illu.data_ptr(), ptr(e), MAP_DTYPES[illu.dtype], int(bool(autocast)),
-             ptr(g_enh), ptr(g_refl), ptr(gx), ptr(gi), ptr(ge), n, h, w, float(eps))
+        _run("upr_retinex_recombine_grad_typed", x.data_ptr(), illu.data_ptr(), MAP_DTYPES[illu.dtype], ptr(e),
+             MAP_DTYPES[e.dtype if e is not None else illu.dtype], int(bool(autocast)), ptr(g_enh), ptr(g_refl), ptr(gx), ptr(gi),
+             ptr(ge), n, h, w, float(eps))
     return gx, gi, ge
 
 
